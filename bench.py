@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""Benchmark of the two hot paths on B200 (contract: see the task prompt).
+"""Benchmark of the two hot paths on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--workload rt_cornell_4k|rt_tess100k_4k|rast_cornell_4k|rast_soup_4k|...]
+                    [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  The headline line is the raytracer on BASELINE
 config 3 (Cornell box at 3840x2160, 9 spp, shadow rays, rows shared by the GPUs):
@@ -23,6 +24,16 @@ afterwards rank 0 renders the whole frame alone and bit-compares it with the ass
 render, D2H of the packed framebuffer into pinned memory): at N = 1 draw_*_band on the
 rank's context, at N > 1 ONE caller (rank 0) with a multi-GPU context (b200_init_multi),
 which is what a user of the reference's Draw(screen*) would hold.
+
+--dump-outputs DIR writes, for every workload, what the last timed step left in the buffers the
+timed path renders into, so that two builds can be compared output for output (the scenes and
+the sample are fixed, so the inputs are the same from run to run):
+    DIR/<workload>_argb.npy   packed 0x80RRGGBB pixels of the assembled frame, as float64 (exact)
+    DIR/<workload>_rgb.npy    float RGB, (n, 3) float32            (N = 1 only)
+    DIR/<workload>_depth.npy  float depth, (n,) float32            (N = 1 only; a raytraced pixel whose
+                              primary ray hits nothing, +inf in the depth plane, is written as -1)
+n pixels, in raster order: every pixel of a frame of at most DUMP_PIXELS, otherwise a fixed
+sample (numpy default_rng(0)) of DUMP_PIXELS of them; the five default workloads take < 32 MB.
 
 `cpu_baseline` (N = 1) runs the unmodified reference (oracle/_ref) on one core over a
 bounded sample of the same frame and bit-compares what it rendered with the GPU's pixels.
@@ -70,6 +81,7 @@ RT_LIGHTS = [((0.0, -0.5, -0.7, 1.0), (14.0, 14.0, 14.0))]
 RAST_CAM = (0.0, 0.0, -3.001, 1.0)
 RAST_LIGHT = dict(pos=(0.0, -0.5, 0.0, 1.0), power=(20.0, 20.0, 20.0), indirect=(0.2, 0.2, 0.2))
 TESS_WINDOW = (1200, 1800, 1440, 1)    # x0, y0, w, h of the config-5 CPU sample: sphere outline, floor, shadow edge (~12 s on one core)
+DUMP_PIXELS = 1 << 18                  # --dump-outputs: 24 B a pixel, 6 MB a workload at most
 
 
 def profile_json(name):
@@ -232,7 +244,7 @@ def run_reference(args, workload):
         # ~16 ms per pixel per core at 100 800 triangles: a 96-pixel piece of a row per core and step
         x0, y0, _, _ = TESS_WINDOW
         wins = [(x0 + 96 * (i % 8), y0 + 40 * (i // 8), 96, 1) for i in range(cores)]
-        warmup, steps = min(warmup, 1), min(steps, 3)
+        warmup = min(warmup, 1)
     else:
         wins = [(0, y, W, hh) for (y, hh) in sample_windows(H, cores * 2, 16)]
     jobs = [(W, H, focal, x, y, w, hh, tris.tobytes(), sph.tobytes(), False) for (x, y, w, hh) in wins]
@@ -265,7 +277,7 @@ def run_reference_rast(args, workload, cores):
     from multiprocessing import get_context
     kind, W, H, focal = WORKLOADS[workload]
     n_proc = max(1, min(cores, 8))      # each process owns ~365 MB of static frame buffers at 4K
-    warmup, steps = min(args.warmup, 1), min(args.steps, 3)   # a soup frame takes seconds on a core
+    warmup, steps = min(args.warmup, 1), args.steps   # a soup frame takes seconds on a core
     ctx = get_context("fork")
     with ctx.Pool(n_proc) as pool:
         times = []
@@ -309,6 +321,24 @@ def _ref_rast_worker(args):
 # ------------------------------------------------------------------------------------------
 def bits(a):
     return np.ascontiguousarray(a).view(np.uint32)
+
+
+def dump_outputs(out_dir, workload, argb, rgb=None, depth=None):
+    """--dump-outputs: the pixels of DUMP_PIXELS (see the module docstring) of the device frames
+    argb (H, W) int32, rgb (H, W, 3) and depth (H, W) float32 as DIR/<workload>_<name>.npy."""
+    import torch
+    n = argb.numel()
+    idx = np.arange(n) if n <= DUMP_PIXELS else np.sort(np.random.default_rng(0).choice(n, DUMP_PIXELS, replace=False))
+    sel = torch.from_numpy(idx).to(argb.device)
+    out = {"argb": argb.reshape(-1)[sel].cpu().numpy().view(np.uint32).astype(np.float64)}
+    if rgb is not None:
+        out["rgb"] = rgb.reshape(-1, 3)[sel].cpu().numpy()
+        d = depth.reshape(-1)[sel].cpu().numpy()
+        d[d == np.inf] = -1.0      # misses: hit distances are positive, so -1 is unambiguous
+        out["depth"] = d
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{workload}_{name}.npy"), a)
 
 
 def cpu_baseline_rt(b200, r, workload, W, H, focal, tris, sph):
@@ -555,6 +585,10 @@ def run_b200_one(args, workload):
         return float(t.item()) / steps, launches, last_stats, clocks, wall
 
     ms, launches, st, clocks, wall = timed(step, args.steps, max(args.warmup, 3))
+    if args.dump_outputs:
+        if rank == 0:       # N > 1: the float planes stay on the rank that rendered them
+            dump_outputs(args.dump_outputs, workload, assembled(), *((loc_rgb, loc_depth) if world == 1 else ()))
+        barrier()
     # whole-job units per step (sum over ranks of what each rank processed)
     if kind == "rt":
         units = torch.tensor([st["primary_rays"] + st["shadow_rays"], st["prim_tests"], st["exact_evals"]],
@@ -592,7 +626,7 @@ def run_b200_one(args, workload):
     # assembled frame is in the caller's pinned buffer); the other ranks wait on the host.
     e2e_note = None
     if world == 1:
-        ms_e2e, _, _, _, _ = timed(step_e2e, max(2, args.steps // 2), 3)
+        ms_e2e, _, _, _, _ = timed(step_e2e, args.steps, 3)
     else:
         host_group = dist.new_group(backend="gloo")
         ms_e2e = float("inf")                    # only rank 0 measures (and prints) it
@@ -609,7 +643,7 @@ def run_b200_one(args, workload):
 
             for _ in range(max(12, args.warmup)):  # warm-up: buffers, pipelined sizes, adaptive bands (they move every other frame), planned RT frames
                 whole_frame()
-            k = max(2, args.steps // 2)
+            k = args.steps
             t0 = time.perf_counter()
             for _ in range(k):
                 whole_frame()
@@ -711,7 +745,13 @@ def main():
                     help="N > 1: peer stores into rank 0's frame (default) or an NCCL gather")
     ap.add_argument("--ref-cores", type=int, default=0,
                     help="--impl reference: worker processes (default: every host core; the count is reported)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step rendered as DIR/<workload>_<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs: the reference arm renders samples of rows, not whole frames")
     # default: the headline raytracer line (BASELINE config 3) carrying the rasteriser figure
     # (config 4) and the large raytracer scene (config 5) as nested objects
     workloads = DEFAULT_WORKLOADS if args.workload == "default" else [args.workload]

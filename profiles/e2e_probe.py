@@ -1,5 +1,5 @@
 import importlib, os, sys, time
-ROOT="/root/repo"; sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np, torch
 import helpers as h, bench
 b = importlib.import_module("computer-graphics_b200")

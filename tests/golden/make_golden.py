@@ -112,10 +112,13 @@ def make_reference_textures():
     """The decoded pixels of the texture files in the reference's repository (rasteriser/Textures: metal grill and
     woven wood; cv2 = the decoder cv::imread uses; the two opacity maps grey + thresholded like main() :148-155), so
     that the GPU box -- which has neither the files nor /root/reference -- can draw with the real images
-    (helpers.reference_textures).  4 MiB compressed."""
-    tex = h.reference_textures(from_files=True)
+    (helpers.reference_textures).  The opacity maps whole, the other images thinned (helpers.coarse_texture):
+    0.3 MB compressed."""
+    tex = h.reference_textures(textures_dir=os.path.join(REF, "rasteriser", "Textures"))
     assert tex is not None, "the reference's texture files (or cv2) are not here"
-    np.savez_compressed(os.path.join(HERE, "rast_reference_textures.npz"), **{k: tex[k] for k in h.TEX_IMAGES if k != "marble"})
+    s = h.REF_TEX_STEP
+    np.savez_compressed(os.path.join(HERE, "rast_reference_textures.npz"),
+                        **{k: tex[k] if k.endswith("opacity") else tex[k][::s, ::s] for k in h.TEX_IMAGES if k != "marble"})
     print("reference textures written")
 
 

