@@ -100,7 +100,7 @@ void b200_destroy(b200_ctx *ctx) {
   if (ctx->multi) { multi_destroy(ctx); delete ctx; return; }
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(ctx->stream);
-  DevBuf *bufs[] = {&ctx->rt_src, &ctx->rt_geom, &ctx->rt_spheres, &ctx->rt_planes, &ctx->rt_dtcam, &ctx->rt_bounds, &ctx->rt_cells, &ctx->rt_cell_rec, &ctx->rt_cell_idx, &ctx->rast_src,
+  DevBuf *bufs[] = {&ctx->rt_src, &ctx->rt_geom, &ctx->rt_spheres, &ctx->rt_planes, &ctx->rt_dtcam, &ctx->rt_selfD, &ctx->rt_bounds, &ctx->rt_cells, &ctx->rt_cell_rec, &ctx->rt_cell_idx, &ctx->rast_src,
                     &ctx->rast_setup, &ctx->rast_rowsA, &ctx->rast_rowsB, &ctx->rast_bins, &ctx->rast_tile_count, &ctx->rast_tile_bits,
                     &ctx->rast_tmp, &ctx->rast_keys, &ctx->rast_trimeta, &ctx->rast_big, &ctx->rast_orig, &ctx->rast_shadow8, &ctx->rast_srowsB, &ctx->rast_srowsL, &ctx->rast_chunks, &ctx->rast_world, &ctx->rast_geom_tmp, &ctx->rast_screen, &ctx->rast_low, &ctx->rast_high, &ctx->rast_shadow,
                     &ctx->rast_depth, &ctx->rast_index, &ctx->out_rgb, &ctx->out_depth, &ctx->out_index,

@@ -123,6 +123,7 @@ struct b200_ctx {
   DevBuf rt_spheres;  // rt_sphere[n]
   DevBuf rt_planes;   // float4[..]: per-origin edge-function planes for the filter
   DevBuf rt_dtcam;    // float[n]: per-frame numerator of t for primary rays
+  DevBuf rt_selfD;    // float[lights][n]: per-frame sign and bound of D for a shadow ray on its own triangle
   DevBuf rt_bounds;   // two words: coordinate / normal bounds of a large scene, reduced on the device
   int rt_bounds_on_device = 0;
   DevBuf rt_cells;    // direction grids: per-cell counts, cursors, padded counts, offsets, scan scratch

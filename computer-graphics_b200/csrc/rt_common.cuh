@@ -18,6 +18,7 @@ struct RtKParams {
   // filtered kernel only
   const float4 *planes;      // see rt_filtered.cuh
   const float *dt_cam;       // per triangle: det(camera - v0, e1, e2)
+  const float *self_D;       // per (light, triangle): see RtPrepParams
   int tris_per_tile;
   // direction grids (rt_grid.cuh), GRID kernels only
   const unsigned *cell_off;  // first entry of each cell's list

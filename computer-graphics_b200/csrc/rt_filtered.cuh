@@ -96,6 +96,10 @@ struct RtPrepParams {
   float4 *planes;    // [(1 + n_lights)][n_tiles * RT_TILE][3]
   size_t origin_stride_f4;
   float *dt_cam;     // [n_tris] det(start - v0, e1, e2) for start = camera, in the reference's own arithmetic
+  // [n_lights][n_tris] for a shadow ray that starts on the triangle (a hit point p): the sign of the
+  // reference's D = det(-(L - p), e1, e2) times an upper bound of |D| below 1e30, or 0 where not known.
+  // Null for frames that go to the grid kernels, which do not use it.
+  float *self_D;
 };
 
 __global__ void rt_prep_planes_kernel(const __grid_constant__ RtPrepParams p) {
@@ -153,6 +157,19 @@ __global__ void rt_prep_planes_kernel(const __grid_constant__ RtPrepParams p) {
     // light closer than 1e-3 S to the plane: the "beyond the light" argument
     // loses its margin, leave the triangle to the reference arithmetic
     if (!(fabs(Dt) > 1e-3 * S * N2) || !(fabs(Dt) - slackT > 0.0)) degenerate = true;
+    // Shadow rays from a hit p on this triangle: D = -(L - p).N up to the rounding of r = L - p and of
+    // xdet3 (together below 36 eps S a1 a2), and (L - p).N = Dt - (p - v0).N.  p = cam + t d in the
+    // reference's arithmetic, off the plane by the errors of t's two determinants and of the products and
+    // sums that form p: |(p - v0).N| < 80 eps (C + S) a1 a2, C = |cam|inf, assuming |t d| and |p| below
+    // C + S / 2 (|cam - v0| is): hit points within the scene, the assumption world_S already makes for slackT
+    // (not proven for a ray that grazes the triangle).  256 eps (C + 2S) a1 a2 covers both with a factor
+    // two; outside that band sign(D) = -sign(Dt) and |D| < |Dt| + B.  rt_ex_shadow's guards on r.r hold
+    // too: |Dt| > 2B and |Dt| > 1e-3 S N2 keep |r| above 5e-4 S (S >= 1e-3), and |r|inf <= S < 1e14.
+    const double C = fmax(fabs((double)p.cam[0]), fmax(fabs((double)p.cam[1]), fabs((double)p.cam[2])));
+    const double B = 256.0 * eps * (C + 2.0 * S) * a1 * a2 + 1e-6 * fabs(Dt);
+    const bool known = !degenerate && fabs(Dt) > 2.0 * B && fabs(Dt) + B < 1e29 && S < 1e14;
+    const float dhi = __double2float_ru((fabs(Dt) + B) * (1.0 + 1e-6));
+    if (p.self_D) p.self_D[(size_t)(o - 1) * p.n_tris + i] = !known ? 0.0f : (Dt > 0.0 ? -dhi : dhi);
     q0 = make_float4((float)PU[0], (float)PU[1], (float)PU[2], (float)PV[0]);
     q1 = make_float4((float)PV[1], (float)PV[2], (float)PW[0], (float)PW[1]);
     q2 = make_float4((float)PW[2], __double2float_ru(E), __double2float_rd(fabs(Dt) - slackT),

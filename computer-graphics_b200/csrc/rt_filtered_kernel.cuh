@@ -135,6 +135,16 @@ __device__ __noinline__ RtShade rt_ex_shade(const rt_triangle *__restrict__ src,
   return o;
 }
 
+// Hit point of sample k = 3 kx + ky, start + t * dir (skeleton.cpp:326): the sample's direction is
+// (dir0 + 0.5 (kx - 1), dir1 + 0.5 (ky - 1), f) (:134-137), formed from the middle sample's
+// (dx1, dy1) -- the same float as from dir0 / dir1, -0 included -- for a k known only at run time.
+__device__ __forceinline__ void rt_hit_point(float cx, float cy, float cz, float dx1, float dy1, float dz, float t,
+                                             int k, float &px, float &py, float &pz) {
+  const int kx = k / 3, ky = k - 3 * kx;
+  const float dx = xadd(dx1, xmul(0.5f, (float)(kx - 1))), dy = xadd(dy1, xmul(0.5f, (float)(ky - 1)));
+  px = xadd(cx, xmul(t, dx)); py = xadd(cy, xmul(t, dy)); pz = xadd(cz, xmul(t, dz));
+}
+
 // The TMA tile ring shared by the primary and the shadow passes.
 struct RtRing {
   float4 *smem;
@@ -317,18 +327,25 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
   float *s_ht = reinterpret_cast<float *>(tile_smem + (size_t)NRING * 2 * TILE * RT_REC_F4) + (GRID ? NRING * 2 * TILE : 0);
   float *s_hd = s_ht + 9 * RT_THREADS;
   int *s_hi = reinterpret_cast<int *>(s_hd + 9 * RT_THREADS);
+  float *s_len = s_hd + 18 * RT_THREADS;
 #define HT(k) s_ht[(k) * RT_THREADS + threadIdx.x]
 #define HD(k) s_hd[(k) * RT_THREADS + threadIdx.x]
 #define HI(k) s_hi[(k) * RT_THREADS + threadIdx.x]
-  float len[9];
+  // The scene-streaming kernel (80 registers) also keeps the nine direction lengths and the pixel's running colour
+  // sum there: in registers, most of its spill traffic was that sum, stored and reloaded around every shading call.
+  // The grid kernels (128 registers, no such spills) keep them in registers: 12 KB more shared memory per block
+  // measured 1.2 % slower on the 100 800-triangle box (B200, 1000 W power limit).
+  float len_r[GRID ? 9 : 1], pix_r[GRID ? 3 : 1];
+#define LEN(k) (GRID ? len_r[GRID ? (k) : 0] : s_len[(k) * RT_THREADS + threadIdx.x])
+#define PIX(c) (GRID ? pix_r[GRID ? (c) : 0] : s_len[(9 + (c)) * RT_THREADS + threadIdx.x])
 #pragma unroll
   for (int k = 0; k < 9; ++k) {
     HT(k) = 0.f; HD(k) = FLT_MAX; HI(k) = 0;
-    len[k] = xsqrt(xdot3(dxs[k / 3], dys[k % 3], dz, dxs[k / 3], dys[k % 3], dz));
+    LEN(k) = xsqrt(xdot3(dxs[k / 3], dys[k % 3], dz, dxs[k / 3], dys[k % 3], dz));
   }
   unsigned n_exact = 0;
 #ifdef RT_PROFILE_COUNTERS
-  unsigned prof_cnt[7] = {0, 0, 0, 0, 0, 0, 0};
+  unsigned prof_cnt[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
 #define RT_PC(i) (++prof_cnt[i])
 #else
 #define RT_PC(i)
@@ -422,11 +439,11 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
               // reference distance >= dt_lo*len/(mN+E): cannot beat the current closest
               RtHit b;
               b.dist = HD(k);
-              const bool farther = (mN > E) && (dt_lo * len[k] > b.dist * (mN + E));
+              const bool farther = (mN > E) && (dt_lo * LEN(k) > b.dist * (mN + E));
               if (!farther) {
                 ++n_exact;
                 b.t = HT(k); b.idx = HI(k);
-                const RtHit nb = rt_ex_primary(p.geom, p.dt_cam, cx, cy, cz, tri, m3 >= E ? 1 : 0, dx, dy, dz, len[k], b);
+                const RtHit nb = rt_ex_primary(p.geom, p.dt_cam, cx, cy, cz, tri, m3 >= E ? 1 : 0, dx, dy, dz, LEN(k), b);
                 if (nb.idx != b.idx || nb.dist != b.dist) { HT(k) = nb.t; HD(k) = nb.dist; HI(k) = nb.idx; }
               }
             }
@@ -483,7 +500,8 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
   // ============================ shadow rays ============================
   constexpr int NL = MULTI ? B200_MAX_LIGHTS : 1;
   float dl[MULTI ? NL * 27 : 1];
-  float pix[3] = {0.f, 0.f, 0.f};
+#pragma unroll
+  for (int c = 0; c < 3; ++c) PIX(c) = 0.f;
   const unsigned warp_active = __ballot_sync(0xffffffffu, active != 0);
   for (int l = 0; l < p.n_lights; ++l) {
     const float Lx = p.lights[l][0], Ly = p.lights[l][1], Lz = p.lights[l][2];
@@ -711,7 +729,39 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
           const float4 q0 = T[(r0 + j) * 3], q1 = T[(r0 + j) * 3 + 1], q2 = T[(r0 + j) * 3 + 2];
           const float Eg = q2.y * pnorm;
           RT_PC(4);
-          // ---- L2 / EX: per shadow ray ----
+          if (GRID) {
+            // ---- L2 / EX: per shadow ray.  The grid kernels keep the reference's call inside the unrolled loop and
+            //      no self-pair test: with the test below they measured 1.2-2.7 % slower on the 100 800-triangle box
+            //      (B200, 1000 W power limit; their warps run out of step and the loop's code size costs more) ----
+#pragma unroll
+            for (int k = 0; k < 9; ++k) {
+              if (!((todo >> k) & 1u) || ((occluded >> k) & 1u)) continue;
+              const float px = xadd(cx, xmul(HT(k), dxs[k / 3])), py = xadd(cy, xmul(HT(k), dys[k % 3])),
+                          pz = xadd(cz, xmul(HT(k), dz));
+              const float gx = -xsub(Lx, px), gy = -xsub(Ly, py), gz = -xsub(Lz, pz);
+              const float mU = fmaf(q0.x, gx, fmaf(q0.y, gy, q0.z * gz));
+              const float mV = fmaf(q0.w, gx, fmaf(q1.x, gy, q1.y * gz));
+              const float mW = fmaf(q1.z, gx, fmaf(q1.w, gy, q2.x * gz));
+              const float m3 = fminf(fminf(mU, mV), mW);
+              const float mN = mU + mV + mW;
+              RT_PC(5);
+              if (m3 < -Eg || mN + Eg < q2.z) continue;          // definite miss / behind the start
+              RT_PC(6);
+              if (m3 >= Eg && mN - Eg >= q2.w && q2.z >= 1e-4f * mN) {
+                occluded |= 1u << k;                              // definite occluder
+                continue;
+              }
+              ++n_exact;
+#ifdef RT_PROFILE_COUNTERS
+              RT_PC(7);
+              if (tri == HI(k)) RT_PC(8);
+#endif
+              if (rt_ex_shadow(p.geom, p.src, p.sph, tri, HI(k), px, py, pz, Lx, Ly, Lz)) occluded |= 1u << k;
+            }
+            continue;
+          }
+          // ---- L2: per shadow ray; what it cannot decide is left in `amb` ----
+          unsigned amb = 0;
 #pragma unroll
           for (int k = 0; k < 9; ++k) {
             if (!((todo >> k) & 1u) || ((occluded >> k) & 1u)) continue;
@@ -730,7 +780,39 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
               occluded |= 1u << k;                              // definite occluder
               continue;
             }
+            amb |= 1u << k;
+          }
+          // ---- the rays that start on this triangle: where rt_prep_planes_kernel knows the sign of the
+          //      reference's D (self_D), Dt formed as rt_ex_shadow forms it decides the pair the way its early
+          //      return does (|self_D| >= |D|): t < 0.  A loop without calls: the triangle's data stay in registers ----
+          if (amb) {
+            const float sD = p.self_D ? __ldg(p.self_D + (size_t)l * p.n_tris + tri) : 0.0f;
+            const float4 g0 = __ldg(p.geom + 3 * tri), g1 = __ldg(p.geom + 3 * tri + 1);
+            const float e2z = __ldg(&p.geom[3 * tri + 2].x);
+            const float *n = p.src[tri].normal;
+            const float n0 = __ldg(n), n1 = __ldg(n + 1), n2 = __ldg(n + 2);
+            for (unsigned m = amb; m; m &= m - 1) {   // (sD tested inside: every load is issued at once)
+              const int k = __ffs(m) - 1;
+              if (sD == 0.0f || HI(k) != tri) continue;
+              float px, py, pz;
+              rt_hit_point(cx, cy, cz, dxs[1], dys[1], dz, HT(k), k, px, py, pz);
+              const float ox = xadd(px, xmul(n0, 0.00001f)), oy = xadd(py, xmul(n1, 0.00001f)),
+                          oz = xadd(pz, xmul(n2, 0.00001f));                                    // :394
+              const float Dt = xdet3(xsub(ox, g0.x), xsub(oy, g0.y), xsub(oz, g0.z), g0.w, g1.x, g1.y, g1.z, g1.w, e2z);
+              if (((Dt < 0.0f) != (sD < 0.0f)) && fabsf(Dt) > 1e-20f * fabsf(sD)) amb &= ~(1u << k);
+            }
+          }
+          // ---- EX: the reference arithmetic, one copy of the code outside the unrolled loop (instruction cache) ----
+          while (amb) {
+            const int k = __ffs(amb) - 1;
+            amb &= amb - 1;
+            float px, py, pz;
+            rt_hit_point(cx, cy, cz, dxs[1], dys[1], dz, HT(k), k, px, py, pz);
             ++n_exact;
+#ifdef RT_PROFILE_COUNTERS
+            RT_PC(7);
+            if (tri == HI(k)) RT_PC(8);
+#endif
             if (rt_ex_shadow(p.geom, p.src, p.sph, tri, HI(k), px, py, pz, Lx, Ly, Lz)) occluded |= 1u << k;
           }
         }
@@ -749,10 +831,10 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
       if (MULTI) {
         dl[(l * 9 + k) * 3 + 0] = s.pw[0]; dl[(l * 9 + k) * 3 + 1] = s.pw[1]; dl[(l * 9 + k) * 3 + 2] = s.pw[2];
       } else {
-        pix[0] = xadd(pix[0], s.pw[0]); pix[1] = xadd(pix[1], s.pw[1]); pix[2] = xadd(pix[2], s.pw[2]);
-        pix[0] = xadd(pix[0], xmul(s.col[0], 0.5f));
-        pix[1] = xadd(pix[1], xmul(s.col[1], 0.5f));
-        pix[2] = xadd(pix[2], xmul(s.col[2], 0.5f));
+        PIX(0) = xadd(PIX(0), s.pw[0]); PIX(1) = xadd(PIX(1), s.pw[1]); PIX(2) = xadd(PIX(2), s.pw[2]);
+        PIX(0) = xadd(PIX(0), xmul(s.col[0], 0.5f));
+        PIX(1) = xadd(PIX(1), xmul(s.col[1], 0.5f));
+        PIX(2) = xadd(PIX(2), xmul(s.col[2], 0.5f));
       }
     }
   }
@@ -764,18 +846,19 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
         if (!((active >> k) & 1u)) continue;
         if (MULTI)
           for (int l = 0; l < p.n_lights; ++l) {
-            pix[0] = xadd(pix[0], dl[(l * 9 + k) * 3 + 0]);
-            pix[1] = xadd(pix[1], dl[(l * 9 + k) * 3 + 1]);
-            pix[2] = xadd(pix[2], dl[(l * 9 + k) * 3 + 2]);
+            PIX(0) = xadd(PIX(0), dl[(l * 9 + k) * 3 + 0]);
+            PIX(1) = xadd(PIX(1), dl[(l * 9 + k) * 3 + 1]);
+            PIX(2) = xadd(PIX(2), dl[(l * 9 + k) * 3 + 2]);
           }
         const float px = xadd(cx, xmul(HT(k), dxs[k / 3])), py = xadd(cy, xmul(HT(k), dys[k % 3])),
                     pz = xadd(cz, xmul(HT(k), dz));
         const RtShade s = rt_ex_shade(p.src, p.sph, 0, HI(k), px, py, pz, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0, 0);
-        pix[0] = xadd(pix[0], xmul(s.col[0], 0.5f));
-        pix[1] = xadd(pix[1], xmul(s.col[1], 0.5f));
-        pix[2] = xadd(pix[2], xmul(s.col[2], 0.5f));
+        PIX(0) = xadd(PIX(0), xmul(s.col[0], 0.5f));
+        PIX(1) = xadd(PIX(1), xmul(s.col[1], 0.5f));
+        PIX(2) = xadd(PIX(2), xmul(s.col[2], 0.5f));
       }
     }
+    const float pix[3] = {PIX(0), PIX(1), PIX(2)};
     rt_store_pixel(p, pid, active != 0, pix);
   }
   rt_count(p.counters + 0, (unsigned long long)__popc(active) * p.n_lights);
@@ -784,6 +867,7 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
     atomicMax(p.block_cost + s_cost_at[warp], (((unsigned)clock() - s_cost_t0[warp]) >> 8) * (s_split ? 8u : 1u));
 #ifdef RT_PROFILE_COUNTERS
   if (live) for (int i = 0; i < 6; ++i) atomicAdd(p.counters + 2 + i, (unsigned long long)prof_cnt[i + (i >= 2 ? 1 : 0)]);
+  if (live) { atomicAdd(p.counters + 8, (unsigned long long)prof_cnt[8]); atomicAdd(p.counters + 14, (unsigned long long)prof_cnt[7]); }
   // diagnostic build only: the depth plane carries this pixel's shadow L1 test count, the index plane its exact evaluations
   if (live && p.depth) p.depth[pid] = (float)prof_cnt[3];
   if (live && p.index) p.index[pid] = (int)n_exact;

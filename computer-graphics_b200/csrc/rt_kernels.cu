@@ -201,6 +201,14 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
   p.planes = (const float4 *)ctx->rt_planes.p;
   if (int rc = ensure(ctx, ctx->rt_dtcam, sizeof(float) * (size_t)(n > 0 ? n : 1))) return rc;
   p.dt_cam = (const float *)ctx->rt_dtcam.p;
+  // large scenes: per-frame direction grids, then the grid kernels stream cell lists (decided here, before the plane
+  // records are made: the self-pair signs are made only for the scene-streaming kernel, which uses them)
+  bool use_grid = n > 0 && (ctx->opt_rt_grid == 1 || (ctx->opt_rt_grid == 0 && n >= RT_GRID_AUTO_TRIS));
+  p.self_D = nullptr;
+  if (!use_grid) {
+    if (int rc = ensure(ctx, ctx->rt_selfD, sizeof(float) * (size_t)(n > 0 ? n : 1) * (f.n_lights > 0 ? f.n_lights : 1))) return rc;
+    p.self_D = (const float *)ctx->rt_selfD.p;
+  }
 
   if (n > 0) {
     RtPrepParams q;
@@ -235,6 +243,7 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
     q.planes = (float4 *)ctx->rt_planes.p;
     q.origin_stride_f4 = origin_stride;
     q.dt_cam = (float *)ctx->rt_dtcam.p;
+    q.self_D = (float *)p.self_D;   // null: a grid frame (a grid frame that falls back to streaming decides every self pair exactly)
     dim3 grid((n + 127) / 128, 1 + f.n_lights);
     rt_prep_planes_kernel<<<grid, 128, 0, ctx->stream>>>(q);
     ctx->stats.kernel_launches++;
@@ -243,11 +252,10 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
 
   const int my_blocks = (p.blocks_y - p.il_r + p.il_n - 1) / p.il_n;
   dim3 grid((f.W + 15) / 16, my_blocks);
-  const size_t hit_smem = 27 * (size_t)RT_THREADS * sizeof(float);   // t, distance, index of the nine samples per thread
-  const size_t smem = 2 * (size_t)RT_TILE * RT_REC_F4 * sizeof(float4) + hit_smem;
+  // per thread: t, distance, index of the nine samples; the scene-streaming kernel also their ray lengths and the colour sum
+  const size_t hit_smem = 27 * (size_t)RT_THREADS * sizeof(float);
+  const size_t smem = 2 * (size_t)RT_TILE * RT_REC_F4 * sizeof(float4) + hit_smem + 12 * (size_t)RT_THREADS * sizeof(float);
 
-  // ---- large scenes: per-frame direction grids, then the kernel streams cell lists ----
-  bool use_grid = n > 0 && (ctx->opt_rt_grid == 1 || (ctx->opt_rt_grid == 0 && n >= RT_GRID_AUTO_TRIS));
   if (use_grid) {
     const size_t cells = (size_t)grid.x * p.blocks_y + (size_t)f.n_lights * 6 * RT_GRID_FACE;   // camera cells: every block of the range
     const size_t scan_tmp = cells / 4096 + 2;

@@ -26,8 +26,9 @@ r.rt_render_device(cam, bench.RT_LIGHTS, 0, H, rgb.data_ptr(), depth.data_ptr(),
 c = (ctypes.c_uint64 * 16)()
 assert b.load_library().b200_debug_counters(r.ctx, c) == 0
 names = ["shadow rays", "exact evals", "primary L1 tests", "primary L1 passes", "shadow L1 tests", "shadow L1 passes",
-         "shadow L2 tests", "shadow L2 non-miss", "-", "grid list entries", "grid: blocks streaming the scene",
-         "grid: light cells walked", "records streamed (camera)", "records streamed (lights)", "-", "-"]
+         "shadow L2 tests", "shadow L2 non-miss", "shadow exact, own triangle", "grid list entries",
+         "grid: blocks streaming the scene", "grid: light cells walked", "records streamed (camera)",
+         "records streamed (lights)", "shadow exact", "-"]
 npx = W * H
 for n, v in zip(names, c):
     print(f"{n:36s} {v:14d}  {v / npx:8.3f} per pixel  {v / (npx / 256):10.2f} per block")
