@@ -86,6 +86,7 @@ ABI_SYMBOLS = [
     "b200_scene_soup_rast",
     "render_raytrace", "render_raytrace_band", "draw_raytrace", "draw_raytrace_band",
     "b200_measure_fp32_peak", "rt_upload_scene", "rt_render_device",
+    "render_raytrace_views", "draw_raytrace_views", "rt_render_views_device",
     "render_raster_clipped", "render_raster", "render_raster_band", "draw_raster", "raster_read_buffers",
     "raster_read_clipped", "rast_upload_clipped", "rast_render_device", "draw_raster_band",
     "rast_upload_scene", "rast_draw_device", "rast_set_textures",
@@ -125,6 +126,21 @@ def make_camera(pos, focal, R, width, height):
     c.R[:] = [float(x) for x in np.asarray(R, np.float32).reshape(-1)]
     c.width, c.height = int(width), int(height)
     return c
+
+
+def make_cameras(cams):
+    """[Camera or (pos, focal, R, width, height), ...] -> ctypes array of camera_t (one per view)."""
+    arr = (Camera * max(1, len(cams)))()
+    for i, c in enumerate(cams):
+        arr[i] = c if isinstance(c, Camera) else make_camera(*c)
+    return arr
+
+
+def _cameras(cams):
+    """(ctypes array of camera_t, number of views) for a list of cameras or an array from make_cameras."""
+    if isinstance(cams, ctypes.Array):
+        return cams, len(cams)
+    return make_cameras(cams), len(cams)
 
 
 def make_lights(lights):
@@ -251,6 +267,42 @@ class Renderer:
                                        int(row_end), _ptr(d_rgb), _ptr(d_depth), _ptr(d_index),
                                        _ptr(d_argb))
         self._check(rc, "rt_render_device")
+
+    def render_raytrace_views(self, tris, spheres, cams, lights, want=("rgb", "depth", "index")):
+        """Whole frames of every camera in `cams` (same width and height) in one call: arrays of shape
+        (K, H, W, 3) / (K, H, W), view k equal to render_raytrace with cams[k]."""
+        ca, k = _cameras(cams)
+        W, H = (ca[0].width, ca[0].height) if k else (0, 0)
+        rgb = np.zeros((k, H, W, 3), np.float32) if "rgb" in want else None
+        depth = np.zeros((k, H, W), np.float32) if "depth" in want else None
+        index = np.zeros((k, H, W), np.int32) if "index" in want else None
+        la = make_lights(lights)
+        rc = self.lib.render_raytrace_views(
+            self.ctx, _ptr(tris), len(tris), _ptr(spheres), 0 if spheres is None else len(spheres),
+            ca, int(k), la, len(lights), _ptr(rgb), _ptr(depth), _ptr(index))
+        self._check(rc, "render_raytrace_views")
+        return dict(rgb=rgb, depth=depth, index=index)
+
+    def draw_raytrace_views(self, tris, spheres, cams, lights, out=None):
+        """Packed frames of every camera in `cams`: (K, H, W) uint32."""
+        ca, k = _cameras(cams)
+        W, H = (ca[0].width, ca[0].height) if k else (0, 0)
+        argb = np.zeros((k, H, W), np.uint32) if out is None else out
+        la = make_lights(lights)
+        rc = self.lib.draw_raytrace_views(self.ctx, _ptr(tris), len(tris), _ptr(spheres),
+                                          0 if spheres is None else len(spheres), ca, int(k), la, len(lights),
+                                          _ptr(argb))
+        self._check(rc, "draw_raytrace_views")
+        return argb
+
+    def rt_render_views_device(self, cams, lights, d_rgb=None, d_depth=None, d_index=None, d_argb=None):
+        """Every camera in `cams` on the uploaded scene into device pointers (ints) holding K whole frames
+        back to back; asynchronous."""
+        ca, k = _cameras(cams)
+        la = make_lights(lights)
+        rc = self.lib.rt_render_views_device(self.ctx, ca, int(k), la, len(lights), _ptr(d_rgb), _ptr(d_depth),
+                                             _ptr(d_index), _ptr(d_argb))
+        self._check(rc, "rt_render_views_device")
 
     # ---- RAST ----------------------------------------------------------------
     def render_raster_clipped(self, clipped, cam, light, want=("rgb", "depth", "index")):

@@ -303,6 +303,98 @@ int rt_render_device(b200_ctx *ctx, const camera_t *cam, const light_t *lights, 
                          ctx->opt_rt_il_n, ctx->opt_rt_il_r);
 }
 
+}  // extern "C"
+
+// ---- RT, batched views: whole frames of n_views cameras of one size ---------------------
+// (also the multi-GPU context's check, before the views are shared out)
+int check_views(b200_ctx *ctx, const camera_t *cams, int n_views, const light_t *lights, int n_lights) {
+  if (n_views < 1) return ctx_fail(ctx, B200_EINVAL, "n_views must be at least 1");
+  if (!cams) return ctx_fail(ctx, B200_EINVAL, "null cameras");
+  for (int k = 0; k < n_views; ++k) {
+    if (int rc = check_camera(ctx, &cams[k])) return rc;
+    if (cams[k].width != cams[0].width || cams[k].height != cams[0].height)
+      return ctx_fail(ctx, B200_EINVAL, "every view must have the same width and height");
+  }
+  if (n_lights < 0 || n_lights > B200_MAX_LIGHTS || (n_lights > 0 && !lights))
+    return ctx_fail(ctx, B200_EINVAL, "bad lights (at most 8)");
+  return B200_OK;
+}
+
+extern "C" {
+
+static int copy_out(b200_ctx *ctx, void *host, const void *dev, size_t bytes);
+
+static int rt_views_device(b200_ctx *ctx, const camera_t *cams, int n_views, const light_t *lights, int n_lights,
+                           float *d_rgb, float *d_depth, int32_t *d_index, uint32_t *d_argb) {
+  if (int rc = check_views(ctx, cams, n_views, lights, n_lights)) return rc;
+  std::vector<RtFrame> fs((size_t)n_views);
+  for (int k = 0; k < n_views; ++k)
+    if (int rc = fill_frame(ctx, &cams[k], lights, n_lights, 0, cams[0].height, fs[k])) return rc;
+  cudaSetDevice(ctx->device);
+  if (ctx->rast_inflight.active) if (int rc = finish_stats(ctx)) return rc;   // the counters are shared
+  ctx->stats.kernel_launches = 0;
+  CU_CHECK(ctx, cudaMemsetAsync(ctx->counters.p, 0, 32 * sizeof(unsigned long long), ctx->stream));
+  CU_CHECK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  if (int rc = rt_launch_views(ctx, fs.data(), n_views, d_rgb, d_depth, d_index, d_argb)) return rc;
+  CU_CHECK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  ctx->stats.primary_rays = (uint64_t)n_views * (uint64_t)cams[0].width * (uint64_t)cams[0].height * 9u;
+  if (int rc = enqueue_counter_readback(ctx)) return rc;
+  ctx->pending = 1;
+  return B200_OK;
+}
+
+int rt_render_views_device(b200_ctx *ctx, const camera_t *cams, int n_views, const light_t *lights, int n_lights,
+                           float *d_rgb, float *d_depth, int32_t *d_index, uint32_t *d_argb) {
+  if (!ctx) return B200_EINVAL;
+  SINGLE_ONLY(ctx);
+  return rt_views_device(ctx, cams, n_views, lights, n_lights, d_rgb, d_depth, d_index, d_argb);
+}
+
+// The host-pointer views entries: the views into the staging buffers, then one copy per output.
+static int rt_views_host(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                         const camera_t *cams, int n_views, const light_t *lights, int n_lights, float *rgb_out,
+                         float *depth_out, int32_t *index_out, uint32_t *argb_out) {
+  if (int rc = check_views(ctx, cams, n_views, lights, n_lights)) return rc;
+  if (int rc = rt_upload_scene(ctx, tris, n_tris, spheres, n_spheres)) return rc;
+  const size_t npix = (size_t)n_views * cams[0].width * cams[0].height;
+  if (rgb_out) if (int rc = ensure(ctx, ctx->out_rgb, npix * 3 * sizeof(float))) return rc;
+  if (depth_out) if (int rc = ensure(ctx, ctx->out_depth, npix * sizeof(float))) return rc;
+  if (index_out) if (int rc = ensure(ctx, ctx->out_index, npix * sizeof(int32_t))) return rc;
+  if (argb_out) if (int rc = ensure(ctx, ctx->out_argb, npix * sizeof(uint32_t))) return rc;
+  if (int rc = rt_views_device(ctx, cams, n_views, lights, n_lights, rgb_out ? (float *)ctx->out_rgb.p : nullptr,
+                               depth_out ? (float *)ctx->out_depth.p : nullptr,
+                               index_out ? (int32_t *)ctx->out_index.p : nullptr,
+                               argb_out ? (uint32_t *)ctx->out_argb.p : nullptr))
+    return rc;
+  if (int rc = copy_out(ctx, rgb_out, ctx->out_rgb.p, npix * 3 * sizeof(float))) return rc;
+  if (int rc = copy_out(ctx, depth_out, ctx->out_depth.p, npix * sizeof(float))) return rc;
+  if (int rc = copy_out(ctx, index_out, ctx->out_index.p, npix * sizeof(int32_t))) return rc;
+  if (int rc = copy_out(ctx, argb_out, ctx->out_argb.p, npix * sizeof(uint32_t))) return rc;
+  return finish_stats(ctx);
+}
+
+int render_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                          const camera_t *cams, int n_views, const light_t *lights, int n_lights, float *rgb_out,
+                          float *depth_out, int32_t *index_out) {
+  if (!ctx) return B200_EINVAL;
+  if (ctx->multi)
+    return multi_raytrace_views(ctx, tris, n_tris, spheres, n_spheres, cams, n_views, lights, n_lights, rgb_out,
+                                depth_out, index_out, nullptr);
+  return rt_views_host(ctx, tris, n_tris, spheres, n_spheres, cams, n_views, lights, n_lights, rgb_out, depth_out,
+                       index_out, nullptr);
+}
+
+int draw_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                        const camera_t *cams, int n_views, const light_t *lights, int n_lights, uint32_t *argb_out) {
+  if (!ctx) return B200_EINVAL;
+  if (!argb_out) return ctx_fail(ctx, B200_EINVAL, "null framebuffer");
+  if (ctx->multi)
+    return multi_raytrace_views(ctx, tris, n_tris, spheres, n_spheres, cams, n_views, lights, n_lights, nullptr,
+                                nullptr, nullptr, argb_out);
+  return rt_views_host(ctx, tris, n_tris, spheres, n_spheres, cams, n_views, lights, n_lights, nullptr, nullptr,
+                       nullptr, argb_out);
+}
+
 static int rast_frame(b200_ctx *ctx, bool whole_draw, const camera_t *cam, const rast_light_t *light, int row_begin,
                       int row_end, float *d_rgb, float *d_depth, int32_t *d_index, uint32_t *d_argb, bool allow_spec);
 

@@ -122,7 +122,7 @@ struct b200_ctx {
   DevBuf rt_geom;     // float4[3n]: v0, e1, e2 for the exact test
   DevBuf rt_spheres;  // rt_sphere[n]
   DevBuf rt_planes;   // float4[..]: per-origin edge-function planes for the filter
-  DevBuf rt_dtcam;    // float[n]: per-frame numerator of t for primary rays
+  DevBuf rt_dtcam;    // float[n]: per-frame numerator of t for primary rays (batched views: [views][n])
   DevBuf rt_selfD;    // float[lights][n]: per-frame sign and bound of D for a shadow ray on its own triangle
   DevBuf rt_bounds;   // two words: coordinate / normal bounds of a large scene, reduced on the device
   int rt_bounds_on_device = 0;
@@ -256,6 +256,9 @@ static inline int band_slice_edge(int row0, int rows, int i, int k, int align) {
 }
 int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int32_t *d_index,
               uint32_t *d_argb);
+// whole frames of n_views cameras of one size, frame k of each output at k * W * H (rgb: times 3)
+int rt_launch_views(b200_ctx *ctx, const RtFrame *fs, int n_views, float *d_rgb, float *d_depth, int32_t *d_index,
+                    uint32_t *d_argb);
 // multi.cu: entry points of a multi-GPU context (api.cu forwards to these)
 void multi_destroy(b200_ctx *ctx);
 int multi_synchronize(b200_ctx *ctx);
@@ -264,6 +267,10 @@ int multi_rast_set_textures(b200_ctx *ctx, const rast_textures_t *tex);
 int multi_raytrace(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
                    const camera_t *cam, const light_t *lights, int n_lights, int row_begin, int row_end,
                    float *rgb_out, float *depth_out, int32_t *index_out, uint32_t *argb_out);
+int multi_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                         const camera_t *cams, int n_views, const light_t *lights, int n_lights, float *rgb_out,
+                         float *depth_out, int32_t *index_out, uint32_t *argb_out);
+int check_views(b200_ctx *ctx, const camera_t *cams, int n_views, const light_t *lights, int n_lights);   // api.cu
 int multi_raster(b200_ctx *ctx, const rast_triangle *room, int n_room, const rast_triangle *boxes, int n_boxes,
                  const camera_t *cam, const rast_light_t *light, int row_begin, int row_end, float *rgb_out,
                  float *depth_out, int32_t *index_out, uint32_t *argb_out);

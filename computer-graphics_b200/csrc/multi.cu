@@ -310,6 +310,32 @@ int multi_raytrace(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_
   return B200_OK;
 }
 
+// Batched views: whole views go to whole devices -- device i renders the contiguous run [k_i, k_i+1) of the views
+// with the single-device views path and returns it straight into its slice of the caller's buffers.  No bands.
+int multi_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                         const camera_t *cams, int n_views, const light_t *lights, int n_lights, float *rgb_out,
+                         float *depth_out, int32_t *index_out, uint32_t *argb_out) {
+  b200_multi *mc = ctx->multi;
+  if (int rc = check_views(ctx, cams, n_views, lights, n_lights)) return rc;
+  const size_t npix = (size_t)cams[0].width * cams[0].height;
+  const int n = mc->n;
+  const int rc = multi_run(ctx, [&](int i) -> int {
+    const int a = (int)((long long)n_views * i / n), b = (int)((long long)n_views * (i + 1) / n);
+    b200_ctx *c = mc->child[i];
+    c->stats = b200_stats{};
+    if (b <= a) return B200_OK;
+    const size_t off = (size_t)a * npix;
+    if (argb_out)
+      return draw_raytrace_views(c, tris, n_tris, spheres, n_spheres, cams + a, b - a, lights, n_lights, argb_out + off);
+    return render_raytrace_views(c, tris, n_tris, spheres, n_spheres, cams + a, b - a, lights, n_lights,
+                                 rgb_out ? rgb_out + 3 * off : nullptr, depth_out ? depth_out + off : nullptr,
+                                 index_out ? index_out + off : nullptr);
+  });
+  if (rc != B200_OK) return rc;
+  multi_sum_stats(ctx);
+  return B200_OK;
+}
+
 // ---- rasteriser -------------------------------------------------------------------------
 // Every device keeps its own copy of the images (each over its own PCIe link).
 int multi_rast_set_textures(b200_ctx *ctx, const rast_textures_t *tex) {

@@ -79,7 +79,7 @@ __device__ __forceinline__ void tma_bulk_g2s(void *dst, const void *src, uint32_
 
 // ---- per-frame plane records ------------------------------------------------------
 // origin 0 = camera (directions (dx, dy, f): the z term is folded into a constant)
-// origin 1+l = light l (directions g = hit - light, general 3-D)
+// origin 1+l = light l (directions g = hit - light, general 3-D)   (batched views: see RtPrepViews)
 //   q0 = (Ux, Uy, Uz|cU, Vx)  q1 = (Vy, Vz|cV, Wx, Wy)  q2 = (Wz|cW, E, T0, T1)
 // camera: E absolute (max |d| folded in), T0 = lower bound of |Dt|, T1 = E + 0.5*max(|Px|+|Py|)
 // light : E per unit |g|_inf, T0/T1 = reject / definite thresholds of d.PN (t >= 0 test)
@@ -102,19 +102,41 @@ struct RtPrepParams {
   float *self_D;
 };
 
-__global__ void rt_prep_planes_kernel(const __grid_constant__ RtPrepParams p) {
+// Batched views (one launch renders up to RT_VIEWS_MAX whole frames of one scene and one set of lights):
+// origin v < n_views is view v's camera, origin n_views + l is light l.  Each view has its own camera
+// records and dt_cam[v][n_tris]; the light records and self_D are shared.  Kernel parameters, indexed by
+// blockIdx.y (preparation) / blockIdx.z (render).
+constexpr int RT_VIEWS_MAX = 64;
+struct RtPrepViews {
+  int n_views;
+  float cam_inf;                 // max over the views of |cam|inf: C of the self_D bound (see below)
+  float cam[RT_VIEWS_MAX][4];    // position, focal
+  float dmax[RT_VIEWS_MAX];
+};
+struct RtViewsParams {
+  int n_views;
+  struct { float cam[3]; float focal; float R[16]; } view[RT_VIEWS_MAX];
+};
+
+template <bool VIEWS>
+__device__ __forceinline__ void rt_prep_planes_body(const RtPrepParams &p, const RtPrepViews *pv) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   const int o = blockIdx.y;  // origin
   if (i >= p.n_tris) return;
+  const bool is_cam = VIEWS ? o < pv->n_views : o == 0;
+  const int l = VIEWS ? o - pv->n_views : o - 1;   // light of a light origin
+  const float *cam = VIEWS ? pv->cam[is_cam ? o : 0] : p.cam;
+  const float focal = VIEWS ? cam[3] : p.focal;
+  const float dmax = VIEWS ? pv->dmax[is_cam ? o : 0] : p.dmax;
   const float4 g0 = p.geom[3 * i], g1 = p.geom[3 * i + 1], g2 = p.geom[3 * i + 2];
   const double e1[3] = {g0.w, g1.x, g1.y}, e2[3] = {g1.z, g1.w, g2.x};
   const float v0[3] = {g0.x, g0.y, g0.z};
   double s[3];
-  if (o == 0) {
+  if (is_cam) {
     // exactly the reference's `start - v0` (skeleton.cpp:296)
-    for (int k = 0; k < 3; ++k) s[k] = (double)xsub(p.cam[k], v0[k]);
+    for (int k = 0; k < 3; ++k) s[k] = (double)xsub(cam[k], v0[k]);
   } else {
-    for (int k = 0; k < 3; ++k) s[k] = (double)p.lights[o - 1][k] - (double)v0[k];
+    for (int k = 0; k < 3; ++k) s[k] = (double)p.lights[l][k] - (double)v0[k];
   }
   const double N[3] = {e1[1] * e2[2] - e1[2] * e2[1], e1[2] * e2[0] - e1[0] * e2[2],
                        e1[0] * e2[1] - e1[1] * e2[0]};
@@ -135,15 +157,15 @@ __global__ void rt_prep_planes_kernel(const __grid_constant__ RtPrepParams p) {
   const double N2 = sqrt(N[0] * N[0] + N[1] * N[1] + N[2] * N[2]);
   float4 q0, q1, q2;
   bool degenerate = !(isfinite(Dt) && isfinite(N1) && a1 < 1e18 && a2 < 1e18);
-  if (o == 0) {
+  if (is_cam) {
     const double sm = fmax(fabs(s[0]), fmax(fabs(s[1]), fabs(s[2])));
     // Rounding-error bound of the reference's three determinants plus this
     // filter's own (planes rounded to float, FMA chains): each is below
     // 54 eps |d|inf X Y; 256 leaves a wide safety factor.
-    const double E = 256.0 * eps * (a1 * a2 + sm * (a1 + a2)) * (double)p.dmax * 1.01;
+    const double E = 256.0 * eps * (a1 * a2 + sm * (a1 + a2)) * (double)dmax * 1.01;
     const double dt_lo = fabs(Dt) * (1.0 - 1e-6) - 256.0 * eps * sm * a1 * a2;
     if (!(dt_lo > 0.0)) degenerate = true;   // camera (numerically) in the triangle's plane
-    const double f = (double)p.focal;
+    const double f = (double)focal;
     const double h = 0.5 * fmax(fabs(PU[0]) + fabs(PU[1]), fmax(fabs(PV[0]) + fabs(PV[1]), fabs(PW[0]) + fabs(PW[1])));
     q0 = make_float4((float)PU[0], (float)PU[1], (float)(PU[2] * f), (float)PV[0]);
     q1 = make_float4((float)PV[1], (float)(PV[2] * f), (float)PW[0], (float)PW[1]);
@@ -165,11 +187,14 @@ __global__ void rt_prep_planes_kernel(const __grid_constant__ RtPrepParams p) {
     // (not proven for a ray that grazes the triangle).  256 eps (C + 2S) a1 a2 covers both with a factor
     // two; outside that band sign(D) = -sign(Dt) and |D| < |Dt| + B.  rt_ex_shadow's guards on r.r hold
     // too: |Dt| > 2B and |Dt| > 1e-3 S N2 keep |r| above 5e-4 S (S >= 1e-3), and |r|inf <= S < 1e14.
-    const double C = fmax(fabs((double)p.cam[0]), fmax(fabs((double)p.cam[1]), fabs((double)p.cam[2])));
+    // Batched views share these records: C is the largest |cam|inf of the launch's views, which only
+    // widens B, so the bound holds for the hit points of every view.
+    const double C = VIEWS ? (double)pv->cam_inf
+                           : fmax(fabs((double)p.cam[0]), fmax(fabs((double)p.cam[1]), fabs((double)p.cam[2])));
     const double B = 256.0 * eps * (C + 2.0 * S) * a1 * a2 + 1e-6 * fabs(Dt);
     const bool known = !degenerate && fabs(Dt) > 2.0 * B && fabs(Dt) + B < 1e29 && S < 1e14;
     const float dhi = __double2float_ru((fabs(Dt) + B) * (1.0 + 1e-6));
-    if (p.self_D) p.self_D[(size_t)(o - 1) * p.n_tris + i] = !known ? 0.0f : (Dt > 0.0 ? -dhi : dhi);
+    if (p.self_D) p.self_D[(size_t)l * p.n_tris + i] = !known ? 0.0f : (Dt > 0.0 ? -dhi : dhi);
     q0 = make_float4((float)PU[0], (float)PU[1], (float)PU[2], (float)PV[0]);
     q1 = make_float4((float)PV[1], (float)PV[2], (float)PW[0], (float)PW[1]);
     q2 = make_float4((float)PW[2], __double2float_ru(E), __double2float_rd(fabs(Dt) - slackT),
@@ -183,11 +208,17 @@ __global__ void rt_prep_planes_kernel(const __grid_constant__ RtPrepParams p) {
   }
   float4 *dst = p.planes + (size_t)o * p.origin_stride_f4 + (size_t)i * RT_REC_F4;
   dst[0] = q0; dst[1] = q1; dst[2] = q2;
-  if (o == 0) {
+  if (is_cam) {
     // numerator of t (skeleton.cpp:305-306): the same for every primary ray, exact float ops
-    const float sx = xsub(p.cam[0], v0[0]), sy = xsub(p.cam[1], v0[1]), sz = xsub(p.cam[2], v0[2]);
-    p.dt_cam[i] = xdet3(sx, sy, sz, g0.w, g1.x, g1.y, g1.z, g1.w, g2.x);
+    const float sx = xsub(cam[0], v0[0]), sy = xsub(cam[1], v0[1]), sz = xsub(cam[2], v0[2]);
+    p.dt_cam[(VIEWS ? (size_t)o * p.n_tris : 0) + i] = xdet3(sx, sy, sz, g0.w, g1.x, g1.y, g1.z, g1.w, g2.x);
   }
+}
+
+__global__ void rt_prep_planes_kernel(const __grid_constant__ RtPrepParams p) { rt_prep_planes_body<false>(p, nullptr); }
+// p.cam / p.focal / p.dmax unused: per view in v
+__global__ void rt_prep_planes_views_kernel(const __grid_constant__ RtPrepParams p, const __grid_constant__ RtPrepViews v) {
+  rt_prep_planes_body<true>(p, &v);
 }
 
 // ---- warp helpers -------------------------------------------------------------------

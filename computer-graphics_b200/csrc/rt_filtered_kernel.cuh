@@ -252,12 +252,28 @@ __device__ __forceinline__ void rt_grid_mark(int cell, int *table, int *cells, i
 #ifndef RT_MIN_BLOCKS
 #define RT_MIN_BLOCKS 3
 #endif
-template <bool MULTI, bool GRID>
-__global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filtered_kernel(const __grid_constant__ RtKParams p) {
+// Pixel of this thread in a batched launch: block (x, y) of whole frame blockIdx.z, warps as in rt_filtered_body.
+// The indices are read afresh (volatile): merged with the kernel's own u and v, they were kept in a spill slot.
+__device__ __forceinline__ size_t rt_views_pid(const RtKParams &p) {
+  unsigned t, bx, by, bz;
+  asm volatile("mov.u32 %0, %%tid.x;" : "=r"(t));
+  asm volatile("mov.u32 %0, %%ctaid.x;" : "=r"(bx));
+  asm volatile("mov.u32 %0, %%ctaid.y;" : "=r"(by));
+  asm volatile("mov.u32 %0, %%ctaid.z;" : "=r"(bz));
+  const int lane = t & 31, warp = t >> 5;
+  const int u = bx * 16 + (warp & 1) * 8 + (lane & 7), v = by * 16 + (warp >> 1) * 4 + (lane >> 3);
+  return ((size_t)bz * p.H + v) * p.W + u;
+}
+
+// VIEWS (scene streaming only): blockIdx.z is the view of a batched launch; its camera comes from vp, its camera
+// records and dt_cam from its own slices, its pixels go to frame blockIdx.z of the outputs.
+template <bool MULTI, bool GRID, bool VIEWS>
+__device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtViewsParams *vp) {
   // Scene streaming (GRID = false): the block shares one double-buffered ring of RT_TILE-record
   // tiles, refilled under __syncthreads.  Cell lists (GRID = true): every WARP has its own ring of
   // RT_WTILE-record tiles, its own cell set and no block barrier at all -- the lists are short,
   // and a warp on a dense or silhouette patch no longer holds the other seven back.
+  static_assert(!(GRID && VIEWS), "batched views run the scene-streaming kernel");
   constexpr int TILE = GRID ? RT_WTILE : RT_TILE;
   constexpr int NRING = GRID ? RT_THREADS / 32 : 1;
   extern __shared__ __align__(128) float4 tile_smem[];  // NRING x 2 x TILE x 3 float4 (+ GRID: NRING x 2 x TILE int)
@@ -292,8 +308,17 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
   const int block_y = by * p.il_n + p.il_r;     // 16-row block of the range (interleaved launches)
   const int v = p.row0 + block_y * 16 + (warp >> 1) * 4 + (lane >> 3);
   const bool live = (u < p.W) && (v < p.row1) && (sub < 0 || (lane & 7) == sub);
-  const size_t pid = (size_t)v * p.W + u;
+  const int view = VIEWS ? (int)blockIdx.z : 0;
+  // VIEWS: frame `view` of the outputs.  Formed again where the pixel is stored (held over the kernel, the
+  // 64-bit offset made it spill more)
+  const size_t pid = VIEWS ? 0 : (size_t)v * p.W + u;
+#define PID (VIEWS ? rt_views_pid(p) : pid)
   const size_t origin_stride = (size_t)((p.n_tris + RT_TILE - 1) / RT_TILE) * RT_TILE * RT_REC_F4;
+  const float *cam = VIEWS ? vp->view[view].cam : p.cam;
+  const float *R = VIEWS ? vp->view[view].R : p.R;
+  const float focal = VIEWS ? vp->view[view].focal : p.focal;
+  const float4 *cam_planes = VIEWS ? p.planes + (size_t)view * origin_stride : p.planes;
+  const int first_light = VIEWS ? vp->n_views : 1;    // origin of light 0's records
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < 2 * NRING; ++i) mbar_init(&bars_all[i], 1);
@@ -314,10 +339,10 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
 
   // dir = R * vec4(u - W/2, v - H/2, f, 1)   (skeleton.cpp:126-128)
   const float x = (float)(u - p.W / 2), y = (float)(v - p.H / 2);
-  const float dir0 = xadd(xadd(xmul(p.R[0], x), xmul(p.R[4], y)), xadd(xmul(p.R[8], p.focal), xmul(p.R[12], 1.0f)));
-  const float dir1 = xadd(xadd(xmul(p.R[1], x), xmul(p.R[5], y)), xadd(xmul(p.R[9], p.focal), xmul(p.R[13], 1.0f)));
-  const float dz = p.focal;
-  const float cx = p.cam[0], cy = p.cam[1], cz = p.cam[2];
+  const float dir0 = xadd(xadd(xmul(R[0], x), xmul(R[4], y)), xadd(xmul(R[8], focal), xmul(R[12], 1.0f)));
+  const float dir1 = xadd(xadd(xmul(R[1], x), xmul(R[5], y)), xadd(xmul(R[9], focal), xmul(R[13], 1.0f)));
+  const float dz = focal;
+  const float cx = cam[0], cy = cam[1], cz = cam[2];
   // the nine sample directions (:134-137): three x offsets, three y offsets
   const float dxs[3] = {xadd(dir0, xmul(0.5f, -1.0f)), xadd(dir0, xmul(0.5f, 0.0f)), xadd(dir0, xmul(0.5f, 1.0f))};
   const float dys[3] = {xadd(dir1, xmul(0.5f, -1.0f)), xadd(dir1, xmul(0.5f, 0.0f)), xadd(dir1, xmul(0.5f, 1.0f))};
@@ -365,7 +390,7 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
     const float wh0 = (0.5f * (hi0 - lo0) + 0.5f) * 1.0001f + 1e-3f;
     const float wh1 = (0.5f * (hi1 - lo1) + 0.5f) * 1.0001f + 1e-3f;
 
-    RtCursor cursor = rt_cursor_scene(p.planes, p.n_tris);   // origin 0
+    RtCursor cursor = rt_cursor_scene(cam_planes, p.n_tris);   // origin 0 (VIEWS: origin `view`)
     if (GRID) {
       if (issuer) s_cells[0] = block_y * (GRID ? p.gx : (int)gridDim.x) + bx;   // this block's own cell
       ring_sync();
@@ -443,7 +468,7 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
               if (!farther) {
                 ++n_exact;
                 b.t = HT(k); b.idx = HI(k);
-                const RtHit nb = rt_ex_primary(p.geom, p.dt_cam, cx, cy, cz, tri, m3 >= E ? 1 : 0, dx, dy, dz, LEN(k), b);
+                const RtHit nb = rt_ex_primary(p.geom, VIEWS ? p.dt_cam + (size_t)blockIdx.z * p.n_tris : p.dt_cam, cx, cy, cz, tri, m3 >= E ? 1 : 0, dx, dy, dz, LEN(k), b);
                 if (nb.idx != b.idx || nb.dist != b.dist) { HT(k) = nb.t; HD(k) = nb.dist; HI(k) = nb.idx; }
               }
             }
@@ -490,8 +515,8 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
     if (live && HD(k) < FLT_MAX) active |= 1u << k;
   if (live) {
     const bool hit4 = (active >> 4) & 1u;
-    if (p.depth) p.depth[pid] = hit4 ? HD(4) : INFINITY;
-    if (p.index) p.index[pid] = hit4 ? HI(4) : INT32_MIN;
+    if (p.depth) p.depth[PID] = hit4 ? HD(4) : INFINITY;
+    if (p.index) p.index[PID] = hit4 ? HI(4) : INT32_MIN;
   }
 
 #ifdef RT_PROFILE_CLOCK
@@ -581,7 +606,7 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
       }
     }
 
-    const float4 *src = p.planes + (size_t)(1 + l) * origin_stride;
+    const float4 *src = p.planes + (size_t)(first_light + l) * origin_stride;
     // the buffer about to be refilled last held the tile before the previous
     // phase's final one; every thread left it at that phase's last barrier
     ring_sync();
@@ -859,7 +884,7 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
       }
     }
     const float pix[3] = {PIX(0), PIX(1), PIX(2)};
-    rt_store_pixel(p, pid, active != 0, pix);
+    rt_store_pixel(p, PID, active != 0, pix);
   }
   rt_count(p.counters + 0, (unsigned long long)__popc(active) * p.n_lights);
   rt_count(p.counters + 1, (unsigned long long)n_exact);
@@ -869,16 +894,27 @@ __global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filte
   if (live) for (int i = 0; i < 6; ++i) atomicAdd(p.counters + 2 + i, (unsigned long long)prof_cnt[i + (i >= 2 ? 1 : 0)]);
   if (live) { atomicAdd(p.counters + 8, (unsigned long long)prof_cnt[8]); atomicAdd(p.counters + 14, (unsigned long long)prof_cnt[7]); }
   // diagnostic build only: the depth plane carries this pixel's shadow L1 test count, the index plane its exact evaluations
-  if (live && p.depth) p.depth[pid] = (float)prof_cnt[3];
-  if (live && p.index) p.index[pid] = (int)n_exact;
+  if (live && p.depth) p.depth[PID] = (float)prof_cnt[3];
+  if (live && p.index) p.index[PID] = (int)n_exact;
 #endif
 #ifdef RT_PROFILE_CLOCK
   // depth plane: cycles of this warp; index plane: records its shadow phases streamed (low 20 bits), cells walked (high bits);
   // rgb plane: shadow-phase L0 survivors this lane tested, candidates it kept, exact evaluations
-  if (live && p.depth) p.depth[pid] = (float)(clock64() - prof_t0);
-  if (live && p.index) p.index[pid] = (int)(min(prof_recs, 0xfffffu) | (min(prof_cells, 2047u) << 20));
-  if (live && p.rgb) { p.rgb[3 * pid] = (float)prof_l1; p.rgb[3 * pid + 1] = (float)prof_l2; p.rgb[3 * pid + 2] = (float)(n_exact - prof_ex0); }
+  if (live && p.depth) p.depth[PID] = (float)(clock64() - prof_t0);
+  if (live && p.index) p.index[PID] = (int)(min(prof_recs, 0xfffffu) | (min(prof_cells, 2047u) << 20));
+  if (live && p.rgb) { p.rgb[3 * PID] = (float)prof_l1; p.rgb[3 * PID + 1] = (float)prof_l2; p.rgb[3 * PID + 2] = (float)(n_exact - prof_ex0); }
 #endif
+}
+
+template <bool MULTI, bool GRID>
+__global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS) rt_filtered_kernel(const __grid_constant__ RtKParams p) {
+  rt_filtered_body<MULTI, GRID, false>(p, nullptr);
+}
+// Batched views: grid (x, y) = the 16x16 pixel blocks of one whole frame, z = view; p.row0 = 0, p.row1 = H, no interleave.
+template <bool MULTI>
+__global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_filtered_views_kernel(const __grid_constant__ RtKParams p,
+                                                                                      const __grid_constant__ RtViewsParams v) {
+  rt_filtered_body<MULTI, false, true>(p, &v);
 }
 
 int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p);

@@ -158,9 +158,8 @@ int rt_prepare_scene(b200_ctx *ctx) {
   return B200_OK;
 }
 
-int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int32_t *d_index,
-              uint32_t *d_argb) {
-  RtKParams p;
+static void rt_kparams(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int32_t *d_index,
+                       uint32_t *d_argb, RtKParams &p) {
   memset(&p, 0, sizeof p);
   memcpy(p.cam, f.cam, sizeof p.cam);
   p.focal = f.focal;
@@ -175,6 +174,12 @@ int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int
   p.n_tris = ctx->rt_n_tris; p.n_sph = ctx->rt_n_spheres;
   p.rgb = d_rgb; p.depth = d_depth; p.index = d_index; p.argb = d_argb;
   p.counters = (unsigned long long *)ctx->counters.p;
+}
+
+int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int32_t *d_index,
+              uint32_t *d_argb) {
+  RtKParams p;
+  rt_kparams(ctx, f, d_rgb, d_depth, d_index, d_argb, p);
   const int rows = f.row1 - f.row0;
   if (rows <= 0 || f.W <= 0) return B200_OK;
   p.blocks_y = (rows + 15) / 16;
@@ -192,6 +197,61 @@ int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int
 
 // scenes this large get direction grids (declared in common.cuh; measured crossover at 4K: ~800 triangles)
 constexpr unsigned long long RT_GRID_MAX_ENTRIES = 1ull << 26;   // 64 Mi list entries = 3.25 GiB
+
+// Upper bound of |d|inf over the primary rays of rows [row0, row1): dir.x / dir.y are affine in (u, v),
+// extremes at the corners.
+static float rt_cam_dmax(const RtFrame &f) {
+  float dmax = fabsf(f.focal);
+  const int us[2] = {0, f.W - 1}, vs[2] = {f.row0, f.row1 - 1};
+  for (int a = 0; a < 2; ++a)
+    for (int b = 0; b < 2; ++b) {
+      const float x = (float)(us[a] - f.W / 2), y = (float)(vs[b] - f.H / 2);
+      for (int r = 0; r < 2; ++r) {
+        const float d = f.R[0 + r] * x + f.R[4 + r] * y + f.R[8 + r] * f.focal + f.R[12 + r];
+        dmax = fmaxf(dmax, fabsf(d) + 0.5f);
+      }
+    }
+  return dmax * 1.001f + 1.0f;
+}
+
+// The camera-independent part of the plane-record preparation: scene, lights, shadow-ray bounds, buffers.
+static void rt_prep_common(b200_ctx *ctx, const RtFrame &f, size_t origin_stride, const float *self_D, RtPrepParams &q) {
+  q.geom = (const float4 *)ctx->rt_geom.p;
+  q.n_tris = ctx->rt_n_tris;
+  // world_S bounds |start - v0|inf of SHADOW rays (the camera's own plane records use the exact
+  // |camera - v0|): their starts are hit points, which lie on the scene's geometry, so the camera
+  // position does not enter (it tripled S, and with it the filter's margin, on the Cornell box)
+  float m = ctx->rt_world_abs;
+  q.n_lights = f.n_lights;
+  for (int l = 0; l < f.n_lights; ++l)
+    for (int k = 0; k < 3; ++k) {
+      q.lights[l][k] = f.lights[l][k];
+      m = fmaxf(m, fabsf(f.lights[l][k]));
+    }
+  q.world_S = 2.0f * m * 1.001f + 1e-3f;
+  q.n_scale = ctx->rt_normal_abs;
+  q.planes = (float4 *)ctx->rt_planes.p;
+  q.origin_stride_f4 = origin_stride;
+  q.dt_cam = (float *)ctx->rt_dtcam.p;
+  q.self_D = (float *)self_D;   // null: a grid frame (a grid frame that falls back to streaming decides every self pair exactly)
+}
+
+// per thread: t, distance, index of the nine samples; the scene-streaming kernel also their ray lengths and the colour sum
+constexpr size_t RT_HIT_SMEM = 27 * (size_t)RT_THREADS * sizeof(float);
+constexpr size_t RT_STREAM_SMEM = 2 * (size_t)RT_TILE * RT_REC_F4 * sizeof(float4) + RT_HIT_SMEM + 12 * (size_t)RT_THREADS * sizeof(float);
+
+static int rt_set_smem_limits(b200_ctx *ctx) {
+  if (ctx->rt_grid_smem_set) return B200_OK;      // per context: function attributes are per device
+  const size_t most = (size_t)(RT_THREADS / 32) * 2 * RT_WTILE * (RT_REC_F4 * sizeof(float4) + sizeof(int)) + RT_HIT_SMEM;
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)most));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)most));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_views_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_views_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
+  ctx->rt_grid_smem_set = 1;
+  return B200_OK;
+}
 
 int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
   const int n = ctx->rt_n_tris;
@@ -212,38 +272,10 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
 
   if (n > 0) {
     RtPrepParams q;
-    q.geom = (const float4 *)ctx->rt_geom.p;
-    q.n_tris = n;
+    rt_prep_common(ctx, f, origin_stride, p.self_D, q);
     q.cam[0] = f.cam[0]; q.cam[1] = f.cam[1]; q.cam[2] = f.cam[2];
     q.focal = f.focal;
-    // |d|inf over the band: dir.x / dir.y are affine in (u, v), extremes at the corners
-    float dmax = fabsf(f.focal);
-    const int us[2] = {0, f.W - 1}, vs[2] = {f.row0, f.row1 - 1};
-    for (int a = 0; a < 2; ++a)
-      for (int b = 0; b < 2; ++b) {
-        const float x = (float)(us[a] - f.W / 2), y = (float)(vs[b] - f.H / 2);
-        for (int r = 0; r < 2; ++r) {
-          const float d = f.R[0 + r] * x + f.R[4 + r] * y + f.R[8 + r] * f.focal + f.R[12 + r];
-          dmax = fmaxf(dmax, fabsf(d) + 0.5f);
-        }
-      }
-    q.dmax = dmax * 1.001f + 1.0f;
-    // world_S bounds |start - v0|inf of SHADOW rays (the camera's own plane records use the exact
-    // |camera - v0|): their starts are hit points, which lie on the scene's geometry, so the camera
-    // position does not enter (it tripled S, and with it the filter's margin, on the Cornell box)
-    float m = ctx->rt_world_abs;
-    q.n_lights = f.n_lights;
-    for (int l = 0; l < f.n_lights; ++l)
-      for (int k = 0; k < 3; ++k) {
-        q.lights[l][k] = f.lights[l][k];
-        m = fmaxf(m, fabsf(f.lights[l][k]));
-      }
-    q.world_S = 2.0f * m * 1.001f + 1e-3f;
-    q.n_scale = ctx->rt_normal_abs;
-    q.planes = (float4 *)ctx->rt_planes.p;
-    q.origin_stride_f4 = origin_stride;
-    q.dt_cam = (float *)ctx->rt_dtcam.p;
-    q.self_D = (float *)p.self_D;   // null: a grid frame (a grid frame that falls back to streaming decides every self pair exactly)
+    q.dmax = rt_cam_dmax(f);   // over the band
     dim3 grid((n + 127) / 128, 1 + f.n_lights);
     rt_prep_planes_kernel<<<grid, 128, 0, ctx->stream>>>(q);
     ctx->stats.kernel_launches++;
@@ -252,9 +284,7 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
 
   const int my_blocks = (p.blocks_y - p.il_r + p.il_n - 1) / p.il_n;
   dim3 grid((f.W + 15) / 16, my_blocks);
-  // per thread: t, distance, index of the nine samples; the scene-streaming kernel also their ray lengths and the colour sum
-  const size_t hit_smem = 27 * (size_t)RT_THREADS * sizeof(float);
-  const size_t smem = 2 * (size_t)RT_TILE * RT_REC_F4 * sizeof(float4) + hit_smem + 12 * (size_t)RT_THREADS * sizeof(float);
+  const size_t hit_smem = RT_HIT_SMEM, smem = RT_STREAM_SMEM;
 
   if (use_grid) {
     const size_t cells = (size_t)grid.x * p.blocks_y + (size_t)f.n_lights * 6 * RT_GRID_FACE;   // camera cells: every block of the range
@@ -319,14 +349,7 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
     }
   }
 
-  if (!ctx->rt_grid_smem_set) {      // per context: function attributes are per device
-    const size_t most = (size_t)(RT_THREADS / 32) * 2 * RT_WTILE * (RT_REC_F4 * sizeof(float4) + sizeof(int)) + hit_smem;
-    CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)most));
-    CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)most));
-    CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ctx->rt_grid_smem_set = 1;
-  }
+  if (int rc = rt_set_smem_limits(ctx)) return rc;
   if (use_grid) {
     // one private double-buffered ring per warp: records + triangle indices
     const size_t gsmem = (size_t)(RT_THREADS / 32) * 2 * RT_WTILE * (RT_REC_F4 * sizeof(float4) + sizeof(int)) + hit_smem;
@@ -371,6 +394,89 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
   }
   ctx->stats.kernel_launches++;
   CU_CHECK(ctx, cudaGetLastError());
+  return B200_OK;
+}
+
+// Whole frames of n_views cameras (same W, H, lights) into outputs that hold the frames back to back.  Scenes
+// for the scene-streaming kernel render up to RT_VIEWS_MAX views per launch: one preparation launch makes each
+// view's camera records and the shared light records, one render launch covers every view (blockIdx.z).  So
+// the per-view buffers are sized for RT_VIEWS_MAX views whatever n_views.  Gridded scenes and the brute-force
+// kernel render view by view: their grids are per camera.  So does a single view: the same frame through the
+// single-view kernels, without the batch's 5 KB of launch parameters (measured 5 % slower at 320x256).
+int rt_launch_views(b200_ctx *ctx, const RtFrame *fs, int n_views, float *d_rgb, float *d_depth, int32_t *d_index,
+                    uint32_t *d_argb) {
+  const RtFrame &f = fs[0];
+  const size_t npix = (size_t)f.W * f.H;
+  const int n = ctx->rt_n_tris;
+  const bool use_grid = n > 0 && (ctx->opt_rt_grid == 1 || (ctx->opt_rt_grid == 0 && n >= RT_GRID_AUTO_TRIS));
+  if (ctx->opt_rt_bruteforce || use_grid || n_views == 1) {
+    for (int k = 0; k < n_views; ++k) {
+      const size_t o = (size_t)k * npix;
+      if (int rc = rt_launch(ctx, fs[k], d_rgb ? d_rgb + 3 * o : nullptr, d_depth ? d_depth + o : nullptr,
+                             d_index ? d_index + o : nullptr, d_argb ? d_argb + o : nullptr))
+        return rc;
+    }
+    return B200_OK;
+  }
+  if (npix == 0) return B200_OK;
+  RtKParams p;
+  rt_kparams(ctx, f, nullptr, nullptr, nullptr, nullptr, p);
+  p.row0 = 0; p.row1 = f.H; p.il_n = 1; p.il_r = 0;
+  p.blocks_y = (f.H + 15) / 16;
+  const int per = n_views < RT_VIEWS_MAX ? n_views : RT_VIEWS_MAX;
+  const size_t origin_stride = (size_t)((n + RT_TILE - 1) / RT_TILE) * RT_TILE * RT_REC_F4;
+  if (int rc = ensure(ctx, ctx->rt_planes, sizeof(float4) * (origin_stride * (per + f.n_lights) + 1))) return rc;
+  if (int rc = ensure(ctx, ctx->rt_dtcam, sizeof(float) * (size_t)(n > 0 ? n : 1) * per)) return rc;
+  if (int rc = ensure(ctx, ctx->rt_selfD, sizeof(float) * (size_t)(n > 0 ? n : 1) * (f.n_lights > 0 ? f.n_lights : 1))) return rc;
+  p.planes = (const float4 *)ctx->rt_planes.p;
+  p.dt_cam = (const float *)ctx->rt_dtcam.p;
+  p.self_D = (const float *)ctx->rt_selfD.p;
+  if (int rc = rt_set_smem_limits(ctx)) return rc;
+
+  for (int k0 = 0; k0 < n_views; k0 += RT_VIEWS_MAX) {
+    const int nv = n_views - k0 < RT_VIEWS_MAX ? n_views - k0 : RT_VIEWS_MAX;
+    RtViewsParams v;
+    memset(&v, 0, sizeof v);
+    v.n_views = nv;
+    for (int j = 0; j < nv; ++j) {
+      const RtFrame &fj = fs[k0 + j];
+      memcpy(v.view[j].cam, fj.cam, sizeof v.view[j].cam);
+      v.view[j].focal = fj.focal;
+      memcpy(v.view[j].R, fj.R, sizeof v.view[j].R);
+    }
+    if (n > 0) {
+      RtPrepParams q;
+      rt_prep_common(ctx, f, origin_stride, p.self_D, q);
+      q.cam[0] = q.cam[1] = q.cam[2] = 0.f; q.focal = 0.f; q.dmax = 0.f;   // per view, below
+      RtPrepViews pv;
+      memset(&pv, 0, sizeof pv);
+      pv.n_views = nv;
+      for (int j = 0; j < nv; ++j) {
+        const RtFrame &fj = fs[k0 + j];
+        for (int k = 0; k < 3; ++k) {
+          pv.cam[j][k] = fj.cam[k];
+          pv.cam_inf = fmaxf(pv.cam_inf, fabsf(fj.cam[k]));
+        }
+        pv.cam[j][3] = fj.focal;
+        pv.dmax[j] = rt_cam_dmax(fj);
+      }
+      rt_prep_planes_views_kernel<<<dim3((n + 127) / 128, nv + f.n_lights), 128, 0, ctx->stream>>>(q, pv);
+      ctx->stats.kernel_launches++;
+      CU_CHECK(ctx, cudaGetLastError());
+    }
+    const size_t o = (size_t)k0 * npix;
+    p.rgb = d_rgb ? d_rgb + 3 * o : nullptr;
+    p.depth = d_depth ? d_depth + o : nullptr;
+    p.index = d_index ? d_index + o : nullptr;
+    p.argb = d_argb ? d_argb + o : nullptr;
+    const dim3 grid((f.W + 15) / 16, p.blocks_y, nv);
+    if (f.n_lights > 1)
+      rt_filtered_views_kernel<true><<<grid, RT_THREADS, RT_STREAM_SMEM, ctx->stream>>>(p, v);
+    else
+      rt_filtered_views_kernel<false><<<grid, RT_THREADS, RT_STREAM_SMEM, ctx->stream>>>(p, v);
+    ctx->stats.kernel_launches++;
+    CU_CHECK(ctx, cudaGetLastError());
+  }
   return B200_OK;
 }
 

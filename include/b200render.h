@@ -247,6 +247,35 @@ int rt_render_device(b200_ctx *ctx, const camera_t *cam, const light_t *lights, 
                      int row_begin, int row_end, float *d_rgb, float *d_depth,
                      int32_t *d_index, uint32_t *d_argb);
 
+/* ---- RT, batched views: many cameras of one scene in one call ----------------
+ * n_views cameras (same width and height, any pos / focal / R) of one scene and one set of lights.
+ * Outputs hold n_views whole frames back to back: view k's pixel (x, y) is at
+ * k*W*H + y*W + x (rgb: times 3).  Each frame is bit-identical to render_raytrace /
+ * draw_raytrace / rt_render_device with cams[k].  Any output of render_raytrace_views and
+ * rt_render_views_device may be NULL; draw_raytrace_views needs argb_out.
+ *   - n_views >= 1, cams non-null, every camera a valid resolution and the same W, H as
+ *     cams[0]; at most 8 lights (non-null when n_lights > 0): otherwise B200_EINVAL.
+ *   - Whole frames only: no row band, and B200_OPT_RT_INTERLEAVE_N / _R do not apply.
+ *   - Scenes that take the scene-streaming kernel (fewer than 1024 triangles, or
+ *     B200_OPT_RT_GRID = 2) render up to 64 views in one launch; larger batches take several
+ *     launches inside the call, and the per-view device buffers stay sized for 64 views.
+ *     Gridded scenes, B200_OPT_RT_BRUTEFORCE = 1 and a batch of one view render view by view.
+ *   - b200_get_stats afterwards: primary_rays = n_views * W * H * 9, shadow_rays and
+ *     exact_evals summed over the views, gpu_ms the device time of the whole call.
+ *   - On a b200_init_multi context the host-pointer entries give each device a contiguous run
+ *     of whole views; rt_render_views_device is per device (B200_EINVAL there). */
+int render_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres,
+                          int n_spheres, const camera_t *cams, int n_views, const light_t *lights,
+                          int n_lights, float *rgb_out, float *depth_out, int32_t *index_out);
+int draw_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres,
+                        int n_spheres, const camera_t *cams, int n_views, const light_t *lights,
+                        int n_lights, uint32_t *argb_out);
+/* Device-resident: the scene of rt_upload_scene, DEVICE output pointers (n_views * W * H pixels
+ * each), asynchronous on b200_stream(ctx). */
+int rt_render_views_device(b200_ctx *ctx, const camera_t *cams, int n_views, const light_t *lights,
+                           int n_lights, float *d_rgb, float *d_depth, int32_t *d_index,
+                           uint32_t *d_argb);
+
 /* ---- RAST: replaces rasteriser Draw(screen*) (skeleton.cpp:203-308) --------*/
 
 /* Tier 1: the triangle loop + post pass (skeleton.cpp:243-307) on an
