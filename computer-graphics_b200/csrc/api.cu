@@ -102,7 +102,7 @@ void b200_destroy(b200_ctx *ctx) {
   cudaStreamSynchronize(ctx->stream);
   DevBuf *bufs[] = {&ctx->rt_src, &ctx->rt_geom, &ctx->rt_spheres, &ctx->rt_planes, &ctx->rt_dtcam, &ctx->rt_selfD, &ctx->rt_bounds, &ctx->rt_cells, &ctx->rt_cell_rec, &ctx->rt_cell_idx, &ctx->rast_src,
                     &ctx->rast_setup, &ctx->rast_rowsA, &ctx->rast_rowsB, &ctx->rast_bins, &ctx->rast_tile_count, &ctx->rast_tile_bits,
-                    &ctx->rast_tmp, &ctx->rast_keys, &ctx->rast_trimeta, &ctx->rast_big, &ctx->rast_orig, &ctx->rast_shadow8, &ctx->rast_srowsB, &ctx->rast_srowsL, &ctx->rast_chunks, &ctx->rast_world, &ctx->rast_geom_tmp, &ctx->rast_screen, &ctx->rast_low, &ctx->rast_high, &ctx->rast_shadow,
+                    &ctx->rast_tmp, &ctx->rast_keys, &ctx->rast_trimeta, &ctx->rast_big, &ctx->rast_orig, &ctx->rast_shadow8, &ctx->rast_srowsB, &ctx->rast_srowsL, &ctx->rast_row_owner, &ctx->rast_world, &ctx->rast_geom_tmp, &ctx->rast_screen, &ctx->rast_low, &ctx->rast_high, &ctx->rast_shadow,
                     &ctx->rast_depth, &ctx->rast_index, &ctx->out_rgb, &ctx->out_depth, &ctx->out_index,
                     &ctx->out_argb, &ctx->counters, &ctx->rt_plan, &ctx->rt_cell_pairs, &ctx->rast_tex_images, &ctx->rast_tex_noise,
                     &ctx->rast_colour_keys, &ctx->rast_colour_rgb, &ctx->rast_colour_tmp};
@@ -448,7 +448,7 @@ static int finish_stats(b200_ctx *ctx) {
     // what this frame needed sizes the next pipelined frame of the same shape
     b200_ctx::RastSpec &sp = ctx->rast_spec;
     sp.tris = (unsigned long long)ctx->rast_n_tris;
-    sp.chunks = c[6]; sp.rows = c[4]; sp.bins = c[3]; sp.big = c[10];
+    sp.rows = c[4]; sp.bins = c[3]; sp.big = c[10];
     sp.has_shadow = ctx->rast_has_shadow;
     sp.valid = 1;
   }
@@ -696,7 +696,9 @@ static int rast_frame(b200_ctx *ctx, bool whole_draw, const camera_t *cam, const
   tl_mark(ctx, "frame start");
   rast_light_t lc = *light;
   ctx->rast_clear_ptr = nullptr; ctx->rast_keys_cleared = 0; ctx->rast_cull_on = 0; ctx->rast_geom_chunks = 1;
-  const bool to_scatter = ctx->opt_rast_path == 2 || (ctx->opt_rast_path == 0 && !ctx->rast_has_shadow && !ctx->rast_tex_on && !ctx->opt_rast_colour);
+  // the path rast_launch will take, for the list bound a pipelined geometry stage writes under (that stage also
+  // caps it at 2^30 - 1, which is past the scatter path's limit either way)
+  const bool to_scatter = rast_scatter_path(ctx, whole_draw ? (long long)rast_spec_cap(sp.tris) : (long long)ctx->rast_n_tris);
   if (ctx->rast_up_chunks > 1) {
     if (spec && whole_draw && to_scatter) {
       ctx->rast_geom_chunks = ctx->rast_up_chunks;   // the frame consumes the upload chunk by chunk
@@ -718,9 +720,7 @@ static int rast_frame(b200_ctx *ctx, bool whole_draw, const camera_t *cam, const
       }
       // ... and, asked to, keeps only the triangles that reach the band's rows.  (Not when the entry
       // value of the indirect light is in play: its one fragment is found on the complete list.)
-      const float steady = 0.2f * 1.0f;
-      const bool quirk = memcmp(&light->indirect[0], &steady, 4) || memcmp(&light->indirect[1], &steady, 4) || memcmp(&light->indirect[2], &steady, 4);
-      if (ctx->opt_rast_band_cull && !quirk && (fb0 > 0 || fb1 < cam->height)) {
+      if (ctx->opt_rast_band_cull && !rast_indirect_entry_differs(light) && (fb0 > 0 || fb1 < cam->height)) {
         ctx->rast_cull_on = 1; ctx->rast_cull0 = fb0; ctx->rast_cull1 = fb1;
       }
     }

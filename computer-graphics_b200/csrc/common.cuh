@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <string.h>
 #include <string>
 #include <vector>
 
@@ -167,7 +168,7 @@ struct b200_ctx {
   int opt_rast_colour = 0;   // B200_OPT_RAST_COLOUR_MODE: randColourSelect (0, 1 random colours, 2 night vision)
   DevBuf rast_colour_keys, rast_colour_rgb, rast_colour_tmp;
   int opt_rast_path = 0;     // 0 auto, 1 ordered tiles, 2 scatter (shadow-free lists only)
-  DevBuf rast_chunks;    // owner triangle of each 8-row chunk of the row tables
+  DevBuf rast_row_owner;   // per slot of the row tables: the triangle that owns it (RastParams::row_owner)
   DevBuf rast_world;     // tier 2: world-space room then boxes, as uploaded
   DevBuf rast_geom_tmp;  // tier 2: per-triangle output counts and their scan
   int rast_n_room = 0, rast_n_boxes = 0;
@@ -181,7 +182,7 @@ struct b200_ctx {
   int opt_rast_pipelined = 0;
   struct RastSpec {
     int valid = 0, has_shadow = 0, n_room = 0, n_boxes = 0, n_list = 0, W = 0, H = 0, row0 = 0, row1 = 0, fast = 0, ts = 0, whole_draw = 0, cull = 0;
-    unsigned long long tris = 0, chunks = 0, rows = 0, bins = 0, big = 0;
+    unsigned long long tris = 0, rows = 0, bins = 0, big = 0;
   } rast_spec;
   struct RastInflight {
     int active = 0, whole_draw = 0, fast = 0;
@@ -233,7 +234,17 @@ int rast_launch(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, i
                 float *d_rgb, float *d_depth, int32_t *d_index, uint32_t *d_argb, bool spec);
 int rast_geometry(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, rast_light_t *light_out,
                   bool spec);
+// true: the frame takes the scatter path, false: ordered screen tiles (n: the list length or a bound on it)
+bool rast_scatter_path(const b200_ctx *ctx, long long n);
 static inline unsigned long long rast_spec_cap(unsigned long long seen) { return seen + seen / 32 + 1024; }   // +3 %
+// PixelShader leaves indirectLightPowerPerArea at 0.2 (:585): whether a Draw is entered with another value, which
+// then reaches its first shaded fragment
+static inline bool rast_indirect_entry_differs(const rast_light_t *light) {
+  const float steady = 0.2f * 1.0f;
+  for (int k = 0; k < 3; ++k)
+    if (memcmp(&light->indirect[k], &steady, sizeof steady)) return true;
+  return false;
+}
 int scan_exclusive(b200_ctx *ctx, const unsigned *counts, unsigned *offs, int n, unsigned *tmp,
                    unsigned long long *total_out);   // rast_geom.cu; tmp: n / 4096 + 2 words
 int rt_prepare_scene(b200_ctx *ctx);

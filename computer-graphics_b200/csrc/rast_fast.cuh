@@ -260,15 +260,15 @@ __global__ void __launch_bounds__(S2_THREADS) rast_scatter2_kernel(const __grid_
 }
 
 // ---- big triangles -----------------------------------------------------------------------
-// Setup record, row space and row chunks (the work items of rast_scatter_kernel) of every
-// triangle rast_scatter2_kernel put on the big list.
+// Setup record, row space and the owners of its row slots (the work items of rast_scatter_kernel)
+// of every triangle rast_scatter2_kernel put on the big list.
 __global__ void __launch_bounds__(128) rast_setup_big_kernel(const __grid_constant__ RastParams p) {
   const unsigned k = blockIdx.x * blockDim.x + threadIdx.x;
   const int lane = threadIdx.x & 31;
   const unsigned n_big = (unsigned)min((unsigned long long)p.big_cap, p.counters[10]);
   int nrows = 0, t = 0;
   RastSetup s;
-  s.flags = 0; s.ymin = 0; s.row0 = 0; s.nrows = 0; s.row_off = 0; s.chunk_off = 0; s.tri = 0;
+  s.flags = 0; s.ymin = 0; s.row0 = 0; s.nrows = 0; s.row_off = 0; s.tri = 0;
   if (k < n_big) {
     t = p.big_list[k];
     rast_tri_setup(reinterpret_cast<const float *>(p.src + t), p.focal, p.W, p.H, s);   // ok: rast_scatter2_kernel checked
@@ -286,42 +286,37 @@ __global__ void __launch_bounds__(128) rast_setup_big_kernel(const __grid_consta
     if (lane >= o) incl += n;
   }
   const unsigned total = __shfl_sync(0xffffffffu, incl, 31);
-  unsigned base = 0, cbase = 0;
-  if (lane == 31 && total) {
-    base = (unsigned)atomicAdd(p.counters + 4, (unsigned long long)total);
-    cbase = (unsigned)atomicAdd(p.counters + 6, (unsigned long long)total);   // one row per chunk
-  }
+  unsigned base = 0;
+  if (lane == 31 && total) base = (unsigned)atomicAdd(p.counters + 4, (unsigned long long)total);
   base = __shfl_sync(0xffffffffu, base, 31);
-  cbase = __shfl_sync(0xffffffffu, cbase, 31);
   s.row_off = base + incl - (unsigned)nrows;
-  s.chunk_off = cbase + incl - (unsigned)nrows;
-  if (k < n_big && (s.row_off + (unsigned)nrows > p.row_cap || s.chunk_off + (unsigned)nrows > p.chunk_cap)) {
+  if (k < n_big && s.row_off + (unsigned)nrows > p.row_cap) {
     s.nrows = 0; nrows = 0;
     atomicExch(p.counters + 5, 1ull);
   }
-  warp_spread(nrows, (int)s.chunk_off, 0, 0, (int)k, [&](int j, int x0, int, int, int owner) { p.chunk_owner[(unsigned)x0 + j] = owner; });
+  warp_spread(nrows, (int)s.row_off, 0, 0, (int)k, [&](int j, int x0, int, int, int owner) { p.row_owner[(unsigned)x0 + j] = owner; });
   if (k < n_big) {
     p.setup[k] = s;
     if (nrows > 0) p.trimeta[t] = make_int2((int)s.row_off, s.row0);
   }
 }
 
-// One thread per (big triangle,row): closed-form row record, slim copy for the resolve pass,
-// the span's fragments.
+// One thread per row slot of the big triangles: closed-form row record, slim copy for the resolve
+// pass, the span's fragments.
 __global__ void rast_scatter_kernel(const __grid_constant__ RastParams p) {
-  const unsigned chunk = blockIdx.x * blockDim.x + threadIdx.x;
+  const unsigned slot = blockIdx.x * blockDim.x + threadIdx.x;
   unsigned long long n_frag = 0;
-  if (chunk < rast_count_chunks(p)) {
-    const unsigned k = min((unsigned)p.chunk_owner[chunk], p.big_cap ? p.big_cap - 1 : 0u);   // stale owner after an overflow
+  if (slot < rast_count_rows(p)) {
+    const unsigned k = min((unsigned)p.row_owner[slot], p.big_cap ? p.big_cap - 1 : 0u);   // stale owner after an overflow
     const RastSetup &s = p.setup[k];
-    const int r = (int)(chunk - s.chunk_off);
+    const int r = (int)(slot - s.row_off);
     if (r >= 0 && r < s.nrows) {
       const int y = s.row0 + r;
       float4 A, B;
       rast_row_record<true>(s, y, A, B);
       const int lx = __float_as_int(A.x), rx = __float_as_int(A.y);
-      __stcs(p.rowsB + s.row_off + r, B);
-      __stcs(p.rowsL + s.row_off + r, lx);
+      __stcs(p.rowsB + slot, B);
+      __stcs(p.rowsL + slot, lx);
       const int x0 = max(lx, 0), x1 = min(rx, p.W);      // right end excluded (:504); bounds (:573)
       rast_span_scatter(p.keys + (size_t)y * p.W, lx, x0, x1, A.z, A.w, ((unsigned)s.tri << 5) | RAST_CODE_BIG, l2_policy_evict_last());
       n_frag = x1 > x0 ? (unsigned long long)(x1 - x0) : 0ull;

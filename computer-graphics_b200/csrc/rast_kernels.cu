@@ -20,13 +20,18 @@
 // sample wins" rule is then replayed on at most six samples.
 //
 // Kernels per frame:
-//   rast_setup_kernel  per triangle: VertexShader, row range, row-table space,
-//                      tile counts
-//   rast_rows_kernel   per (triangle,row): left/right span ends + steps
-//   rast_scan_kernel   exclusive scan of tile counts
-//   rast_spread_kernel per triangle fan-out: row chunks, tile counts, tile lists (atomics)
-//   rast_fill_kernel   per tile: sort list, depth/shadow fold, deferred shading
-//   rast_post_kernel   shadow softening + 5-tap AA + "HDR" mean (:283-307)
+//   rast_short_kernel   per triangle of a list of at most 2048: setup record, row records
+//                       and the bits of the tiles it touches, in one launch
+//   rast_setup_kernel   per triangle of a longer list: VertexShader, row range,
+//                       row-table space (and, above 8192 triangles, the owners of its rows)
+//   rast_spread_kernel  per triangle fan-out: owners of its row slots, tile counts,
+//                       tile lists (atomics)
+//   rast_scan_kernel    exclusive scan of tile counts
+//   rast_rows_kernel    per row slot: left/right span ends + steps
+//   rast_fill_kernel    per tile: sort list, depth/shadow fold, deferred shading
+//   rast_resolve_kernel per 32x8 pixels (rast_fast.cuh): shading of the winners, shadow
+//                       softening + 5-tap AA + "HDR" mean (:283-307)
+//   rast_post_kernel    the same post pass from the six intermediate buffers
 #include "common.cuh"
 #include <limits.h>
 #include <stdlib.h>
@@ -35,28 +40,28 @@
 
 constexpr int RAST_LIST_CAP = 2048;   // tile list entries sorted in shared memory
 constexpr int RAST_BATCH = 32;        // triangles per shared-memory row batch
-constexpr int RAST_CHUNK_LOG2 = 0;    // rows per work item of the per-row kernels (2^k consecutive rows of one triangle)
-constexpr int RAST_CHUNK = 1 << RAST_CHUNK_LOG2;
 
 struct RastVtx {
   int x, y;
   float zinv, px, py;
 };
 
-struct RastSetup {   // 160 bytes
+struct RastSetup {
   RastVtx v[3];
   int ymin;          // smallest vertex y (row 0 of the reference's row table)
   int row0;          // first stored row (clamped to the band being rendered)
   int nrows;         // stored rows (0: nothing to draw)
   unsigned row_off;  // index of the first stored row in the row arrays
   int flags;         // bit0: shadow-volume triangle (colour.x < 0)
-  unsigned chunk_off;  // first row chunk of this triangle in chunk_owner
   // Interpolate's per-edge steps for edge e = v[e] -> v[(e+1)%3] with
   // N = max(|dx|,|dy|)+1 samples (:533-538): they depend on the edge only
   float sx[3], sy[3], sz[3], spx[3], spy[3];
   int tri;           // scatter path: list index of this (big) triangle; setup records are indexed by big-list position
-  float pad[3];
+  float pad[4];
 };
+// 40 words: rast_setup_kernel's shared-memory staging (record stride 41, conflict-free) and rast_short_kernel's
+// word stream (lane k: words k and k + 32) are laid out for that size
+static_assert(sizeof(RastSetup) == 160, "RastSetup is 160 bytes");
 
 struct RastParams {
   int W, H;
@@ -77,7 +82,6 @@ struct RastParams {
   float4 *rowsA;     // lx, rx (bit-cast ints), left zinv, zinv step (ordered path only)
   float4 *rowsB;     // left px*zinv, its step, left py*zinv, its step
   unsigned row_cap;
-  int fast;          // shadow-free list: scatter/resolve path (rast_fast.cuh)
   unsigned long long *keys;   // fast path: per-pixel (zinv bits, triangle + 1)
   int *rowsL;        // fast path: left x of every stored row (big triangles; rowsB likewise)
   float4 *srowsB;    // fast path, small triangles: row records at triangle * S2_ROWS + y mod S2_ROWS
@@ -88,12 +92,12 @@ struct RastParams {
   const int *orig;   // band-culled list: index of every triangle in the complete list (null: the list is complete)
   int *big_list;     // fast path: triangles too large for rast_scatter2_kernel's shared-memory row table
   unsigned big_cap;
-  int *chunk_owner;  // triangle (fast path: big-list position) owning each RAST_CHUNK-row chunk
-  unsigned chunk_cap, n_chunks;
-  // pipelined mode: the list length / chunk count are not known on the host yet; n_tris and
-  // n_chunks above are then launch bounds and the kernels clamp to these device values
-  const unsigned long long *n_tris_dev, *n_chunks_dev;
-  int spread_in_setup;   // long lists: rast_setup_kernel hands the row chunks out itself (no rast_spread_kernel<0>)
+  int *row_owner;    // per slot of the row tables: the triangle (fast path: big-list position) that owns it
+  unsigned n_rows;   // row slots claimed
+  // pipelined mode: the list length / row count are not known on the host yet; n_tris and
+  // n_rows above are then launch bounds and the kernels clamp to these device values
+  const unsigned long long *n_tris_dev, *n_rows_dev;
+  int spread_in_setup;   // long lists: rast_setup_kernel names the owners of its rows itself (no rast_spread_kernel<0>)
   unsigned *tile_count, *tile_off, *tile_cursor;
   // short lists (n_tris <= RAST_BITS_MAX_TRIS): a tile's list is a bit per triangle -- no count /
   // scan / append passes and nothing to sort, the bits come out in list order
@@ -122,14 +126,14 @@ struct RastParams {
   const unsigned long long *colour_sorted;  // resolve: the sorted keys
   unsigned long long colour_n;
   const float *colour_rgb;                  // 3 floats per ordinal
-  unsigned long long *counters;  // [3] bin entries, [4] rows, [5] overflow flag, [6] row chunks, [9] first shaded fragment, [10] big triangles, [11] their rows (counting pass), second cache line: [16] fragments (updated while [6] is read), [24] list length (read while [4]/[6] are updated)
+  unsigned long long *counters;  // [3] bin entries, [4] rows, [5] overflow flag, [9] first shaded fragment, [10] big triangles, [11] their rows (counting pass), second cache line: [16] fragments (updated while [4] is read), [24] list length (read while [4] is updated)
 };
 
 __device__ __forceinline__ int rast_count_tris(const RastParams &p) {
   return p.n_tris_dev ? (int)min((unsigned long long)p.n_tris, *p.n_tris_dev) : p.n_tris;
 }
-__device__ __forceinline__ unsigned rast_count_chunks(const RastParams &p) {
-  return p.n_chunks_dev ? (unsigned)min((unsigned long long)p.n_chunks, *p.n_chunks_dev) : p.n_chunks;
+__device__ __forceinline__ unsigned rast_count_rows(const RastParams &p) {
+  return p.n_rows_dev ? (unsigned)min((unsigned long long)p.n_rows, *p.n_rows_dev) : p.n_rows;
 }
 
 // ---- VertexShader (:510-522) ---------------------------------------------------------
@@ -212,7 +216,7 @@ __global__ void __launch_bounds__(SETUP_THREADS) rast_setup_kernel(const __grid_
   __syncthreads();
   int nrows = 0;
   RastSetup s;
-  s.flags = 0; s.ymin = 0; s.row0 = 0; s.nrows = 0; s.row_off = 0; s.chunk_off = 0; s.tri = t;
+  s.flags = 0; s.ymin = 0; s.row0 = 0; s.nrows = 0; s.row_off = 0; s.tri = t;
   int xmin = 0, xmax = -1;
   if (t < n_tris) {
     const float *tr = reinterpret_cast<const float *>(stage) + threadIdx.x * TRI_WORDS;   // v0[4] v1[4] v2[4] normal[4] color[3]
@@ -241,25 +245,13 @@ __global__ void __launch_bounds__(SETUP_THREADS) rast_setup_kernel(const __grid_
   unsigned base = 0;
   if (lane == 31 && total) base = (unsigned)atomicAdd(p.counters + 4, (unsigned long long)total);
   base = __shfl_sync(0xffffffffu, base, 31);
-  // and chunks of it, the work items of the per-row kernels
-  unsigned nch = (unsigned)(nrows + RAST_CHUNK - 1) >> RAST_CHUNK_LOG2, cincl = nch;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const unsigned n = __shfl_up_sync(0xffffffffu, cincl, o);
-    if (lane >= o) cincl += n;
-  }
-  const unsigned ctotal = __shfl_sync(0xffffffffu, cincl, 31);
-  unsigned cbase = 0;
-  if (lane == 31 && ctotal) cbase = (unsigned)atomicAdd(p.counters + 6, (unsigned long long)ctotal);
-  cbase = __shfl_sync(0xffffffffu, cbase, 31);
   s.row_off = base + incl - (unsigned)nrows;
-  s.chunk_off = cbase + cincl - nch;
-  if (t < n_tris && (s.row_off + (unsigned)nrows > p.row_cap || s.chunk_off + nch > p.chunk_cap)) {
-    s.nrows = 0; nrows = 0; nch = 0;
+  if (t < n_tris && s.row_off + (unsigned)nrows > p.row_cap) {
+    s.nrows = 0; nrows = 0;
     atomicExch(p.counters + 5, 1ull);
   }
-  if (p.spread_in_setup)   // the triangle's row chunks, the work items of the per-row kernels
-    warp_spread((int)nch, (int)s.chunk_off, 0, 0, t, [&](int k, int x0, int, int, int tri) { p.chunk_owner[(unsigned)x0 + k] = tri; });
+  if (p.spread_in_setup)   // the owner of each of the triangle's row slots, for rast_rows_kernel
+    warp_spread(nrows, (int)s.row_off, 0, 0, t, [&](int k, int x0, int, int, int tri) { p.row_owner[(unsigned)x0 + k] = tri; });
   __syncthreads();   // every thread has read its triangle: the buffer now carries the records out
   if (t < n_tris) {
     const uint32_t *w = reinterpret_cast<const uint32_t *>(&s);
@@ -443,21 +435,20 @@ __global__ void rast_first_fragment_kernel(const __grid_constant__ RastParams p,
   }
 }
 
-// One thread per stored row: lane groups take the row chunks handed out by
-// rast_setup_kernel, so tall triangles spread over many groups.
+// One thread per row slot: the owner table names its triangle, so tall triangles
+// spread over many threads.
 __global__ void rast_rows_kernel(const __grid_constant__ RastParams p) {
-  const unsigned gid = blockIdx.x * blockDim.x + threadIdx.x;
-  const unsigned chunk = gid >> RAST_CHUNK_LOG2, sub = gid & (RAST_CHUNK - 1);
-  if (chunk >= rast_count_chunks(p)) return;
-  const int t = p.chunk_owner[chunk];
-  if ((unsigned)t >= (unsigned)p.n_tris) return;   // chunk of a triangle dropped on overflow (stale owner)
+  const unsigned slot = blockIdx.x * blockDim.x + threadIdx.x;
+  if (slot >= rast_count_rows(p)) return;
+  const int t = p.row_owner[slot];
+  if ((unsigned)t >= (unsigned)p.n_tris) return;   // slot of a triangle dropped on overflow (stale owner)
   const RastSetup &s = p.setup[t];
-  const int r = (int)((chunk - s.chunk_off) << RAST_CHUNK_LOG2) + (int)sub;
+  const int r = (int)(slot - s.row_off);
   if (r < 0 || r >= s.nrows) return;
   float4 A, B;
   rast_row_record(s, s.row0 + r, A, B);
-  p.rowsA[s.row_off + r] = A;
-  p.rowsB[s.row_off + r] = B;
+  p.rowsA[slot] = A;
+  p.rowsB[slot] = B;
 }
 
 // ---- short lists: everything between the clipped list and the fold in one launch ----------------
@@ -495,8 +486,8 @@ __global__ void __launch_bounds__(SHORT_THREADS) rast_short_kernel(const __grid_
   }
   s.ymin = ymin; s.row0 = row0; s.nrows = nrows;
   s.row_off = (unsigned)t * (unsigned)(p.fb1 - p.fb0) + (unsigned)(row0 - p.fb0);
-  s.chunk_off = 0; s.tri = t;
-  s.pad[0] = s.pad[1] = s.pad[2] = 0.f;
+  s.tri = t;
+  s.pad[0] = s.pad[1] = s.pad[2] = s.pad[3] = 0.f;
   for (int r = threadIdx.x; r < nrows; r += SHORT_THREADS) {
     float4 A, B;
     rast_row_record(s, row0 + r, A, B);
@@ -510,10 +501,8 @@ __global__ void __launch_bounds__(SHORT_THREADS) rast_short_kernel(const __grid_
     for (int k = 0; k < SETUP_WORDS; ++k)
       if ((k & 31) == (int)threadIdx.x) dst[k] = w[k];
   }
-  if (threadIdx.x == 0 && nrows > 0) {   // statistics, and what a later frame of another shape sizes its launches from
+  if (threadIdx.x == 0 && nrows > 0)   // statistics, and what a later frame of another shape sizes its launches from
     atomicAdd(p.counters + 4, (unsigned long long)nrows);
-    atomicAdd(p.counters + 6, (unsigned long long)nrows);
-  }
   if (nrows > 0) {
     const int ts = p.ts_log2;
     const int a = max(0, xmin) >> ts;                               // first tile column
@@ -563,9 +552,9 @@ __global__ void rast_scan_kernel(const __grid_constant__ RastParams p, int n_til
   if (threadIdx.x == 0) { p.tile_off[n_tiles] = carry; p.counters[3] = carry; }
 }
 
-// Per-triangle fan-out work: WHAT = 0 hands the triangle's row chunks to the per-row
-// kernels (chunk_owner), 1 counts the screen tiles its bounding box touches, 2 appends
-// it to those tiles' lists.  Two launch shapes: one thread per triangle (long lists;
+// Per-triangle fan-out work: WHAT = 0 names the triangle as the owner of its row slots
+// (row_owner, for rast_rows_kernel), 1 counts the screen tiles its bounding box touches,
+// 2 appends it to those tiles' lists.  Two launch shapes: one thread per triangle (long lists;
 // outliers are spread over the warp) or one block per triangle (short lists of big
 // triangles, e.g. the Cornell box with its shadow volumes at 4K).
 template <int WHAT>
@@ -575,8 +564,8 @@ __global__ void rast_spread_kernel(const __grid_constant__ RastParams p, int blo
   if (t < rast_count_tris(p)) {
     const RastSetup &s = p.setup[t];
     if (WHAT == 0) {
-      n = (s.nrows + RAST_CHUNK - 1) >> RAST_CHUNK_LOG2;
-      a = (int)s.chunk_off;
+      n = s.nrows;
+      a = (int)s.row_off;
     } else if (s.nrows > 0) {
       const int ts = p.ts_log2;
       const int xmin = min(s.v[0].x, min(s.v[1].x, s.v[2].x)) - 1;
@@ -588,10 +577,9 @@ __global__ void rast_spread_kernel(const __grid_constant__ RastParams p, int blo
     }
   }
   auto body = [&](int k, int x0, int w, int y0, int tri) {
-    if (WHAT == 0) { p.chunk_owner[(unsigned)x0 + k] = tri; return; }
+    if (WHAT == 0) { p.row_owner[(unsigned)x0 + k] = tri; return; }
     const size_t tile = (size_t)(y0 + k / w - p.ty0) * p.tiles_x + x0 + k % w;
     if (WHAT == 1) { atomicAdd(p.tile_count + tile, 1u); return; }
-    if (WHAT == 3) { atomicOr(p.tile_bits + tile * p.bits_words + (tri >> 5), 1u << (tri & 31)); return; }
     const unsigned pos = atomicAdd(p.tile_cursor + tile, 1u);
     const unsigned at = p.tile_off[tile] + pos;
     if (at < p.bin_cap) p.bins[at] = tri;
@@ -603,15 +591,13 @@ __global__ void rast_spread_kernel(const __grid_constant__ RastParams p, int blo
   }
 }
 
-static void rast_spread_launch(b200_ctx *ctx, const RastParams &p, int what) {
+template <int WHAT>
+static void rast_spread_launch(b200_ctx *ctx, const RastParams &p) {
   const int n = p.n_tris;
   if (n <= 0) return;
   const int per_block = n <= 8192;
   const dim3 grid(per_block ? n : (n + 255) / 256);
-  if (what == 0) rast_spread_kernel<0><<<grid, 256, 0, ctx->stream>>>(p, per_block);
-  else if (what == 1) rast_spread_kernel<1><<<grid, 256, 0, ctx->stream>>>(p, per_block);
-  else if (what == 3) rast_spread_kernel<3><<<grid, 256, 0, ctx->stream>>>(p, per_block);
-  else rast_spread_kernel<2><<<grid, 256, 0, ctx->stream>>>(p, per_block);
+  rast_spread_kernel<WHAT><<<grid, 256, 0, ctx->stream>>>(p, per_block);
   ctx->stats.kernel_launches++;
   tl_mark(ctx, "rast_spread_kernel");
 }
@@ -1069,203 +1055,155 @@ extern "C" int b200_debug_rast_inverse(const float *R16, float *out16, int *use_
   return B200_OK;
 }
 
-int rast_launch(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, int row0, int row1,
-                float *d_rgb, float *d_depth, int32_t *d_index, uint32_t *d_argb, bool spec) {
-  // n is the list length, or in a pipelined whole-Draw frame the bound the geometry stage wrote under
-  const int W = cam->width, H = cam->height, n = ctx->rast_n_tris;
-  RastParams p;
-  memset(&p, 0, sizeof p);
-  p.W = W; p.H = H;
-  p.row0 = row0; p.row1 = row1;
-  p.fb0 = row0 - 2 > 0 ? row0 - 2 : 0;
-  p.fb1 = row1 + 2 < H ? row1 + 2 : H;
-  p.ts_log2 = ctx->opt_rast_tile_log2;
-  const int ts = p.ts_log2, TS = 1 << ts;
-  p.tiles_x = (W + TS - 1) >> ts;
-  p.ty0 = p.fb0 >> ts;
-  p.tiles_y = ((p.fb1 - 1) >> ts) - p.ty0 + 1;
-  const int n_tiles = p.tiles_x * p.tiles_y;
-  p.focal = cam->focal;
-  memcpy(p.light, light->pos, sizeof p.light);
-  memcpy(p.power, light->power, sizeof p.power);
-  memcpy(p.indirect, light->indirect, sizeof p.indirect);
-  p.src = (const rast_triangle *)ctx->rast_src.p;
-  p.n_tris = n;
-  p.spread_in_setup = n > 8192 ? 1 : 0;   // short lists of big triangles: one block per triangle spreads better
+// The back end of a frame of n triangles: scatter / resolve (rast_fast.cuh) or ordered screen tiles.  rast_frame
+// asks before the geometry stage (n: the list bound a pipelined geometry stage writes under) and acts on the answer
+// there; rast_launch asks again for the list it is given.
+bool rast_scatter_path(const b200_ctx *ctx, long long n) {
+  return ctx->opt_rast_path == 2 || (ctx->opt_rast_path == 0 && !ctx->rast_has_shadow && !ctx->rast_tex_on &&
+                                     !ctx->opt_rast_colour && n < RAST_FAST_MAX_TRIS);
+}
 
-  const size_t npix = (size_t)W * H;
-  if (ctx->opt_rast_path == 2 && ctx->rast_has_shadow)
-    return ctx_fail(ctx, B200_EINVAL, "the scatter path cannot draw shadow-volume triangles");
-  if (ctx->opt_rast_path == 2 && n >= RAST_FAST_MAX_TRIS) return ctx_fail(ctx, B200_EINVAL, "too many triangles for the scatter path");
-  const int colour = ctx->opt_rast_colour;
-  if (ctx->opt_rast_path == 2 && (ctx->rast_tex_on || colour))
-    return ctx_fail(ctx, B200_EINVAL, "the scatter path cannot draw textures or colour modes (both depend on the order of the fragments)");
-  if (colour && (row0 != 0 || row1 != H)) return ctx_fail(ctx, B200_EINVAL, "colour modes 1 / 2 number the fragments of the whole frame: no row bands");
-  if (colour && (W > 4096 || H > 4096)) return ctx_fail(ctx, B200_EINVAL, "colour modes 1 / 2: frames up to 4096 x 4096");
-  const bool fast = ctx->opt_rast_path == 2 || (ctx->opt_rast_path == 0 && !ctx->rast_has_shadow && !ctx->rast_tex_on && !colour && n < RAST_FAST_MAX_TRIS);
-  p.tex_on = ctx->rast_tex_on && !colour;   // the colour modes never look at the texture fields (:575)
-  p.colour_mode = colour;
-  const bool texk = p.tex_on || colour;     // the kernel variants that know about textures / colour modes
-  if (p.tex_on) {
-    p.tex = ctx->rast_tex;
-    memcpy(p.tex.cam, cam->pos, sizeof p.tex.cam);
-    rast_tex_view(cam->R, p.tex.Rinv, &p.tex.use_rinv);
+// rast_fill_kernel at the frame's tile size (TEX: the variant that knows about textures / colour modes)
+template <bool TEX>
+static int rast_fill_launch(b200_ctx *ctx, const RastParams &p, const char *name) {
+  const dim3 grid(p.tiles_x, p.tiles_y);
+  switch (p.ts_log2) {
+    case 3: rast_fill_kernel<3, TEX><<<grid, 64, 0, ctx->stream>>>(p); break;
+    case 4: rast_fill_kernel<4, TEX><<<grid, 256, 0, ctx->stream>>>(p); break;
+    default: rast_fill_kernel<5, TEX><<<grid, 1024, 0, ctx->stream>>>(p); break;
   }
-  p.fast = fast ? 1 : 0;
-  p.out_rgb = d_rgb; p.out_depth = d_depth; p.out_index = d_index; p.out_argb = d_argb;
-  p.counters = (unsigned long long *)ctx->counters.p;
-  // worst case rows: every triangle spans the whole band
-  size_t row_cap = (size_t)n * (size_t)(p.fb1 - p.fb0);
-  const size_t row_budget = (size_t)64 << 20;   // 64 Mi rows = 2 GiB of row records
-  if (row_cap < 1) row_cap = 1;
-  size_t chunk_cap = (row_cap > row_budget ? row_budget : row_cap) / RAST_CHUNK + (size_t)n + 1;
-  size_t bin_cap = 0;
+  ctx->stats.kernel_launches++;
+  tl_mark(ctx, name);
+  CU_CHECK(ctx, cudaGetLastError());
+  return B200_OK;
+}
+
+// ---- scatter / resolve (rast_fast.cuh); p: the frame as rast_launch set it up ----
+static int rast_launch_scatter(b200_ctx *ctx, RastParams &p, bool spec) {
+  const int W = p.W, n = p.n_tris, row0 = p.row0, row1 = p.row1;
+  const size_t npix = (size_t)W * p.H;
+  ctx->rast_w = 0; ctx->rast_h = 0;   // no intermediate buffers in this path
+  if (int rc = ensure(ctx, ctx->rast_keys, npix * sizeof(unsigned long long))) return rc;
+  p.keys = (unsigned long long *)ctx->rast_keys.p;
+  if (int rc = ensure(ctx, ctx->rast_trimeta, sizeof(int2) * (size_t)(n ? n : 1))) return rc;
+  p.trimeta = (int2 *)ctx->rast_trimeta.p;
+  p.orig = ctx->rast_culled ? (const int *)ctx->rast_orig.p : nullptr;
+  // small triangles: S2_ROWS record places each, addressed by the key (only the rows drawn are touched)
+  if (int rc = ensure(ctx, ctx->rast_srowsB, sizeof(float4) * S2_ROWS * (size_t)(n ? n : 1))) return rc;
+  if (int rc = ensure(ctx, ctx->rast_srowsL, sizeof(int) * S2_ROWS * (size_t)(n ? n : 1))) return rc;
+  p.srowsB = (float4 *)ctx->rast_srowsB.p;
+  p.srowsL = (int *)ctx->rast_srowsL.p;
+  const int s2_blocks = (n + S2_THREADS - 1) / S2_THREADS;
+  size_t n_rows = 0, big_cap = 0;   // rows of the big triangles, entries of the big list
   if (spec) {
-    // sizes guessed from the last verified frame; the setup / scan kernels flag any overflow
-    row_cap = (size_t)rast_spec_cap(ctx->rast_spec.rows);
-    chunk_cap = (size_t)rast_spec_cap(ctx->rast_spec.chunks);
-    bin_cap = (size_t)rast_spec_cap(ctx->rast_spec.bins);
-    p.n_tris_dev = ctx->rast_inflight.whole_draw ? p.counters + 24 : nullptr;
-    p.n_chunks_dev = p.counters + 6;
-    p.n_chunks = (unsigned)(chunk_cap > 0xffffffffull ? 0xffffffffull : chunk_cap);
-    ctx->rast_inflight.cap_bins = bin_cap;
-    ctx->rast_inflight.fast = fast ? 1 : 0;
-  }
-  unsigned long long *hc = (unsigned long long *)ctx->pinned;
-
-  // the entry value of indirectLightPowerPerArea reaches the first shaded fragment only (:585)
-  const float steady = 0.2f * 1.0f;
-  if (n > 0 && !colour && (memcmp(&light->indirect[0], &steady, 4) || memcmp(&light->indirect[1], &steady, 4) ||
-                memcmp(&light->indirect[2], &steady, 4))) {
-    unsigned long long *first = p.counters + 9;
-    CU_CHECK(ctx, cudaMemsetAsync(first, 0xff, sizeof(unsigned long long), ctx->stream));
-    rast_first_fragment_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(p, first);
+    // sizes guessed from the last verified frame; the kernels flag any overflow.  A frame whose
+    // predecessor had no big triangle does not launch the big-triangle kernels at all.
+    n_rows = (size_t)rast_spec_cap(ctx->rast_spec.rows);
+    big_cap = ctx->rast_spec.big ? (size_t)rast_spec_cap(ctx->rast_spec.big) : 0;
+  } else if (n > 0) {
+    // exact sizes from a counting pass: [10] big triangles, [11] their rows
+    unsigned long long *hc = (unsigned long long *)ctx->pinned;
+    rast_scatter2_kernel<true><<<s2_blocks, S2_THREADS, 0, ctx->stream>>>(p);
     ctx->stats.kernel_launches++;
-    tl_mark(ctx, "rast_first_fragment_kernel");
-    p.first_frag = first;
+    tl_mark(ctx, "rast_scatter2_kernel<count>");
+    CU_CHECK(ctx, cudaGetLastError());
+    CU_CHECK(ctx, cudaMemcpyAsync(hc, ctx->counters.p, 16 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    CU_CHECK(ctx, cudaMemsetAsync(p.counters + 10, 0, 2 * sizeof(unsigned long long), ctx->stream));
+    CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
+    if (hc[11] > 0xfffffff0ull) return ctx_fail(ctx, B200_ENOMEM, "row table budget exceeded");
+    n_rows = (size_t)hc[11];
+    big_cap = (size_t)hc[10];
   }
-
-  if (fast) {
-    // ---- scatter / resolve (rast_fast.cuh) ----
-    ctx->rast_w = 0; ctx->rast_h = 0;   // no intermediate buffers in this path
-    if (int rc = ensure(ctx, ctx->rast_keys, npix * sizeof(unsigned long long))) return rc;
-    p.keys = (unsigned long long *)ctx->rast_keys.p;
-    if (int rc = ensure(ctx, ctx->rast_trimeta, sizeof(int2) * (size_t)(n ? n : 1))) return rc;
-    p.trimeta = (int2 *)ctx->rast_trimeta.p;
-    p.orig = ctx->rast_culled ? (const int *)ctx->rast_orig.p : nullptr;
-    // small triangles: S2_ROWS record places each, addressed by the key (only the rows drawn are touched)
-    if (int rc = ensure(ctx, ctx->rast_srowsB, sizeof(float4) * S2_ROWS * (size_t)(n ? n : 1))) return rc;
-    if (int rc = ensure(ctx, ctx->rast_srowsL, sizeof(int) * S2_ROWS * (size_t)(n ? n : 1))) return rc;
-    p.srowsB = (float4 *)ctx->rast_srowsB.p;
-    p.srowsL = (int *)ctx->rast_srowsL.p;
-    const int s2_blocks = (n + S2_THREADS - 1) / S2_THREADS;
-    size_t n_rows = 1, big_cap = 0;
-    if (spec) {
-      // sizes guessed from the last verified frame; the kernels flag any overflow.  A frame whose
-      // predecessor had no big triangle does not launch the big-triangle kernels at all.
-      n_rows = row_cap;
-      big_cap = ctx->rast_spec.big ? (size_t)rast_spec_cap(ctx->rast_spec.big) : 0;
+  p.n_rows = (unsigned)(n_rows > 0xffffffffull ? 0xffffffffull : n_rows);
+  if (n_rows < 1) n_rows = 1;
+  if (big_cap > 0x7fffffffull) big_cap = 0x7fffffffull;
+  if (int rc = ensure(ctx, ctx->rast_rowsA, sizeof(int) * n_rows)) return rc;
+  if (int rc = ensure(ctx, ctx->rast_rowsB, sizeof(float4) * n_rows)) return rc;
+  if (int rc = ensure(ctx, ctx->rast_setup, sizeof(RastSetup) * (big_cap ? big_cap : 1))) return rc;
+  if (int rc = ensure(ctx, ctx->rast_big, sizeof(int) * (big_cap ? big_cap : 1))) return rc;
+  if (int rc = ensure(ctx, ctx->rast_row_owner, sizeof(int) * n_rows)) return rc;
+  p.rowsL = (int *)ctx->rast_rowsA.p;
+  p.rowsB = (float4 *)ctx->rast_rowsB.p;
+  p.row_cap = (unsigned)(n_rows > 0xffffffffull ? 0xffffffffull : n_rows);
+  p.setup = (RastSetup *)ctx->rast_setup.p;
+  p.big_list = (int *)ctx->rast_big.p;
+  p.big_cap = (unsigned)big_cap;
+  p.row_owner = (int *)ctx->rast_row_owner.p;
+  // cleared right before the scatter so that the 64-bit keys (66 MB at 4K, less than the L2)
+  // are still cache-resident when the atomics arrive
+  if (!ctx->rast_keys_cleared) {   // (a pipelined whole-Draw frame: already done by its geometry kernel)
+    CU_CHECK(ctx, cudaMemsetAsync(p.keys + (size_t)p.fb0 * W, 0, (size_t)(p.fb1 - p.fb0) * W * sizeof(unsigned long long), ctx->stream));
+    tl_mark(ctx, "memset keys");
+  }
+  ctx->rast_keys_cleared = 0;
+  if (n > 0) {
+    if (spec && ctx->rast_geom_chunks > 1) {
+      // chunk k of the list is scattered on the second stream as soon as the geometry kernel's
+      // k-th launch is done, while chunk k + 1 of the scene is still on the link; the frame goes on
+      // when all are in
+      for (int c = 0; c < ctx->rast_geom_chunks; ++c) {
+        RastParams pc = p;
+        pc.range_lo = c ? p.counters + 12 + (c - 1) : nullptr;
+        pc.range_hi = p.counters + 12 + c;
+        const int bound = ctx->rast_geom_chunk_tris[c] + ctx->rast_geom_chunk_tris[c] / 32 + 1024;   // + 3 %: clipping can add triangles
+        CU_CHECK(ctx, cudaStreamWaitEvent(ctx->aux_stream, ctx->ev_chunk[c], 0));
+        rast_scatter2_kernel<false><<<(bound + S2_THREADS - 1) / S2_THREADS, S2_THREADS, 0, ctx->aux_stream>>>(pc);
+        ctx->stats.kernel_launches++;
+      }
+      CU_CHECK(ctx, cudaEventRecord(ctx->ev_join, ctx->aux_stream));
+      CU_CHECK(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
     } else {
-      chunk_cap = 1;
-      p.n_chunks = 0;
-      if (n > 0) {
-        // exact sizes from a counting pass: [10] big triangles, [11] their rows
-        rast_scatter2_kernel<true><<<s2_blocks, S2_THREADS, 0, ctx->stream>>>(p);
-        ctx->stats.kernel_launches++;
-        tl_mark(ctx, "rast_scatter2_kernel<count>");
-        CU_CHECK(ctx, cudaGetLastError());
-        CU_CHECK(ctx, cudaMemcpyAsync(hc, ctx->counters.p, 16 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
-        CU_CHECK(ctx, cudaMemsetAsync(p.counters + 10, 0, 2 * sizeof(unsigned long long), ctx->stream));
-        CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
-        if (hc[11] > 0xfffffff0ull) return ctx_fail(ctx, B200_ENOMEM, "row table budget exceeded");
-        n_rows = (size_t)hc[11];
-        big_cap = (size_t)hc[10];
-        chunk_cap = (size_t)hc[11];
-        p.n_chunks = (unsigned)hc[11];
-        if (n_rows < 1) n_rows = 1;
-        if (chunk_cap < 1) chunk_cap = 1;
-      }
-    }
-    if (big_cap > 0x7fffffffull) big_cap = 0x7fffffffull;
-    if (int rc = ensure(ctx, ctx->rast_rowsA, sizeof(int) * n_rows)) return rc;
-    if (int rc = ensure(ctx, ctx->rast_rowsB, sizeof(float4) * n_rows)) return rc;
-    if (int rc = ensure(ctx, ctx->rast_setup, sizeof(RastSetup) * (big_cap ? big_cap : 1))) return rc;
-    if (int rc = ensure(ctx, ctx->rast_big, sizeof(int) * (big_cap ? big_cap : 1))) return rc;
-    if (int rc = ensure(ctx, ctx->rast_chunks, sizeof(int) * chunk_cap)) return rc;
-    p.rowsL = (int *)ctx->rast_rowsA.p;
-    p.rowsB = (float4 *)ctx->rast_rowsB.p;
-    p.row_cap = (unsigned)(n_rows > 0xffffffffull ? 0xffffffffull : n_rows);
-    p.setup = (RastSetup *)ctx->rast_setup.p;
-    p.big_list = (int *)ctx->rast_big.p;
-    p.big_cap = (unsigned)big_cap;
-    p.chunk_owner = (int *)ctx->rast_chunks.p;
-    p.chunk_cap = (unsigned)(chunk_cap > 0xffffffffull ? 0xffffffffull : chunk_cap);
-    // cleared right before the scatter so that the 64-bit keys (66 MB at 4K, less than the L2)
-    // are still cache-resident when the atomics arrive
-    if (!ctx->rast_keys_cleared) {   // (a pipelined whole-Draw frame: already done by its geometry kernel)
-      CU_CHECK(ctx, cudaMemsetAsync(p.keys + (size_t)p.fb0 * W, 0, (size_t)(p.fb1 - p.fb0) * W * sizeof(unsigned long long), ctx->stream));
-      tl_mark(ctx, "memset keys");
-    }
-    ctx->rast_keys_cleared = 0;
-    if (n > 0) {
-      if (spec && ctx->rast_geom_chunks > 1) {
-        // chunk k of the list is scattered on the second stream as soon as the geometry kernel's
-        // k-th launch is done, while chunk k + 1 of the scene is still on the link; the frame goes on
-        // when all are in
-        for (int c = 0; c < ctx->rast_geom_chunks; ++c) {
-          RastParams pc = p;
-          pc.range_lo = c ? p.counters + 12 + (c - 1) : nullptr;
-          pc.range_hi = p.counters + 12 + c;
-          const int bound = ctx->rast_geom_chunk_tris[c] + ctx->rast_geom_chunk_tris[c] / 32 + 1024;   // + 3 %: clipping can add triangles
-          CU_CHECK(ctx, cudaStreamWaitEvent(ctx->aux_stream, ctx->ev_chunk[c], 0));
-          rast_scatter2_kernel<false><<<(bound + S2_THREADS - 1) / S2_THREADS, S2_THREADS, 0, ctx->aux_stream>>>(pc);
-          ctx->stats.kernel_launches++;
-        }
-        CU_CHECK(ctx, cudaEventRecord(ctx->ev_join, ctx->aux_stream));
-        CU_CHECK(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-      } else {
-        rast_scatter2_kernel<false><<<s2_blocks, S2_THREADS, 0, ctx->stream>>>(p);
-        ctx->stats.kernel_launches++;
-      }
-      tl_mark(ctx, "rast_scatter2_kernel");
-      if (big_cap > 0) {
-        rast_setup_big_kernel<<<(int)((big_cap + 127) / 128), 128, 0, ctx->stream>>>(p);
-        ctx->stats.kernel_launches++;
-        tl_mark(ctx, "rast_setup_big_kernel");
-        if (p.n_chunks > 0) {
-          rast_scatter_kernel<<<(int)(((size_t)p.n_chunks + 255) / 256), 256, 0, ctx->stream>>>(p);
-          ctx->stats.kernel_launches++;
-          tl_mark(ctx, "rast_scatter_kernel");
-        }
-      }
-      CU_CHECK(ctx, cudaGetLastError());
-    }
-    // host-pointer entries: resolve in slices, each slice's packed rows leave for the host
-    // while the next one is resolved (band_slice_done is a no-op otherwise)
-    const int k = (ctx->slice_host && (size_t)(row1 - row0) * W >= B200_SLICE_MIN_PIXELS) ? B200_SLICES : 1;
-    for (int i = 0; i < k; ++i) {
-      p.row0 = band_slice_edge(row0, row1 - row0, i, k, RS_H);
-      p.row1 = band_slice_edge(row0, row1 - row0, i + 1, k, RS_H);
-      if (p.row1 <= p.row0) continue;
-      dim3 rg((W + RS_W - 1) / RS_W, (p.row1 - p.row0 + RS_H - 1) / RS_H);
-      rast_resolve_kernel<false, false><<<rg, RS_W * RS_H, 0, ctx->stream>>>(p);
+      rast_scatter2_kernel<false><<<s2_blocks, S2_THREADS, 0, ctx->stream>>>(p);
       ctx->stats.kernel_launches++;
-      tl_mark(ctx, "rast_resolve_kernel");
-      CU_CHECK(ctx, cudaGetLastError());
-      if (int rc = band_slice_done(ctx, p.row0, p.row1)) return rc;
     }
-    return B200_OK;
+    tl_mark(ctx, "rast_scatter2_kernel");
+    if (big_cap > 0) {
+      rast_setup_big_kernel<<<(int)((big_cap + 127) / 128), 128, 0, ctx->stream>>>(p);
+      ctx->stats.kernel_launches++;
+      tl_mark(ctx, "rast_setup_big_kernel");
+      if (p.n_rows > 0) {
+        rast_scatter_kernel<<<(int)(((size_t)p.n_rows + 255) / 256), 256, 0, ctx->stream>>>(p);
+        ctx->stats.kernel_launches++;
+        tl_mark(ctx, "rast_scatter_kernel");
+      }
+    }
+    CU_CHECK(ctx, cudaGetLastError());
   }
+  // host-pointer entries: resolve in slices, each slice's packed rows leave for the host
+  // while the next one is resolved (band_slice_done is a no-op otherwise)
+  const int k = (ctx->slice_host && (size_t)(row1 - row0) * W >= B200_SLICE_MIN_PIXELS) ? B200_SLICES : 1;
+  for (int i = 0; i < k; ++i) {
+    p.row0 = band_slice_edge(row0, row1 - row0, i, k, RS_H);
+    p.row1 = band_slice_edge(row0, row1 - row0, i + 1, k, RS_H);
+    if (p.row1 <= p.row0) continue;
+    dim3 rg((W + RS_W - 1) / RS_W, (p.row1 - p.row0 + RS_H - 1) / RS_H);
+    rast_resolve_kernel<false, false><<<rg, RS_W * RS_H, 0, ctx->stream>>>(p);
+    ctx->stats.kernel_launches++;
+    tl_mark(ctx, "rast_resolve_kernel");
+    CU_CHECK(ctx, cudaGetLastError());
+    if (int rc = band_slice_done(ctx, p.row0, p.row1)) return rc;
+  }
+  return B200_OK;
+}
 
-  // ---- ordered tile path ----
+// ---- ordered screen tiles; p: the frame as rast_launch set it up ----
+static int rast_launch_ordered(b200_ctx *ctx, RastParams &p, bool spec) {
+  const int W = p.W, H = p.H, n = p.n_tris, row0 = p.row0, row1 = p.row1, colour = p.colour_mode;
+  const int n_tiles = p.tiles_x * p.tiles_y;
+  const size_t npix = (size_t)W * H;
+  const bool texk = p.tex_on || colour;           // the kernel variants that know about textures / colour modes
+  const bool bits = n <= RAST_BITS_MAX_TRIS;      // short list: bit-per-triangle tile lists
+  unsigned long long *hc = (unsigned long long *)ctx->pinned;
+  p.spread_in_setup = n > 8192 ? 1 : 0;   // short lists of big triangles: one block per triangle spreads better
   if (int rc = ensure(ctx, ctx->rast_setup, sizeof(RastSetup) * (size_t)(n ? n : 1))) return rc;
   p.setup = (RastSetup *)ctx->rast_setup.p;
-  if (int rc = ensure(ctx, ctx->rast_chunks, sizeof(int) * chunk_cap)) return rc;
-  p.chunk_owner = (int *)ctx->rast_chunks.p;
-  p.chunk_cap = (unsigned)(chunk_cap > 0xffffffffull ? 0xffffffffull : chunk_cap);
-  // a short list (bit-per-triangle tile lists, rast_short_kernel): every triangle owns a band's worth of rows
-  if (n <= RAST_BITS_MAX_TRIS) row_cap = (size_t)(n ? n : 1) * (size_t)(p.fb1 - p.fb0);
+  // row slots: a short list (rast_short_kernel) gives every triangle a band's worth; a long one claims what its
+  // triangles reach, at worst the whole band each (pipelined: what the last verified frame claimed, + 3 %)
+  size_t row_cap = spec && !bits ? (size_t)rast_spec_cap(ctx->rast_spec.rows) : (size_t)(n ? n : 1) * (size_t)(p.fb1 - p.fb0);
+  const size_t row_budget = (size_t)64 << 20;   // 64 Mi rows = 2 GiB of row records
   if (row_cap > row_budget) row_cap = row_budget;
+  if (int rc = ensure(ctx, ctx->rast_row_owner, sizeof(int) * row_cap)) return rc;
+  p.row_owner = (int *)ctx->rast_row_owner.p;
   if (int rc = ensure(ctx, ctx->rast_rowsA, sizeof(float4) * row_cap)) return rc;
   if (int rc = ensure(ctx, ctx->rast_rowsB, sizeof(float4) * row_cap)) return rc;
   if (int rc = ensure(ctx, ctx->rast_tile_count, sizeof(unsigned) * (size_t)(n_tiles + 1) * 3)) return rc;
@@ -1291,6 +1229,7 @@ int rast_launch(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, i
   p.rowsA = (float4 *)ctx->rast_rowsA.p;
   p.rowsB = (float4 *)ctx->rast_rowsB.p;
   p.row_cap = (unsigned)(row_cap > 0xffffffffull ? 0xffffffffull : row_cap);
+  p.n_rows = p.row_cap;   // a launch bound until the rows claimed are read back (pipelined: clamped on the device)
   p.tile_count = (unsigned *)ctx->rast_tile_count.p;
   p.tile_off = p.tile_count + (n_tiles + 1);
   p.tile_cursor = p.tile_off + (n_tiles + 1);
@@ -1301,7 +1240,6 @@ int rast_launch(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, i
   p.shadow = (int *)ctx->rast_shadow.p;
   p.index = (int *)ctx->rast_index.p;
 
-  const bool bits = n <= RAST_BITS_MAX_TRIS;      // short list: bit-per-triangle tile lists
   if (bits) {
     p.bits_words = (n + 31) / 32 > 0 ? (n + 31) / 32 : 1;
     if (int rc = ensure(ctx, ctx->rast_tile_bits, sizeof(unsigned) * (size_t)n_tiles * p.bits_words)) return rc;
@@ -1319,8 +1257,8 @@ int rast_launch(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, i
     rast_setup_kernel<<<(n + SETUP_THREADS - 1) / SETUP_THREADS, SETUP_THREADS, 0, ctx->stream>>>(p);
     ctx->stats.kernel_launches++;
     tl_mark(ctx, "rast_setup_kernel");
-    if (!p.spread_in_setup) rast_spread_launch(ctx, p, 0);
-    rast_spread_launch(ctx, p, 1);
+    if (!p.spread_in_setup) rast_spread_launch<0>(ctx, p);
+    rast_spread_launch<1>(ctx, p);
   }
   if (!bits) {
     rast_scan_kernel<<<1, 1024, 0, ctx->stream>>>(p, n_tiles);
@@ -1328,45 +1266,32 @@ int rast_launch(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, i
     tl_mark(ctx, "rast_scan_kernel");
   }
   CU_CHECK(ctx, cudaGetLastError());
-  if (!spec) {
+  size_t bin_cap = 0;
+  if (spec) {
+    // sizes guessed from the last verified frame; the setup / scan kernels flag any overflow
+    bin_cap = (size_t)rast_spec_cap(ctx->rast_spec.bins);
+    ctx->rast_inflight.cap_bins = bin_cap;
+  } else {
     // the bin array is sized from the scanned total: read it back (tiny, one sync)
     CU_CHECK(ctx, cudaMemcpyAsync(hc, ctx->counters.p, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
     CU_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
     if (hc[5]) return ctx_fail(ctx, B200_ENOMEM, "row table budget exceeded (triangles too tall for this band)");
     bin_cap = (size_t)hc[3];
-    p.n_chunks = (unsigned)hc[6];
+    p.n_rows = (unsigned)hc[4];
   }
   if (int rc = ensure(ctx, ctx->rast_bins, sizeof(int) * (bin_cap ? bin_cap : 1))) return rc;
   if (int rc = ensure(ctx, ctx->rast_tmp, sizeof(int) * (bin_cap ? bin_cap : 1))) return rc;
   p.bins = (int *)ctx->rast_bins.p;
   p.bins_tmp = (int *)ctx->rast_tmp.p;
   p.bin_cap = (unsigned)(bin_cap > 0xffffffffull ? 0xffffffffull : bin_cap);
-  if (p.n_chunks > 0 && n > 0 && !bits) {
-    rast_rows_kernel<<<(int)(((size_t)p.n_chunks * RAST_CHUNK + 255) / 256), 256, 0, ctx->stream>>>(p);
+  if (p.n_rows > 0 && n > 0 && !bits) {
+    rast_rows_kernel<<<(int)(((size_t)p.n_rows + 255) / 256), 256, 0, ctx->stream>>>(p);
     ctx->stats.kernel_launches++;
     tl_mark(ctx, "rast_rows_kernel");
   }
-  if (n > 0 && bin_cap > 0 && !bits) rast_spread_launch(ctx, p, 2);
-  dim3 grid(p.tiles_x, p.tiles_y);
-  auto fill_tex = [&](const RastParams &pp) {
-    switch (ts) {
-      case 3: rast_fill_kernel<3, true><<<grid, 64, 0, ctx->stream>>>(pp); break;
-      case 4: rast_fill_kernel<4, true><<<grid, 256, 0, ctx->stream>>>(pp); break;
-      default: rast_fill_kernel<5, true><<<grid, 1024, 0, ctx->stream>>>(pp); break;
-    }
-  };
-  if (texk) {
-    fill_tex(p);
-  } else {
-    switch (ts) {
-      case 3: rast_fill_kernel<3, false><<<grid, 64, 0, ctx->stream>>>(p); break;
-      case 4: rast_fill_kernel<4, false><<<grid, 256, 0, ctx->stream>>>(p); break;
-      default: rast_fill_kernel<5, false><<<grid, 1024, 0, ctx->stream>>>(p); break;
-    }
-  }
-  ctx->stats.kernel_launches++;
-  tl_mark(ctx, "rast_fill_kernel");
-  CU_CHECK(ctx, cudaGetLastError());
+  if (n > 0 && bin_cap > 0 && !bits) rast_spread_launch<2>(ctx, p);
+  if (int rc = texk ? rast_fill_launch<true>(ctx, p, "rast_fill_kernel") : rast_fill_launch<false>(ctx, p, "rast_fill_kernel"))
+    return rc;
   if (colour) {
     // the accepted fragments in the reference's serial order: count, emit, sort; then the host draws
     // three rand() values per fragment, exactly as PixelShader would have (:649-651, :657-659)
@@ -1382,10 +1307,7 @@ int rast_launch(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, i
       RastParams pe = p;
       pe.colour_emit = keys_a;
       pe.colour_n = n_acc;
-      fill_tex(pe);
-      ctx->stats.kernel_launches++;
-      tl_mark(ctx, "rast_fill_kernel<emit>");
-      CU_CHECK(ctx, cudaGetLastError());
+      if (int rc = rast_fill_launch<true>(ctx, pe, "rast_fill_kernel<emit>")) return rc;
       int tri_bits = 1;
       while (tri_bits < 31 && (1ll << tri_bits) < (long long)n) ++tri_bits;
       if (int rc = rast_colour_sort(ctx, keys_a, keys_b, n_acc, 24 + tri_bits)) return rc;
@@ -1422,4 +1344,63 @@ int rast_launch(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, i
     if (int rc = band_slice_done(ctx, p.row0, p.row1)) return rc;
   }
   return B200_OK;
+}
+
+int rast_launch(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, int row0, int row1,
+                float *d_rgb, float *d_depth, int32_t *d_index, uint32_t *d_argb, bool spec) {
+  // n is the list length, or in a pipelined whole-Draw frame the bound the geometry stage wrote under
+  const int W = cam->width, H = cam->height, n = ctx->rast_n_tris;
+  const int colour = ctx->opt_rast_colour;
+  if (ctx->opt_rast_path == 2 && ctx->rast_has_shadow)
+    return ctx_fail(ctx, B200_EINVAL, "the scatter path cannot draw shadow-volume triangles");
+  if (ctx->opt_rast_path == 2 && n >= RAST_FAST_MAX_TRIS) return ctx_fail(ctx, B200_EINVAL, "too many triangles for the scatter path");
+  if (ctx->opt_rast_path == 2 && (ctx->rast_tex_on || colour))
+    return ctx_fail(ctx, B200_EINVAL, "the scatter path cannot draw textures or colour modes (both depend on the order of the fragments)");
+  if (colour && (row0 != 0 || row1 != H)) return ctx_fail(ctx, B200_EINVAL, "colour modes 1 / 2 number the fragments of the whole frame: no row bands");
+  if (colour && (W > 4096 || H > 4096)) return ctx_fail(ctx, B200_EINVAL, "colour modes 1 / 2: frames up to 4096 x 4096");
+
+  RastParams p;
+  memset(&p, 0, sizeof p);
+  p.W = W; p.H = H;
+  p.row0 = row0; p.row1 = row1;
+  p.fb0 = row0 - 2 > 0 ? row0 - 2 : 0;
+  p.fb1 = row1 + 2 < H ? row1 + 2 : H;
+  p.ts_log2 = ctx->opt_rast_tile_log2;
+  const int ts = p.ts_log2, TS = 1 << ts;
+  p.tiles_x = (W + TS - 1) >> ts;
+  p.ty0 = p.fb0 >> ts;
+  p.tiles_y = ((p.fb1 - 1) >> ts) - p.ty0 + 1;
+  p.focal = cam->focal;
+  memcpy(p.light, light->pos, sizeof p.light);
+  memcpy(p.power, light->power, sizeof p.power);
+  memcpy(p.indirect, light->indirect, sizeof p.indirect);
+  p.src = (const rast_triangle *)ctx->rast_src.p;
+  p.n_tris = n;
+  p.tex_on = ctx->rast_tex_on && !colour;   // the colour modes never look at the texture fields (:575)
+  p.colour_mode = colour;
+  if (p.tex_on) {
+    p.tex = ctx->rast_tex;
+    memcpy(p.tex.cam, cam->pos, sizeof p.tex.cam);
+    rast_tex_view(cam->R, p.tex.Rinv, &p.tex.use_rinv);
+  }
+  p.out_rgb = d_rgb; p.out_depth = d_depth; p.out_index = d_index; p.out_argb = d_argb;
+  p.counters = (unsigned long long *)ctx->counters.p;
+  if (spec) {   // the list length (whole-Draw frames) and the rows claimed are known on the device only
+    p.n_tris_dev = ctx->rast_inflight.whole_draw ? p.counters + 24 : nullptr;
+    p.n_rows_dev = p.counters + 4;
+  }
+
+  // the entry value of indirectLightPowerPerArea reaches the first shaded fragment only (:585)
+  if (n > 0 && !colour && rast_indirect_entry_differs(light)) {
+    unsigned long long *first = p.counters + 9;
+    CU_CHECK(ctx, cudaMemsetAsync(first, 0xff, sizeof(unsigned long long), ctx->stream));
+    rast_first_fragment_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(p, first);
+    ctx->stats.kernel_launches++;
+    tl_mark(ctx, "rast_first_fragment_kernel");
+    p.first_frag = first;
+  }
+
+  const bool scatter = rast_scatter_path(ctx, n);
+  if (spec) ctx->rast_inflight.fast = scatter ? 1 : 0;
+  return scatter ? rast_launch_scatter(ctx, p, spec) : rast_launch_ordered(ctx, p, spec);
 }

@@ -314,7 +314,7 @@ def test_pipelined_frames_walk(b200, renderer):
         st = renderer.stats()
         # (a short list has fixed row-table space and bit-per-triangle tile lists: only its length is guessed)
         assert st["respeculated"] - before < len(poses) - 2, "small camera moves must stay pipelined"
-        # a long list with shadow volumes (ordered path, guessed row / chunk / tile-list sizes): the jump from far
+        # a long list with shadow volumes (ordered path, guessed row / tile-list sizes): the jump from far
         # away into the cloud outgrows them and the frame is rendered again
         soup = b200.scene_soup_rast(3000, edge=0.08)
         renderer.rast_upload_scene(soup, boxes)

@@ -1,7 +1,7 @@
 """Sweep of the rasteriser's triangle-loop strategies and size classes against the plain-C oracle, bit for bit.
 
 The triangle loop picks its kernels from the list length (bit-per-triangle tile lists up to 2048 triangles, then
-setup / spread / scan, and from 8193 on the row chunks handed out by the setup kernel), from each triangle's
+setup / spread / scan, and from 8193 on the owners of the row slots written by the setup kernel), from each triangle's
 footprint (the scatter path's small / big split at 24 rows and 60 columns), from shadow-volume triangles, textures
 and colour modes, from the tile size, the row band and pipelining.  Every case below is a clipped list with exact
 pixel footprints (tests/rast_sweep_cases.py); `test_sweep_reaches_every_class` checks, without a GPU, that the
@@ -73,7 +73,7 @@ CASES = [
     C("n8192_boundary", 8192, "250x170", BOUNDARY, ALL),
     C("n8192_tex", 8192, "250x170", MIXED, (AUTO, ORD16), tex=True),
     C("n8192_colour2", 8192, "250x170", MIXED, (AUTO, ORD8), colour=2),
-    # ---- over 8192: the setup kernel hands out the row chunks, one thread per triangle in the spread kernel ----
+    # ---- over 8192: the setup kernel writes the row-slot owners, one thread per triangle in the spread kernel ----
     C("n8193_big_shadow", 8193, "250x170", BIG_MIX, A_ORD, shadow=0.25),
     C("n8193_big_shadow_37x23", 8193, "37x23", BIG_MIX, A_ORD, shadow=0.25),
     C("n8193_big", 8193, "250x170", BIG_MIX, ALL),
@@ -146,7 +146,7 @@ def test_sweep_reaches_every_class():
                 mark("crowded tile", s[1])
                 if c["tex"]:
                     mark("crowded tile, textured", s[1])
-            # a range of more than 32 row chunks and of more than 32 tiles: warp_spread's cooperative branch
+            # a range of more than 32 row slots and of more than 32 tiles: warp_spread's cooperative branch
             if (s[0] == 1 and n > sc.SPREAD_BLOCK_MAX and (d["nrows"] > 32).any() and (d["tile_span"][s[1]] > 32).any()):
                 mark("over 8192, ordered, cooperative warp_spread", "big" if d["big"].any() else "",
                      "shadow" if d["shadow"].any() else "")
@@ -269,7 +269,7 @@ def check_kernels(tag, names, c, s, d):
     need("rast_short_kernel", n <= sc.BITS_MAX_TRIS)
     need("rast_setup_kernel", n > sc.BITS_MAX_TRIS); need("rast_scan_kernel", n > sc.BITS_MAX_TRIS)
     if n > sc.BITS_MAX_TRIS:
-        # fan-out: chunks + tile counts + tile lists; from 8193 triangles on the setup kernel hands out the chunks
+        # fan-out: row-slot owners + tile counts + tile lists; from 8193 triangles on the setup kernel writes the owners
         want = 2 if n > sc.SPREAD_BLOCK_MAX else 3
         assert names.count("rast_spread_kernel") == want, f"{tag}: {names.count('rast_spread_kernel')} spread launches"
     fused = path == 0 or bool(c["colour"])
