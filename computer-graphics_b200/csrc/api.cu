@@ -281,6 +281,8 @@ static int rt_frame_device(b200_ctx *ctx, const camera_t *cam, const light_t *li
   ctx->stats.kernel_launches = 0;
   CU_CHECK(ctx, cudaMemsetAsync(ctx->counters.p, 0, 32 * sizeof(unsigned long long), ctx->stream));
   CU_CHECK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  ctx->tl_n = 0;
+  tl_mark(ctx, "frame start");
   if (int rc = rt_launch(ctx, f, d_rgb, d_depth, d_index, d_argb)) return rc;
   CU_CHECK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
   uint64_t my_rows = 0;   // rows of this context's 16-row blocks
@@ -335,6 +337,8 @@ static int rt_views_device(b200_ctx *ctx, const camera_t *cams, int n_views, con
   ctx->stats.kernel_launches = 0;
   CU_CHECK(ctx, cudaMemsetAsync(ctx->counters.p, 0, 32 * sizeof(unsigned long long), ctx->stream));
   CU_CHECK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  ctx->tl_n = 0;
+  tl_mark(ctx, "frame start");
   if (int rc = rt_launch_views(ctx, fs.data(), n_views, d_rgb, d_depth, d_index, d_argb)) return rc;
   CU_CHECK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
   ctx->stats.primary_rays = (uint64_t)n_views * (uint64_t)cams[0].width * (uint64_t)cams[0].height * 9u;
@@ -429,7 +433,7 @@ static int finish_stats(b200_ctx *ctx) {
   float ms = 0.f;
   cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
   ctx->stats.gpu_ms = ms;
-  if (ctx->timeline && ctx->pending == 2 && ctx->tl_n > 1) {
+  if (ctx->timeline && ctx->pending && ctx->tl_n > 1) {
     for (int i = 1; i < ctx->tl_n; ++i) {
       float d = 0.f;
       cudaEventElapsedTime(&d, ctx->tl_ev[i - 1], ctx->tl_ev[i]);
@@ -528,6 +532,8 @@ int draw_raytrace_band(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const
   ctx->stats.kernel_launches = 0;
   CU_CHECK(ctx, cudaMemsetAsync(ctx->counters.p, 0, 32 * sizeof(unsigned long long), ctx->stream));
   CU_CHECK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  ctx->tl_n = 0;
+  tl_mark(ctx, "frame start");
   // Large frames are rendered in slices of whole 16-row blocks so that the copy of one slice to
   // the host overlaps the rendering of the next (scenes with per-frame grids: one slice, the
   // grids are built per launch).

@@ -7,8 +7,12 @@
 //   rt_filtered_kernel    (rt_filtered.cuh) the production kernel: conservative
 //                         edge-function filters decide almost every pair, the
 //                         reference arithmetic runs only where it can matter.
+//   rt_lattice_kernel     (rt_lattice_kernel.cuh) the same filters for frames whose
+//                         sample rays form a half-pixel lattice: each shared sample
+//                         ray is traced once per 16x16 pixel block.
 #include "rt_exact.cuh"
 #include "rt_filtered.cuh"
+#include "rt_lattice_kernel.cuh"
 #include "rt_grid.cuh"
 
 // ------------------------------------------------------------------------------
@@ -188,6 +192,7 @@ int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int
   if (ctx->opt_rt_bruteforce) {
     dim3 grid((f.W + 15) / 16, 2 * my_blocks);
     rt_bruteforce_kernel<<<grid, 128, 0, ctx->stream>>>(p);
+    tl_mark(ctx, "rt_bruteforce_kernel");
     ctx->stats.kernel_launches++;
     CU_CHECK(ctx, cudaGetLastError());
     return B200_OK;
@@ -212,6 +217,35 @@ static float rt_cam_dmax(const RtFrame &f) {
       }
     }
   return dmax * 1.001f + 1.0f;
+}
+
+// Whether the frame's sample directions form a half-pixel lattice (rt_lattice_kernel.cuh): dir0 depends on u only and
+// dir1 on v only (R[4] = R[1] = 0), every value is finite, and sample 2 of every pixel but the last of the band has the
+// bits of sample 0 of its right (lower) neighbour.  The kernel's own expression for dir (skeleton.cpp:126-128), one
+// rounding per operation like the device's __f*_rn (no FMA contraction on the host); O(W + rows) per launch.  With
+// R[4] = 0 the y term is a zero, which can change only the sign of a zero dir0, and no sample (dir0 - 0.5, dir0 + 0,
+// dir0 + 0.5) keeps that sign: one row stands for all (likewise x for dir1).
+static float rt_dir_host(const RtFrame &f, int r, float x, float y) {
+  const float a = f.R[r] * x, b = f.R[4 + r] * y, c = f.R[8 + r] * f.focal, d = f.R[12 + r] * 1.0f;
+  return (a + b) + (c + d);
+}
+static bool rt_lattice_exact(const RtFrame &f) {
+  if (f.R[1] != 0.0f || f.R[4] != 0.0f) return false;
+  for (int r = 0; r < 2; ++r) {   // r = 0: dir0 over the columns, r = 1: dir1 over the band's rows
+    const int lo = r ? f.row0 : 0, hi = r ? f.row1 : f.W;
+    uint32_t prev = 0;
+    for (int c = lo; c < hi; ++c) {
+      const float d = r ? rt_dir_host(f, 1, (float)(0 - f.W / 2), (float)(c - f.H / 2))
+                        : rt_dir_host(f, 0, (float)(c - f.W / 2), (float)(f.row0 - f.H / 2));
+      const float s0 = d + 0.5f * -1.0f, s1 = d + 0.5f * 0.0f, s2 = d + 0.5f * 1.0f;
+      if (!std::isfinite(s0) || !std::isfinite(s1) || !std::isfinite(s2)) return false;
+      uint32_t b0, b2;
+      memcpy(&b0, &s0, sizeof b0); memcpy(&b2, &s2, sizeof b2);
+      if (c > lo && b0 != prev) return false;
+      prev = b2;
+    }
+  }
+  return true;
 }
 
 // The camera-independent part of the plane-record preparation: scene, lights, shadow-ray bounds, buffers.
@@ -249,6 +283,7 @@ static int rt_set_smem_limits(b200_ctx *ctx) {
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_views_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_views_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_lattice_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_LAT_SMEM));
   ctx->rt_grid_smem_set = 1;
   return B200_OK;
 }
@@ -278,6 +313,7 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
     q.dmax = rt_cam_dmax(f);   // over the band
     dim3 grid((n + 127) / 128, 1 + f.n_lights);
     rt_prep_planes_kernel<<<grid, 128, 0, ctx->stream>>>(q);
+    tl_mark(ctx, "rt_prep_planes_kernel");
     ctx->stats.kernel_launches++;
     CU_CHECK(ctx, cudaGetLastError());
   }
@@ -386,11 +422,16 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
       rt_filtered_kernel<true, true><<<lgrid, RT_THREADS, gsmem, ctx->stream>>>(p);
     else
       rt_filtered_kernel<false, true><<<lgrid, RT_THREADS, gsmem, ctx->stream>>>(p);
+    tl_mark(ctx, "rt_filtered_kernel<grid>");
+  } else if (f.n_lights <= 1 && rt_lattice_exact(f)) {
+    rt_lattice_kernel<<<grid, RT_THREADS, RT_LAT_SMEM, ctx->stream>>>(p);
+    tl_mark(ctx, "rt_lattice_kernel");
   } else {
     if (f.n_lights > 1)
       rt_filtered_kernel<true, false><<<grid, RT_THREADS, smem, ctx->stream>>>(p);
     else
       rt_filtered_kernel<false, false><<<grid, RT_THREADS, smem, ctx->stream>>>(p);
+    tl_mark(ctx, "rt_filtered_kernel");
   }
   ctx->stats.kernel_launches++;
   CU_CHECK(ctx, cudaGetLastError());
@@ -474,6 +515,7 @@ int rt_launch_views(b200_ctx *ctx, const RtFrame *fs, int n_views, float *d_rgb,
       rt_filtered_views_kernel<true><<<grid, RT_THREADS, RT_STREAM_SMEM, ctx->stream>>>(p, v);
     else
       rt_filtered_views_kernel<false><<<grid, RT_THREADS, RT_STREAM_SMEM, ctx->stream>>>(p, v);
+    tl_mark(ctx, "rt_filtered_views_kernel");
     ctx->stats.kernel_launches++;
     CU_CHECK(ctx, cudaGetLastError());
   }
