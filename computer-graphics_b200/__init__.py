@@ -67,6 +67,23 @@ class RastTextures(ctypes.Structure):
                 ("woven_normal", RastImage)]
 
 
+class RtRay(ctypes.Structure):
+    """rt_ray: the (start, dir) arguments of ClosestIntersection (32 bytes)."""
+    _fields_ = [("start", ctypes.c_float * 4), ("dir", ctypes.c_float * 4)]
+
+
+class RtIntersection(ctypes.Structure):
+    """rt_intersection: the reference's `struct Intersection` (28 bytes, offsets 0 / 16 / 20 / 24)."""
+    _fields_ = [("position", ctypes.c_float * 4), ("distance", ctypes.c_float),
+                ("triangle_index", ctypes.c_int32), ("sphere_index", ctypes.c_int32)]
+
+
+# numpy views of the same layouts
+RT_RAY = np.dtype([("start", "<f4", 4), ("dir", "<f4", 4)])
+RT_INTERSECTION = np.dtype([("position", "<f4", 4), ("distance", "<f4"), ("triangle_index", "<i4"),
+                            ("sphere_index", "<i4")])
+
+
 class Stats(ctypes.Structure):
     _fields_ = [("primary_rays", ctypes.c_uint64), ("shadow_rays", ctypes.c_uint64),
                 ("prim_tests", ctypes.c_uint64), ("exact_evals", ctypes.c_uint64),
@@ -87,6 +104,7 @@ ABI_SYMBOLS = [
     "render_raytrace", "render_raytrace_band", "draw_raytrace", "draw_raytrace_band",
     "b200_measure_fp32_peak", "rt_upload_scene", "rt_render_device",
     "render_raytrace_views", "draw_raytrace_views", "rt_render_views_device",
+    "rt_closest_hits", "rt_occluded", "rt_closest_hits_device", "rt_occluded_device",
     "render_raster_clipped", "render_raster", "render_raster_band", "draw_raster", "raster_read_buffers",
     "raster_read_clipped", "rast_upload_clipped", "rast_render_device", "draw_raster_band",
     "rast_upload_scene", "rast_draw_device", "rast_set_textures",
@@ -107,6 +125,11 @@ def load_library():
         _lib = ctypes.CDLL(LIB_PATH)
         _lib.b200_last_error.restype = ctypes.c_char_p
         _lib.b200_stream.restype = ctypes.c_void_p
+        vp, i32 = ctypes.c_void_p, ctypes.c_int
+        _lib.rt_closest_hits.argtypes = [vp, vp, i32, vp, i32, vp, i32, vp]
+        _lib.rt_occluded.argtypes = [vp, vp, i32, vp, i32, vp, vp, i32, vp]
+        _lib.rt_closest_hits_device.argtypes = [vp, vp, i32, vp]
+        _lib.rt_occluded_device.argtypes = [vp, vp, vp, i32, vp]
     return _lib
 
 
@@ -303,6 +326,48 @@ class Renderer:
         rc = self.lib.rt_render_views_device(self.ctx, ca, int(k), la, len(lights), _ptr(d_rgb), _ptr(d_depth),
                                              _ptr(d_index), _ptr(d_argb))
         self._check(rc, "rt_render_views_device")
+
+    # ---- RT, ray queries --------------------------------------------------------
+    @staticmethod
+    def _rays(rays):
+        """rays: an RT_RAY array, or (n, 8) float32 (start xyzw, dir xyzw)."""
+        rays = np.ascontiguousarray(rays)
+        if rays.dtype != RT_RAY:
+            rays = np.ascontiguousarray(rays, np.float32).reshape(-1, 8).view(RT_RAY).reshape(-1)
+        return rays
+
+    def rt_closest_hits(self, tris, spheres, rays):
+        """ClosestIntersection for every ray: dict of numpy arrays position (n, 4), distance, triangle_index and
+        sphere_index (distance < FLT_MAX iff the ray hit something)."""
+        rays = self._rays(rays)
+        out = np.zeros(len(rays), RT_INTERSECTION)
+        rc = self.lib.rt_closest_hits(self.ctx, _ptr(tris), 0 if tris is None else len(tris), _ptr(spheres),
+                                      0 if spheres is None else len(spheres), _ptr(rays), len(rays), _ptr(out))
+        self._check(rc, "rt_closest_hits")
+        return dict(position=out["position"].copy(), distance=out["distance"].copy(),
+                    triangle_index=out["triangle_index"].copy(), sphere_index=out["sphere_index"].copy())
+
+    def rt_occluded(self, tris, spheres, rays, max_distance):
+        """DirectLight's shadow test for every ray: bool array, ClosestIntersection && distance < max_distance."""
+        rays = self._rays(rays)
+        md = np.ascontiguousarray(max_distance, np.float32).reshape(-1)
+        if len(md) != len(rays):
+            raise ValueError("one max_distance per ray")
+        out = np.zeros(len(rays), np.uint8)
+        rc = self.lib.rt_occluded(self.ctx, _ptr(tris), 0 if tris is None else len(tris), _ptr(spheres),
+                                  0 if spheres is None else len(spheres), _ptr(rays), _ptr(md), len(rays), _ptr(out))
+        self._check(rc, "rt_occluded")
+        return out.astype(bool)
+
+    def rt_closest_hits_device(self, d_rays, n_rays, d_out):
+        """Device pointers (ints): n_rays rt_ray in, rt_intersection out; the scene of rt_upload_scene; asynchronous."""
+        self._check(self.lib.rt_closest_hits_device(self.ctx, _ptr(d_rays), int(n_rays), _ptr(d_out)),
+                    "rt_closest_hits_device")
+
+    def rt_occluded_device(self, d_rays, d_max_distance, n_rays, d_out):
+        """Device pointers (ints): rt_ray and float limits in, one byte per ray out; asynchronous."""
+        self._check(self.lib.rt_occluded_device(self.ctx, _ptr(d_rays), _ptr(d_max_distance), int(n_rays),
+                                                _ptr(d_out)), "rt_occluded_device")
 
     # ---- RAST ----------------------------------------------------------------
     def render_raster_clipped(self, clipped, cam, light, want=("rgb", "depth", "index")):

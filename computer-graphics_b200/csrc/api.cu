@@ -105,7 +105,7 @@ void b200_destroy(b200_ctx *ctx) {
                     &ctx->rast_tmp, &ctx->rast_keys, &ctx->rast_trimeta, &ctx->rast_big, &ctx->rast_orig, &ctx->rast_shadow8, &ctx->rast_srowsB, &ctx->rast_srowsL, &ctx->rast_row_owner, &ctx->rast_world, &ctx->rast_geom_tmp, &ctx->rast_screen, &ctx->rast_low, &ctx->rast_high, &ctx->rast_shadow,
                     &ctx->rast_depth, &ctx->rast_index, &ctx->out_rgb, &ctx->out_depth, &ctx->out_index,
                     &ctx->out_argb, &ctx->counters, &ctx->rt_plan, &ctx->rt_cell_pairs, &ctx->rast_tex_images, &ctx->rast_tex_noise,
-                    &ctx->rast_colour_keys, &ctx->rast_colour_rgb, &ctx->rast_colour_tmp};
+                    &ctx->rast_colour_keys, &ctx->rast_colour_rgb, &ctx->rast_colour_tmp, &ctx->rt_query};
   for (DevBuf *b : bufs) if (b->p) cudaFree(b->p);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
   cudaEventDestroy(ctx->ev0);
@@ -399,6 +399,101 @@ int draw_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, cons
                        nullptr, argb_out);
 }
 
+}  // extern "C"
+
+// ---- RT, ray queries: ClosestIntersection / DirectLight's shadow test for caller-supplied rays --------------
+static int check_ray_buffers(b200_ctx *ctx, const void *rays, const float *max_distance, int n_rays, const void *out,
+                             bool occlusion) {
+  if (n_rays < 0) return ctx_fail(ctx, B200_EINVAL, "negative ray count");
+  if (n_rays > 0 && (!rays || !out || (occlusion && !max_distance)))
+    return ctx_fail(ctx, B200_EINVAL, "null rays, limits or output");
+  return B200_OK;
+}
+
+// (also the multi-GPU context's check, before the rays are shared out)
+int check_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+               const rt_ray *rays, const float *max_distance, int n_rays, const void *out, bool occlusion) {
+  if (n_tris < 0 || n_spheres < 0 || (n_tris > 0 && !tris) || (n_spheres > 0 && !spheres))
+    return ctx_fail(ctx, B200_EINVAL, "bad scene arguments");
+  return check_ray_buffers(ctx, rays, max_distance, n_rays, out, occlusion);
+}
+
+// One query on device buffers and the uploaded scene: d_hits for closest hits, d_occ (+ d_max) for occlusion.
+static int rt_query_device(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max, int n_rays, rt_intersection *d_hits,
+                           uint8_t *d_occ) {
+  cudaSetDevice(ctx->device);
+  if (ctx->rast_inflight.active) if (int rc = finish_stats(ctx)) return rc;   // the counters are shared
+  ctx->stats.kernel_launches = 0;
+  CU_CHECK(ctx, cudaMemsetAsync(ctx->counters.p, 0, 32 * sizeof(unsigned long long), ctx->stream));
+  CU_CHECK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  ctx->tl_n = 0;
+  tl_mark(ctx, "query start");
+  if (int rc = rt_launch_rays(ctx, d_rays, d_max, n_rays, d_hits, d_occ)) return rc;
+  CU_CHECK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  ctx->stats.primary_rays = d_occ ? 0 : (uint64_t)n_rays;
+  ctx->stats.shadow_rays = d_occ ? (uint64_t)n_rays : 0;
+  if (int rc = enqueue_counter_readback(ctx)) return rc;
+  ctx->pending = 3;
+  return B200_OK;
+}
+
+// The host-pointer query entries: rays (and limits) to a staging buffer, the query, the results back.
+static int rt_query_host(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                         const rt_ray *rays, const float *max_distance, int n_rays, rt_intersection *out,
+                         uint8_t *occ_out, bool occlusion) {
+  if (int rc = check_rays(ctx, tris, n_tris, spheres, n_spheres, rays, max_distance, n_rays,
+                          occlusion ? (const void *)occ_out : (const void *)out, occlusion))
+    return rc;
+  if (n_rays == 0) return B200_OK;
+  if (int rc = rt_upload_scene(ctx, tris, n_tris, spheres, n_spheres)) return rc;
+  const size_t n = (size_t)n_rays;
+  const size_t off_max = n * sizeof(rt_ray), off_out = (off_max + n * sizeof(float) + 255) & ~(size_t)255;
+  const size_t out_bytes = occlusion ? n : n * sizeof(rt_intersection);
+  if (int rc = ensure(ctx, ctx->rt_query, off_out + out_bytes)) return rc;
+  char *buf = (char *)ctx->rt_query.p;
+  CU_CHECK(ctx, cudaMemcpyAsync(buf, rays, n * sizeof(rt_ray), cudaMemcpyHostToDevice, ctx->stream));
+  if (occlusion)
+    CU_CHECK(ctx, cudaMemcpyAsync(buf + off_max, max_distance, n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+  if (int rc = rt_query_device(ctx, (const rt_ray *)buf, occlusion ? (const float *)(buf + off_max) : nullptr, n_rays,
+                               occlusion ? nullptr : (rt_intersection *)(buf + off_out),
+                               occlusion ? (uint8_t *)(buf + off_out) : nullptr))
+    return rc;
+  if (int rc = copy_out(ctx, occlusion ? (void *)occ_out : (void *)out, buf + off_out, out_bytes)) return rc;
+  return finish_stats(ctx);
+}
+
+extern "C" {
+
+int rt_closest_hits(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                    const rt_ray *rays, int n_rays, rt_intersection *out) {
+  if (!ctx) return B200_EINVAL;
+  if (ctx->multi) return multi_rays(ctx, tris, n_tris, spheres, n_spheres, rays, nullptr, n_rays, out, nullptr, false);
+  return rt_query_host(ctx, tris, n_tris, spheres, n_spheres, rays, nullptr, n_rays, out, nullptr, false);
+}
+
+int rt_occluded(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                const rt_ray *rays, const float *max_distance, int n_rays, uint8_t *out) {
+  if (!ctx) return B200_EINVAL;
+  if (ctx->multi) return multi_rays(ctx, tris, n_tris, spheres, n_spheres, rays, max_distance, n_rays, nullptr, out, true);
+  return rt_query_host(ctx, tris, n_tris, spheres, n_spheres, rays, max_distance, n_rays, nullptr, out, true);
+}
+
+int rt_closest_hits_device(b200_ctx *ctx, const rt_ray *d_rays, int n_rays, rt_intersection *d_out) {
+  if (!ctx) return B200_EINVAL;
+  SINGLE_ONLY(ctx);
+  if (int rc = check_ray_buffers(ctx, d_rays, nullptr, n_rays, d_out, false)) return rc;
+  if (n_rays == 0) return B200_OK;
+  return rt_query_device(ctx, d_rays, nullptr, n_rays, d_out, nullptr);
+}
+
+int rt_occluded_device(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max_distance, int n_rays, uint8_t *d_out) {
+  if (!ctx) return B200_EINVAL;
+  SINGLE_ONLY(ctx);
+  if (int rc = check_ray_buffers(ctx, d_rays, d_max_distance, n_rays, d_out, true)) return rc;
+  if (n_rays == 0) return B200_OK;
+  return rt_query_device(ctx, d_rays, d_max_distance, n_rays, nullptr, d_out);
+}
+
 static int rast_frame(b200_ctx *ctx, bool whole_draw, const camera_t *cam, const rast_light_t *light, int row_begin,
                       int row_end, float *d_rgb, float *d_depth, int32_t *d_index, uint32_t *d_argb, bool allow_spec);
 
@@ -441,8 +536,8 @@ static int finish_stats(b200_ctx *ctx) {
     }
     fprintf(stderr, "[b200 timeline] frame %.1f us\n", ms * 1000.f);
   }
-  if (ctx->pending == 1) {
-    ctx->stats.shadow_rays = c[0];
+  if (ctx->pending == 1 || ctx->pending == 3) {
+    if (ctx->pending == 1) ctx->stats.shadow_rays = c[0];   // a ray query (3) set its ray counts when it was enqueued
     ctx->stats.exact_evals = c[1];
     ctx->stats.prim_tests = (ctx->stats.primary_rays + ctx->stats.shadow_rays) *
                             (uint64_t)(ctx->rt_n_tris + ctx->rt_n_spheres);

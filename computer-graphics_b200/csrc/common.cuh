@@ -129,6 +129,7 @@ struct b200_ctx {
   int rt_bounds_on_device = 0;
   DevBuf rt_cells;    // direction grids: per-cell counts, cursors, padded counts, offsets, scan scratch
   DevBuf rt_cell_rec, rt_cell_idx;   // the cells' lists: plane records and triangle indices
+  DevBuf rt_query;   // host-pointer ray queries: rays, limits and results (rt_closest_hits, rt_occluded)
   DevBuf rt_plan;                    // gridded frames: two per-block cost arrays, the block plan, its length (rt_plan_kernel)
   unsigned long long rt_plan_shape = 0;
   int rt_plan_valid = 0, rt_plan_flip = 0;
@@ -144,7 +145,7 @@ struct b200_ctx {
   int rt_n_tris = 0, rt_n_spheres = 0;
   float rt_world_abs = 0.f;   // max |coordinate| over the uploaded scene
   float rt_normal_abs = 1.f;  // max(1, max |normal component|): scales the 1e-5 * normal shadow-ray offset (:394)
-  int pending = 0;            // 1 = RT, 2 = RAST render whose counters are not read back yet
+  int pending = 0;            // 1 = RT, 2 = RAST render, 3 = RT ray query whose counters are not read back yet
 
   // RAST scene (device)
   DevBuf rast_src;    // rast_triangle[n] clipped list
@@ -267,6 +268,9 @@ static inline int band_slice_edge(int row0, int rows, int i, int k, int align) {
 }
 int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int32_t *d_index,
               uint32_t *d_argb);
+// rt_rays.cu: one ray query on the uploaded scene, n > 0 rays; d_hits (closest hits) or d_occ + d_max (occlusion)
+int rt_launch_rays(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max, int n, rt_intersection *d_hits,
+                   uint8_t *d_occ);
 // whole frames of n_views cameras of one size, frame k of each output at k * W * H (rgb: times 3)
 int rt_launch_views(b200_ctx *ctx, const RtFrame *fs, int n_views, float *d_rgb, float *d_depth, int32_t *d_index,
                     uint32_t *d_argb);
@@ -282,6 +286,12 @@ int multi_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, con
                          const camera_t *cams, int n_views, const light_t *lights, int n_lights, float *rgb_out,
                          float *depth_out, int32_t *index_out, uint32_t *argb_out);
 int check_views(b200_ctx *ctx, const camera_t *cams, int n_views, const light_t *lights, int n_lights);   // api.cu
+// ray queries: max_distance / occ_out for an occlusion query, out for a closest-hit query
+int multi_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+               const rt_ray *rays, const float *max_distance, int n_rays, rt_intersection *out, uint8_t *occ_out,
+               bool occlusion);
+int check_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+               const rt_ray *rays, const float *max_distance, int n_rays, const void *out, bool occlusion);   // api.cu
 int multi_raster(b200_ctx *ctx, const rast_triangle *room, int n_room, const rast_triangle *boxes, int n_boxes,
                  const camera_t *cam, const rast_light_t *light, int row_begin, int row_end, float *rgb_out,
                  float *depth_out, int32_t *index_out, uint32_t *argb_out);

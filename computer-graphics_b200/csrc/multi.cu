@@ -336,6 +336,30 @@ int multi_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, con
   return B200_OK;
 }
 
+// Ray queries: device i answers the contiguous run [k_i, k_i+1) of the rays with the single-device entry and returns
+// it straight into its slice of the caller's output, as multi_raytrace_views does with views.
+int multi_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+               const rt_ray *rays, const float *max_distance, int n_rays, rt_intersection *out, uint8_t *occ_out,
+               bool occlusion) {
+  b200_multi *mc = ctx->multi;
+  if (int rc = check_rays(ctx, tris, n_tris, spheres, n_spheres, rays, max_distance, n_rays,
+                          occlusion ? (const void *)occ_out : (const void *)out, occlusion))
+    return rc;
+  if (n_rays == 0) return B200_OK;
+  const int n = mc->n;
+  const int rc = multi_run(ctx, [&](int i) -> int {
+    const int a = (int)((long long)n_rays * i / n), b = (int)((long long)n_rays * (i + 1) / n);
+    b200_ctx *c = mc->child[i];
+    c->stats = b200_stats{};
+    if (b <= a) return B200_OK;
+    if (occlusion) return rt_occluded(c, tris, n_tris, spheres, n_spheres, rays + a, max_distance + a, b - a, occ_out + a);
+    return rt_closest_hits(c, tris, n_tris, spheres, n_spheres, rays + a, b - a, out + a);
+  });
+  if (rc != B200_OK) return rc;
+  multi_sum_stats(ctx);
+  return B200_OK;
+}
+
 // ---- rasteriser -------------------------------------------------------------------------
 // Every device keeps its own copy of the images (each over its own PCIe link).
 int multi_rast_set_textures(b200_ctx *ctx, const rast_textures_t *tex) {

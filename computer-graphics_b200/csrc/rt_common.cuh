@@ -1,6 +1,7 @@
 // Kernel parameters and per-pixel epilogue shared by the two raytracer kernels.
 #pragma once
 #include "common.cuh"
+#include "rt_exact.cuh"
 
 struct RtKParams {
   float cam[4];
@@ -74,4 +75,19 @@ __device__ __forceinline__ void rt_count(unsigned long long *counter, unsigned l
 
 __device__ __forceinline__ void rt_count_shadow(const RtKParams &p, unsigned long long n) {
   rt_count(p.counters + 0, n);
+}
+
+// ClosestIntersection (skeleton.cpp:263-363) by brute force: the reference arithmetic on every triangle, then every
+// sphere (rt_bruteforce_kernel, rt_rays_bruteforce_kernel).
+__device__ __forceinline__ RtHit rt_closest_bruteforce(const RtKParams &p, float sx, float sy, float sz,
+                                                       float dx, float dy, float dz) {
+  RtHit best;
+  best.t = 0.f; best.dist = FLT_MAX; best.idx = 0;
+  const float len = xsqrt(xdot3(dx, dy, dz, dx, dy, dz));  // glm::length(dir3), :307
+  for (int i = 0; i < p.n_tris; ++i) {
+    const float4 g0 = __ldg(p.geom + 3 * i), g1 = __ldg(p.geom + 3 * i + 1), g2 = __ldg(p.geom + 3 * i + 2);
+    rt_exact_triangle(sx, sy, sz, dx, dy, dz, len, g0, g1, g2, i, best);
+  }
+  rt_exact_spheres(p.sph, p.n_sph, sx, sy, sz, dx, dy, dz, best);
+  return best;
 }

@@ -30,6 +30,7 @@
 #pragma once
 #include "rt_common.cuh"
 #include "rt_exact.cuh"
+#include "rt_tma.cuh"
 
 constexpr int RT_TILE = 256;      // triangles per shared-memory tile
 constexpr int RT_THREADS = 256;   // 8 warps: a 16x16 pixel block
@@ -41,41 +42,6 @@ constexpr int RT_WTILE = 64;               // records per tile of a warp's priva
 constexpr int RT_GRID_MAX_CELLS = 96;      // shadow phase: distinct cells one warp (8x4 pixels, 288 rays) may walk, else it streams the scene
 constexpr int RT_GRID_TABLE_LOG2 = 8;      // hash set used to collect them
 constexpr int RT_SEEN_LOG2 = 8, RT_SEEN = 1 << RT_SEEN_LOG2;   // per-warp set of triangles already met in this light phase
-
-// ---- mbarrier / TMA bulk-copy primitives (sm_90+/sm_100a PTX) ------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint64_t *bar, int count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_fence_init() {
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "WAIT_%=:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-      "@p bra DONE_%=;\n"
-      "bra WAIT_%=;\n"
-      "DONE_%=:\n"
-      "}\n" ::"r"(smem_u32(bar)), "r"(parity)
-      : "memory");
-}
-// 1-D bulk copy global -> shared, completion signalled on the mbarrier.
-__device__ __forceinline__ void tma_bulk_g2s(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-          smem_u32(dst)),
-      "l"(src), "r"(bytes), "r"(smem_u32(bar))
-      : "memory");
-}
 
 // ---- per-frame plane records ------------------------------------------------------
 // origin 0 = camera (directions (dx, dy, f): the z term is folded into a constant)
@@ -219,18 +185,6 @@ __global__ void rt_prep_planes_kernel(const __grid_constant__ RtPrepParams p) { 
 // p.cam / p.focal / p.dmax unused: per view in v
 __global__ void rt_prep_planes_views_kernel(const __grid_constant__ RtPrepParams p, const __grid_constant__ RtPrepViews v) {
   rt_prep_planes_body<true>(p, &v);
-}
-
-// ---- warp helpers -------------------------------------------------------------------
-__device__ __forceinline__ float warp_min(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fminf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
 }
 
 // ---- bundle-box tests shared by the render kernel (L0) and the grid builder -------

@@ -64,19 +64,6 @@ __global__ void rt_prep_geom_kernel(const rt_triangle *__restrict__ src, int n, 
 // ------------------------------------------------------------------------------
 // brute force, reference arithmetic everywhere
 // ------------------------------------------------------------------------------
-__device__ __forceinline__ RtHit rt_closest_bruteforce(const RtKParams &p, float sx, float sy, float sz,
-                                                       float dx, float dy, float dz) {
-  RtHit best;
-  best.t = 0.f; best.dist = FLT_MAX; best.idx = 0;
-  const float len = xsqrt(xdot3(dx, dy, dz, dx, dy, dz));  // glm::length(dir3), :307
-  for (int i = 0; i < p.n_tris; ++i) {
-    const float4 g0 = __ldg(p.geom + 3 * i), g1 = __ldg(p.geom + 3 * i + 1), g2 = __ldg(p.geom + 3 * i + 2);
-    rt_exact_triangle(sx, sy, sz, dx, dy, dz, len, g0, g1, g2, i, best);
-  }
-  rt_exact_spheres(p.sph, p.n_sph, sx, sy, sz, dx, dy, dz, best);
-  return best;
-}
-
 __global__ void __launch_bounds__(128) rt_bruteforce_kernel(const __grid_constant__ RtKParams p) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   // each warp owns an 8x4 pixel patch; a 128-thread block covers 16x8 pixels

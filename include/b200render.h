@@ -132,7 +132,9 @@ int b200_set_stream(b200_ctx *ctx, void *cuda_stream);
 
 /* Tunables.  B200_OPT_RT_BRUTEFORCE = 1 switches the raytracer to the
  * unfiltered kernel that runs the reference arithmetic on every ray/triangle
- * pair (on-device cross-check of the filtered kernel; results are identical). */
+ * pair (on-device cross-check of the filtered kernel; results are identical).
+ * It also switches the ray queries (rt_closest_hits, rt_occluded) to the
+ * per-ray exact loop over every pair, without cull or early exit. */
 #define B200_OPT_RT_BRUTEFORCE 1
 #define B200_OPT_RAST_TILE_LOG2 2   /* ordered-tile path: log2 of the screen-tile edge, 3..5 (default 5) */
 /* Rasteriser strategy: 0 = automatic, 1 = ordered screen tiles (any list; keeps
@@ -275,6 +277,57 @@ int draw_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, cons
 int rt_render_views_device(b200_ctx *ctx, const camera_t *cams, int n_views, const light_t *lights,
                            int n_lights, float *d_rgb, float *d_depth, int32_t *d_index,
                            uint32_t *d_argb);
+
+/* ---- RT, ray queries: ClosestIntersection for rays the caller supplies --------
+ * raytracer/Source/skeleton.cpp:40-45 (struct Intersection), :263-363 (ClosestIntersection) and
+ * :394-397 (DirectLight's shadow test `ClosestIntersection(...) && distance < r_mag`), for any rays:
+ * picking from any point, visibility between two points, other sampling patterns, code that calls
+ * ClosestIntersection directly.  Every result is bit-identical to the reference's.
+ *   - One thread per ray, in the caller's order.  There is no spatial index: the cost of a call is
+ *     rays x (triangles + spheres) minus what a per-warp cull removes; coherent rays (neighbouring
+ *     pixels, shadow rays of neighbouring points) cull far better than incoherent ones.  Scenes of
+ *     1024 triangles or more stream all their triangles like small ones.
+ *   - n_rays < 0, a null rays / out / max_distance with n_rays > 0, or bad scene arguments:
+ *     B200_EINVAL.  n_rays == 0: B200_OK, nothing written.  An empty scene misses everywhere.
+ *   - b200_get_stats afterwards: primary_rays = n_rays (closest) or shadow_rays = n_rays (occlusion),
+ *     prim_tests = n_rays * (n_tris + n_spheres), exact_evals = ray/triangle pairs that ran the
+ *     reference arithmetic, kernel_launches and gpu_ms as for frames.
+ *   - B200_OPT_RT_BRUTEFORCE = 1: the per-ray exact loop over every pair (on-device cross-check).
+ *   - A query leaves the context as it was for the next frame (pixels, the gridded-frame block plan
+ *     of B200_OPT_RT_PLAN); a pipelined raster frame in flight is finished first.
+ *   - On a b200_init_multi context the host-pointer entries give each device a contiguous run of the
+ *     rays, returned straight into its slice of out; the _device entries return B200_EINVAL there. */
+
+/* The (start, dir) arguments of ClosestIntersection: 32 bytes.  Only xyz of dir is read
+ * (glm::length(dir3) :307, mat3(-dir, e1, e2) :289); start.w only reaches position.w. */
+typedef struct rt_ray {
+  float start[4];
+  float dir[4];
+} rt_ray;
+
+/* raytracer/Source/skeleton.cpp:40-45 `struct Intersection`: 28 bytes, offsets 0 / 16 / 20 / 24. */
+typedef struct rt_intersection {
+  float position[4];       /* start + vec4(t * dir3, 0): position.w = start.w + 0.0f (so -0 becomes +0) */
+  float distance;          /* t * |dir3| for triangles, the raw t for spheres (:350); FLT_MAX on a miss  */
+  int32_t triangle_index;  /* -1 when a sphere or nothing was hit                                      */
+  int32_t sphere_index;    /* -1 when a triangle or nothing was hit                                    */
+} rt_intersection;
+
+/* out[i] = the Intersection ClosestIntersection(rays[i].start, rays[i].dir, ...) leaves behind.  A ray
+ * hit something iff distance < FLT_MAX; on a miss the reference leaves every other field untouched,
+ * and the library sets position to 0 and both indices to -1.  Host pointers; uploads the scene like
+ * render_raytrace. */
+int rt_closest_hits(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres,
+                    int n_spheres, const rt_ray *rays, int n_rays, rt_intersection *out);
+/* out[i] = 1 iff ClosestIntersection returns true AND distance < max_distance[i] (DirectLight's shadow
+ * test, :394-397, sphere distances included as the reference has them); a NaN or non-positive limit
+ * gives 0.  Host pointers. */
+int rt_occluded(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres,
+                int n_spheres, const rt_ray *rays, const float *max_distance, int n_rays, uint8_t *out);
+/* Device-resident: the scene of rt_upload_scene, DEVICE pointers, asynchronous on b200_stream(ctx). */
+int rt_closest_hits_device(b200_ctx *ctx, const rt_ray *d_rays, int n_rays, rt_intersection *d_out);
+int rt_occluded_device(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max_distance, int n_rays,
+                       uint8_t *d_out);
 
 /* ---- RAST: replaces rasteriser Draw(screen*) (skeleton.cpp:203-308) --------*/
 
