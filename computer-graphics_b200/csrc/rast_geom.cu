@@ -120,7 +120,7 @@ __global__ void __launch_bounds__(128) rast_geom_kernel(const __grid_constant__ 
       for (int k = 0; k < 3; ++k) {
         const GV &v = cur[i].v[k];
         const float y = xadd(xmul(p.x.focal, xdiv(v.y, v.z)), (float)(p.x.H / 2));   // :513
-        ok = ok && fabsf(y) < 8.0e6f;                       // not convertible: the triangle loop drops it
+        ok = ok && fabsf(y) < 2147483648.0f;                // not convertible: the triangle loop drops it (rast_vertex)
         const int yi = ok ? (int)y : 0;                     // :516 static_cast<int>
         ymin = min(ymin, yi); ymax = max(ymax, yi);
       }
@@ -189,11 +189,11 @@ __global__ void __launch_bounds__(128) rast_geom_kernel(const __grid_constant__ 
     if (kept) {
       float *o = reinterpret_cast<float *>(stage) + slot * TW;
       const GTri &g = cur[0];
-      o[0] = g.v[0].x; o[1] = g.v[0].y; o[2] = g.v[0].z; o[3] = g.v[0].w;
-      o[4] = g.v[1].x; o[5] = g.v[1].y; o[6] = g.v[1].z; o[7] = g.v[1].w;
-      o[8] = g.v[2].x; o[9] = g.v[2].y; o[10] = g.v[2].z; o[11] = g.v[2].w;
+      o[0] = x86_nan(g.v[0].x); o[1] = x86_nan(g.v[0].y); o[2] = x86_nan(g.v[0].z); o[3] = x86_nan(g.v[0].w);
+      o[4] = x86_nan(g.v[1].x); o[5] = x86_nan(g.v[1].y); o[6] = x86_nan(g.v[1].z); o[7] = x86_nan(g.v[1].w);
+      o[8] = x86_nan(g.v[2].x); o[9] = x86_nan(g.v[2].y); o[10] = x86_nan(g.v[2].z); o[11] = x86_nan(g.v[2].w);
 #pragma unroll
-      for (int k = 0; k < 9; ++k) o[12 + k] = attr[k];
+      for (int k = 0; k < 9; ++k) o[12 + k] = attr[k];   // (room triangles: the caller's attributes)
       if (MODE == 2 && p.orig && my_off < p.out_cap) p.orig[my_off] = (int)my_all;
     }
     const unsigned n_out = MODE == 2 ? (s_warp[0] + s_warp[1] + s_warp[2] + s_warp[3]) >> 16 : (unsigned)GT;
@@ -210,11 +210,11 @@ __global__ void __launch_bounds__(128) rast_geom_kernel(const __grid_constant__ 
     if (off >= p.out_cap) break;
     rast_triangle *o = p.out + off;
     const GTri &g = cur[i];
-    o->v0[0] = g.v[0].x; o->v0[1] = g.v[0].y; o->v0[2] = g.v[0].z; o->v0[3] = g.v[0].w;
-    o->v1[0] = g.v[1].x; o->v1[1] = g.v[1].y; o->v1[2] = g.v[1].z; o->v1[3] = g.v[1].w;
-    o->v2[0] = g.v[2].x; o->v2[1] = g.v[2].y; o->v2[2] = g.v[2].z; o->v2[3] = g.v[2].w;
+    o->v0[0] = x86_nan(g.v[0].x); o->v0[1] = x86_nan(g.v[0].y); o->v0[2] = x86_nan(g.v[0].z); o->v0[3] = x86_nan(g.v[0].w);
+    o->v1[0] = x86_nan(g.v[1].x); o->v1[1] = x86_nan(g.v[1].y); o->v1[2] = x86_nan(g.v[1].z); o->v1[3] = x86_nan(g.v[1].w);
+    o->v2[0] = x86_nan(g.v[2].x); o->v2[1] = x86_nan(g.v[2].y); o->v2[2] = x86_nan(g.v[2].z); o->v2[3] = x86_nan(g.v[2].w);
 #pragma unroll
-    for (int k = 0; k < 4; ++k) o->normal[k] = attr[k];
+    for (int k = 0; k < 4; ++k) o->normal[k] = s ? x86_nan(attr[k]) : attr[k];
 #pragma unroll
     for (int k = 0; k < 3; ++k) o->color[k] = attr[4 + k];
     o->texture = __float_as_int(attr[7]);
@@ -324,11 +324,11 @@ __global__ void __launch_bounds__(32 * GW_WARPS) rast_geom_warp_kernel(const __g
   const unsigned off = s_prefix + before + (unsigned)lane;
   if (j < n_pre && lane < n_cur && off < p.out_cap) {
     rast_triangle *o = p.out + off;
-    o->v0[0] = mine.v[0].x; o->v0[1] = mine.v[0].y; o->v0[2] = mine.v[0].z; o->v0[3] = mine.v[0].w;
-    o->v1[0] = mine.v[1].x; o->v1[1] = mine.v[1].y; o->v1[2] = mine.v[1].z; o->v1[3] = mine.v[1].w;
-    o->v2[0] = mine.v[2].x; o->v2[1] = mine.v[2].y; o->v2[2] = mine.v[2].z; o->v2[3] = mine.v[2].w;
+    o->v0[0] = x86_nan(mine.v[0].x); o->v0[1] = x86_nan(mine.v[0].y); o->v0[2] = x86_nan(mine.v[0].z); o->v0[3] = x86_nan(mine.v[0].w);
+    o->v1[0] = x86_nan(mine.v[1].x); o->v1[1] = x86_nan(mine.v[1].y); o->v1[2] = x86_nan(mine.v[1].z); o->v1[3] = x86_nan(mine.v[1].w);
+    o->v2[0] = x86_nan(mine.v[2].x); o->v2[1] = x86_nan(mine.v[2].y); o->v2[2] = x86_nan(mine.v[2].z); o->v2[3] = x86_nan(mine.v[2].w);
 #pragma unroll
-    for (int k = 0; k < 4; ++k) o->normal[k] = attr[k];
+    for (int k = 0; k < 4; ++k) o->normal[k] = s ? x86_nan(attr[k]) : attr[k];
 #pragma unroll
     for (int k = 0; k < 3; ++k) o->color[k] = attr[4 + k];
     o->texture = __float_as_int(attr[7]);

@@ -140,9 +140,11 @@ __device__ __forceinline__ unsigned rast_count_rows(const RastParams &p) {
 __device__ __forceinline__ bool rast_vertex(const float *v, float focal, int W, int H, RastVtx &o) {
   const float x = xadd(xmul(focal, xdiv(v[0], v[2])), (float)(W / 2));
   const float y = xadd(xmul(focal, xdiv(v[1], v[2])), (float)(H / 2));
-  // static_cast<int> of a value outside int range is undefined in the reference;
-  // such triangles (never produced by its clip stage) are dropped
-  if (!(fabsf(x) < 8.0e6f) || !(fabsf(y) < 8.0e6f)) return false;
+  // static_cast<int> of a value outside int range (or NaN) is undefined in the reference; such
+  // triangles are dropped.  Everything inside converts and is drawn as the reference draws it:
+  // the far plane's (w1 - w0) divisor (:1615) can put a clipped vertex of finite scene input
+  // tens of millions of pixels off screen (5e7 at W = 32768, tests/test_rast_clip_gpu.py)
+  if (!(fabsf(x) < 2147483648.0f) || !(fabsf(y) < 2147483648.0f)) return false;
   o.x = (int)x;
   o.y = (int)y;
   o.zinv = xdiv(1.0f, v[2]);

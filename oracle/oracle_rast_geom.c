@@ -44,6 +44,31 @@ static void lerp4(const float *a, const float *b, float t, float *o) {
   for (int k = 0; k < 4; ++k) o[k] = a[k] + t * (b[k] - a[k]);
 }
 
+/* Clip census: how often each branch of clip_one was taken since the last reset, so that tests can
+ * check which cases their scenes reach.  Counting only; the arithmetic is untouched.  Layout (the
+ * indices oracle_rast_clip_census copies out):
+ *   CEN_BRANCH + 8 * i + k   plane i = 0..4 for planes 1, 2, 3, 4, 6; k = 0 all in, 1 only v0 in,
+ *                            2 only v1, 3 only v2, 4 v0 and v1, 5 v0 and v2, 6 v1 and v2, 7 all out
+ *   CEN_FAR_REFUSED          far plane, v0 and v2 in but v2.x > 5 / f (:1607): dropped
+ *   CEN_NEAR_KEPT / _DROPPED plane 5 (:1497-1505)
+ *   CEN_NAN                  dropped because a vertex is neither inside nor outside (NaN)
+ *   CEN_ZERO_DEN             intersection parameters whose denominator is exactly 0 (t = +-inf or NaN; odd W or H
+ *                            make one possible on planes 1-4, whose t uses the truncated W / 2, H / 2)
+ *   CEN_ON_LIMIT + p - 1     vertices exactly on plane p's limit (x or y == the bound, z == 0.01,
+ *                            w == 5 / f), each time a triangle meets that plane
+ *   CEN_DESC + n             pre-clip triangles with n descendants in the final list (0..32) */
+enum { CEN_BRANCH = 0, CEN_FAR_REFUSED = 40, CEN_NEAR_KEPT, CEN_NEAR_DROPPED, CEN_NAN, CEN_ZERO_DEN, CEN_ON_LIMIT,
+       CEN_DESC = CEN_ON_LIMIT + 6, CEN_N = CEN_DESC + 33 };
+static long long census[CEN_N];
+
+/* Copies min(cap, CEN_N) counters to out (when not NULL), clears them when reset != 0 and returns
+ * CEN_N. */
+int oracle_rast_clip_census(long long *out, int cap, int reset) {
+  if (out) memcpy(out, census, (size_t)(cap < CEN_N ? cap : CEN_N) * sizeof(long long));
+  if (reset) memset(census, 0, sizeof census);
+  return CEN_N;
+}
+
 typedef struct { int plane, W, H; float focal; } clip_ctx;
 
 static int inside(const clip_ctx *c, const float *v) {
@@ -65,45 +90,71 @@ static int outside(const clip_ctx *c, const float *v) {
   }
 }
 
+/* num / den, counting an exactly zero denominator */
+static float t_div(float num, float den) {
+  census[CEN_ZERO_DEN] += den == 0.0f;
+  return num / den;
+}
+
 /* intersection parameter along a (inside) -> b (outside) */
 static float t_param(const clip_ctx *c, const float *a, const float *b) {
   switch (c->plane) {
     case 1: { float h = (float)(c->W / 2), nh = (float)((-c->W) / 2);   /* :753 */
-      return (a[0] + h * a[3]) / (((nh * b[3] + h * a[3]) - b[0]) + a[0]); }
+      return t_div(a[0] + h * a[3], ((nh * b[3] + h * a[3]) - b[0]) + a[0]); }
     case 2: { float h = (float)(c->W / 2);                               /* :943 */
-      return (a[0] - h * a[3]) / (((h * b[3] - h * a[3]) - b[0]) + a[0]); }
+      return t_div(a[0] - h * a[3], ((h * b[3] - h * a[3]) - b[0]) + a[0]); }
     case 3: { float h = (float)(c->H / 2);                               /* :1136 */
-      return (a[1] - h * a[3]) / (((h * b[3] - h * a[3]) - b[1]) + a[1]); }
+      return t_div(a[1] - h * a[3], ((h * b[3] - h * a[3]) - b[1]) + a[1]); }
     case 4: { float h = (float)(c->H / 2), nh = (float)((-c->H) / 2);   /* :1328 */
-      return (a[1] + h * a[3]) / (((nh * b[3] + h * a[3]) - b[1]) + a[1]); }
+      return t_div(a[1] + h * a[3], ((nh * b[3] + h * a[3]) - b[1]) + a[1]); }
     default: { float wl = 5.0f / c->focal;                               /* :1524 */
-      return (wl - a[3]) / (b[3] - a[3]); }
+      return t_div(wl - a[3], b[3] - a[3]); }
+  }
+}
+
+/* a vertex exactly on the plane's limit */
+static int on_limit(const clip_ctx *c, const float *v) {
+  switch (c->plane) {
+    case 1: return v[0] == (v[3] * (float)(-c->W)) / 2.0f;
+    case 2: return v[0] == (v[3] * (float)(c->W)) / 2.0f;
+    case 3: return v[1] == (v[3] * (float)(c->H)) / 2.0f;
+    case 4: return v[1] == (v[3] * (float)(-c->H)) / 2.0f;
+    case 5: return v[2] == 0.01f;
+    default: return v[3] == 5.0f / c->focal;
   }
 }
 
 /* One triangle through one plane (0, 1 or 2 results appended to out). */
 static int clip_one(const clip_ctx *c, const g_tri *in, g_tri *out) {
+  for (int k = 0; k < 3; ++k) census[CEN_ON_LIMIT + c->plane - 1] += on_limit(c, in->v[k]);
   if (c->plane == 5) {                                                   /* :1497-1505 */
-    if (in->v[0][2] > 0.01f && in->v[1][2] > 0.01f && in->v[2][2] > 0.01f) { out[0] = *in; return 1; }
+    if (in->v[0][2] > 0.01f && in->v[1][2] > 0.01f && in->v[2][2] > 0.01f) {
+      census[CEN_NEAR_KEPT]++; out[0] = *in; return 1;
+    }
+    census[CEN_NEAR_DROPPED]++;
     return 0;
   }
   const int i0 = inside(c, in->v[0]), i1 = inside(c, in->v[1]), i2 = inside(c, in->v[2]);
   const int o0 = outside(c, in->v[0]), o1 = outside(c, in->v[1]), o2 = outside(c, in->v[2]);
+  long long *br = census + CEN_BRANCH + 8 * (c->plane == 6 ? 4 : c->plane - 1);
   g_tri t = *in;
-  if (i0 && i1 && i2) { out[0] = t; return 1; }
+  if (i0 && i1 && i2) { br[0]++; out[0] = t; return 1; }
   if (i0 && o1 && o2) {                                                  /* only v0 in */
+    br[1]++;
     float t01 = t_param(c, t.v[0], t.v[1]), t02 = t_param(c, t.v[0], t.v[2]);
     lerp4(in->v[0], in->v[1], t01, t.v[1]);
     lerp4(in->v[0], in->v[2], t02, t.v[2]);
     out[0] = t; return 1;
   }
   if (o0 && i1 && o2) {                                                  /* only v1 in */
+    br[2]++;
     float t10 = t_param(c, t.v[1], t.v[0]), t12 = t_param(c, t.v[1], t.v[2]);
     lerp4(in->v[1], in->v[0], t10, t.v[0]);
     lerp4(in->v[1], in->v[2], t12, t.v[2]);
     out[0] = t; return 1;
   }
   if (o0 && o1 && i2) {                                                  /* only v2 in */
+    br[3]++;
     float t21 = t_param(c, t.v[2], t.v[1]), t20 = t_param(c, t.v[2], t.v[0]);
     lerp4(in->v[2], in->v[1], t21, t.v[1]);
     lerp4(in->v[2], in->v[0], t20, t.v[0]);
@@ -111,6 +162,7 @@ static int clip_one(const clip_ctx *c, const g_tri *in, g_tri *out) {
   }
   g_tri extra = *in;   /* keeps the parent's normal / colour / texture / index (:838-841) */
   if (i0 && i1 && o2) {                                                  /* v0, v1 in */
+    br[4]++;
     float t12 = t_param(c, in->v[1], in->v[2]), t02 = t_param(c, in->v[0], in->v[2]);
     float np12[4], np02[4];
     lerp4(in->v[1], in->v[2], t12, np12);
@@ -122,6 +174,7 @@ static int clip_one(const clip_ctx *c, const g_tri *in, g_tri *out) {
   /* v0, v2 in: the far plane's version of this test reads v2.x (:1607) */
   int c02 = c->plane == 6 ? (i0 && o1 && in->v[2][0] <= 5.0f / c->focal) : (i0 && o1 && i2);
   if (c02) {
+    br[5]++;
     float t01 = t_param(c, in->v[0], in->v[1]);
     float t21 = c->plane == 6 ? (5.0f / c->focal - in->v[2][3]) / (in->v[1][3] - in->v[0][3])   /* :1615 */
                               : t_param(c, in->v[2], in->v[1]);
@@ -133,6 +186,7 @@ static int clip_one(const clip_ctx *c, const g_tri *in, g_tri *out) {
     out[0] = t; out[1] = extra; return 2;
   }
   if (o0 && i1 && i2) {                                                  /* v1, v2 in */
+    br[6]++;
     float t10 = t_param(c, in->v[1], in->v[0]), t20 = t_param(c, in->v[2], in->v[0]);
     float np10[4], np20[4];
     lerp4(in->v[1], in->v[0], t10, np10);
@@ -141,6 +195,9 @@ static int clip_one(const clip_ctx *c, const g_tri *in, g_tri *out) {
     memcpy(extra.v[0], np10, 16); memcpy(extra.v[1], np20, 16); memcpy(extra.v[2], in->v[2], 16);
     out[0] = t; out[1] = extra; return 2;
   }
+  if (o0 && o1 && o2) br[7]++;
+  else if (i0 && o1 && i2) census[CEN_FAR_REFUSED]++;
+  else census[CEN_NAN]++;
   return 0;   /* NaNs, or the far plane's unmatched combination: dropped */
 }
 
@@ -194,6 +251,7 @@ int oracle_rast_geometry(int W, int H, float focal, const float *cam, const floa
       memcpy(cur, nxt, (size_t)n_nxt * sizeof(g_tri));
       n_cur = n_nxt;
     }
+    census[CEN_DESC + n_cur]++;
     if (n_out + n_cur > out_cap) return -1;
     memcpy(out + n_out, cur, (size_t)n_cur * sizeof(g_tri));
     n_out += n_cur;

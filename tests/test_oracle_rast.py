@@ -94,7 +94,8 @@ def test_geometry_matches_committed_clipped_lists(name):
 
 @pytest.mark.parametrize("seed", range(8))
 def test_geometry_vs_compiled_reference_random_poses(seed):
-    """Cameras inside the room, yaw, moved lights: every clip case gets exercised."""
+    """Cameras inside the room, yaw, moved lights (which clip branches a scene reaches is counted by the oracle's
+    census: tests/test_rast_clip_gpu.py)."""
     if not h.have_ref(h.ref_rast_name(320, 240)):
         pytest.skip("oracle/_ref not built")
     W, H, f = (320, 240, 170.0) if seed % 2 else (64, 48, 36.0)
