@@ -105,6 +105,7 @@ ABI_SYMBOLS = [
     "b200_measure_fp32_peak", "rt_upload_scene", "rt_render_device",
     "render_raytrace_views", "draw_raytrace_views", "rt_render_views_device",
     "rt_closest_hits", "rt_occluded", "rt_closest_hits_device", "rt_occluded_device",
+    "rt_direct_light", "rt_direct_light_device",
     "render_raster_clipped", "render_raster", "render_raster_band", "draw_raster", "raster_read_buffers",
     "raster_read_clipped", "rast_upload_clipped", "rast_render_device", "draw_raster_band",
     "rast_upload_scene", "rast_draw_device", "rast_set_textures",
@@ -130,6 +131,8 @@ def load_library():
         _lib.rt_occluded.argtypes = [vp, vp, i32, vp, i32, vp, vp, i32, vp]
         _lib.rt_closest_hits_device.argtypes = [vp, vp, i32, vp]
         _lib.rt_occluded_device.argtypes = [vp, vp, vp, i32, vp]
+        _lib.rt_direct_light.argtypes = [vp, vp, i32, vp, i32, vp, i32, vp, i32, vp]
+        _lib.rt_direct_light_device.argtypes = [vp, vp, i32, vp, i32, vp]
     return _lib
 
 
@@ -368,6 +371,38 @@ class Renderer:
         """Device pointers (ints): rt_ray and float limits in, one byte per ray out; asynchronous."""
         self._check(self.lib.rt_occluded_device(self.ctx, _ptr(d_rays), _ptr(d_max_distance), int(n_rays),
                                                 _ptr(d_out)), "rt_occluded_device")
+
+    @staticmethod
+    def _hits(hits):
+        """hits: an RT_INTERSECTION array, or the dict of rt_closest_hits."""
+        if isinstance(hits, dict):
+            out = np.zeros(len(hits["distance"]), RT_INTERSECTION)
+            for f in RT_INTERSECTION.names:
+                out[f] = hits[f]
+            return out
+        hits = np.ascontiguousarray(hits)
+        if hits.dtype != RT_INTERSECTION:
+            raise TypeError("hits must be an RT_INTERSECTION array or the dict of rt_closest_hits")
+        return hits
+
+    def rt_direct_light(self, tris, spheres, hits, lights):
+        """DirectLight of every hit for every light (lights as for render_raytrace): (n_hits, n_lights, 3) float32.
+        An entry that names no primitive (a miss record, an index out of range) gives 0."""
+        hits = self._hits(hits)
+        out = np.zeros((len(hits), len(lights), 3), np.float32)
+        la = make_lights(lights)
+        rc = self.lib.rt_direct_light(self.ctx, _ptr(tris), 0 if tris is None else len(tris), _ptr(spheres),
+                                      0 if spheres is None else len(spheres), _ptr(hits), len(hits), la, len(lights),
+                                      _ptr(out))
+        self._check(rc, "rt_direct_light")
+        return out
+
+    def rt_direct_light_device(self, d_hits, n_hits, lights, d_power):
+        """Device pointers (ints): n_hits rt_intersection in, n_hits * n_lights * 3 floats out; the scene of
+        rt_upload_scene; asynchronous."""
+        la = make_lights(lights)
+        self._check(self.lib.rt_direct_light_device(self.ctx, _ptr(d_hits), int(n_hits), la, len(lights),
+                                                    _ptr(d_power)), "rt_direct_light_device")
 
     # ---- RAST ----------------------------------------------------------------
     def render_raster_clipped(self, clipped, cam, light, want=("rgb", "depth", "index")):

@@ -410,17 +410,40 @@ static int check_ray_buffers(b200_ctx *ctx, const void *rays, const float *max_d
   return B200_OK;
 }
 
+static int check_rt_scene(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres) {
+  if (n_tris < 0 || n_spheres < 0 || (n_tris > 0 && !tris) || (n_spheres > 0 && !spheres))
+    return ctx_fail(ctx, B200_EINVAL, "bad scene arguments");
+  return B200_OK;
+}
+
 // (also the multi-GPU context's check, before the rays are shared out)
 int check_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
                const rt_ray *rays, const float *max_distance, int n_rays, const void *out, bool occlusion) {
-  if (n_tris < 0 || n_spheres < 0 || (n_tris > 0 && !tris) || (n_spheres > 0 && !spheres))
-    return ctx_fail(ctx, B200_EINVAL, "bad scene arguments");
+  if (int rc = check_rt_scene(ctx, tris, n_tris, spheres, n_spheres)) return rc;
   return check_ray_buffers(ctx, rays, max_distance, n_rays, out, occlusion);
 }
 
-// One query on device buffers and the uploaded scene: d_hits for closest hits, d_occ (+ d_max) for occlusion.
-static int rt_query_device(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max, int n_rays, rt_intersection *d_hits,
-                           uint8_t *d_occ) {
+static int check_direct_buffers(b200_ctx *ctx, const rt_intersection *hits, int n_hits, const light_t *lights,
+                                int n_lights, const float *power_out) {
+  if (n_hits < 0) return ctx_fail(ctx, B200_EINVAL, "negative hit count");
+  if (n_lights < 0 || n_lights > B200_MAX_LIGHTS || (n_lights > 0 && !lights))
+    return ctx_fail(ctx, B200_EINVAL, "bad lights (at most 8)");
+  if (n_hits > 0 && n_lights > 0 && (!hits || !power_out)) return ctx_fail(ctx, B200_EINVAL, "null hits or output");
+  return B200_OK;
+}
+
+// (also the multi-GPU context's check, before the hits are shared out)
+int check_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                       const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights,
+                       const float *power_out) {
+  if (int rc = check_rt_scene(ctx, tris, n_tris, spheres, n_spheres)) return rc;
+  return check_direct_buffers(ctx, hits, n_hits, lights, n_lights, power_out);
+}
+
+// Enqueues one query on device buffers and the uploaded scene: `launch` enqueues its kernels between the timing
+// events, with the counters zeroed before and read back after.
+template <class Launch>
+static int rt_query_enqueue(b200_ctx *ctx, Launch launch) {
   cudaSetDevice(ctx->device);
   if (ctx->rast_inflight.active) if (int rc = finish_stats(ctx)) return rc;   // the counters are shared
   ctx->stats.kernel_launches = 0;
@@ -428,13 +451,49 @@ static int rt_query_device(b200_ctx *ctx, const rt_ray *d_rays, const float *d_m
   CU_CHECK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
   ctx->tl_n = 0;
   tl_mark(ctx, "query start");
-  if (int rc = rt_launch_rays(ctx, d_rays, d_max, n_rays, d_hits, d_occ)) return rc;
+  if (int rc = launch()) return rc;
   CU_CHECK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+  return enqueue_counter_readback(ctx);
+}
+
+// One query on device buffers and the uploaded scene: d_hits for closest hits, d_occ (+ d_max) for occlusion.
+static int rt_query_device(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max, int n_rays, rt_intersection *d_hits,
+                           uint8_t *d_occ) {
+  if (int rc = rt_query_enqueue(ctx, [&] { return rt_launch_rays(ctx, d_rays, d_max, n_rays, d_hits, d_occ); }))
+    return rc;
   ctx->stats.primary_rays = d_occ ? 0 : (uint64_t)n_rays;
   ctx->stats.shadow_rays = d_occ ? (uint64_t)n_rays : 0;
-  if (int rc = enqueue_counter_readback(ctx)) return rc;
   ctx->pending = 3;
   return B200_OK;
+}
+
+// DirectLight on device buffers and the uploaded scene; the kernels count the shadow rays (pending = 1).
+static int rt_direct_device(b200_ctx *ctx, const rt_intersection *d_hits, int n_hits, const light_t *lights,
+                            int n_lights, float *d_power) {
+  if (int rc = rt_query_enqueue(ctx, [&] { return rt_launch_direct_light(ctx, d_hits, n_hits, lights, n_lights, d_power); }))
+    return rc;
+  ctx->stats.primary_rays = 0;
+  ctx->pending = 1;
+  return B200_OK;
+}
+
+// The host-pointer DirectLight entry: hits to the staging buffer, the query, the powers back.
+static int rt_direct_host(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                          const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights, float *power_out) {
+  if (int rc = check_direct_light(ctx, tris, n_tris, spheres, n_spheres, hits, n_hits, lights, n_lights, power_out))
+    return rc;
+  if (n_hits == 0 || n_lights == 0) return B200_OK;
+  if (int rc = rt_upload_scene(ctx, tris, n_tris, spheres, n_spheres)) return rc;
+  const size_t n = (size_t)n_hits;
+  const size_t off_out = (n * sizeof(rt_intersection) + 255) & ~(size_t)255;
+  const size_t out_bytes = n * (size_t)n_lights * 3 * sizeof(float);
+  if (int rc = ensure(ctx, ctx->rt_query, off_out + out_bytes)) return rc;
+  char *buf = (char *)ctx->rt_query.p;
+  CU_CHECK(ctx, cudaMemcpyAsync(buf, hits, n * sizeof(rt_intersection), cudaMemcpyHostToDevice, ctx->stream));
+  if (int rc = rt_direct_device(ctx, (const rt_intersection *)buf, n_hits, lights, n_lights, (float *)(buf + off_out)))
+    return rc;
+  if (int rc = copy_out(ctx, power_out, buf + off_out, out_bytes)) return rc;
+  return finish_stats(ctx);
 }
 
 // The host-pointer query entries: rays (and limits) to a staging buffer, the query, the results back.
@@ -492,6 +551,23 @@ int rt_occluded_device(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max_d
   if (int rc = check_ray_buffers(ctx, d_rays, d_max_distance, n_rays, d_out, true)) return rc;
   if (n_rays == 0) return B200_OK;
   return rt_query_device(ctx, d_rays, d_max_distance, n_rays, nullptr, d_out);
+}
+
+int rt_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                    const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights, float *power_out) {
+  if (!ctx) return B200_EINVAL;
+  if (ctx->multi)
+    return multi_direct_light(ctx, tris, n_tris, spheres, n_spheres, hits, n_hits, lights, n_lights, power_out);
+  return rt_direct_host(ctx, tris, n_tris, spheres, n_spheres, hits, n_hits, lights, n_lights, power_out);
+}
+
+int rt_direct_light_device(b200_ctx *ctx, const rt_intersection *d_hits, int n_hits, const light_t *lights,
+                           int n_lights, float *d_power) {
+  if (!ctx) return B200_EINVAL;
+  SINGLE_ONLY(ctx);
+  if (int rc = check_direct_buffers(ctx, d_hits, n_hits, lights, n_lights, d_power)) return rc;
+  if (n_hits == 0 || n_lights == 0) return B200_OK;
+  return rt_direct_device(ctx, d_hits, n_hits, lights, n_lights, d_power);
 }
 
 static int rast_frame(b200_ctx *ctx, bool whole_draw, const camera_t *cam, const rast_light_t *light, int row_begin,

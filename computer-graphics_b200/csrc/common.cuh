@@ -22,6 +22,10 @@ __device__ __forceinline__ float xsqrt(float a) { return __fsqrt_rn(a); }
 // same sample, ...) sends the whole warp through __fdiv_rn's slow path (ncu: 13 % of the small-
 // triangle kernel's instructions at 9 of 32 lanes); 0 / den = a exactly, sign included.
 __device__ __forceinline__ float xdiv_pos(float a, float den) { return a == 0.0f ? a : __fdiv_rn(a, den); }
+// On x86 an invalid operation (0 * inf, inf - inf, 0 / 0) yields the indefinite NaN 0xffc00000 and later
+// operations pass it on unchanged; here it yields 0x7fffffff.  Outputs whose every NaN begins as such an operation
+// store it as the reference's bits (the rasteriser's clipped list, DESIGN §4.1; rt_direct_light, §3.4).
+__device__ __forceinline__ float x86_nan(float v) { return v != v ? __int_as_float(0xffc00000) : v; }
 
 // IEEE-exact x / C for the constants the reference divides by (5, 3, 9):
 // q = x*rc; r = fma(-C, q, x); q' = fma(r, rc, q) with rc = RN(1/C) is the
@@ -129,7 +133,7 @@ struct b200_ctx {
   int rt_bounds_on_device = 0;
   DevBuf rt_cells;    // direction grids: per-cell counts, cursors, padded counts, offsets, scan scratch
   DevBuf rt_cell_rec, rt_cell_idx;   // the cells' lists: plane records and triangle indices
-  DevBuf rt_query;   // host-pointer ray queries: rays, limits and results (rt_closest_hits, rt_occluded)
+  DevBuf rt_query;   // host-pointer ray queries: rays or hits, limits and results (rt_closest_hits, rt_occluded, rt_direct_light)
   DevBuf rt_plan;                    // gridded frames: two per-block cost arrays, the block plan, its length (rt_plan_kernel)
   unsigned long long rt_plan_shape = 0;
   int rt_plan_valid = 0, rt_plan_flip = 0;
@@ -145,7 +149,8 @@ struct b200_ctx {
   int rt_n_tris = 0, rt_n_spheres = 0;
   float rt_world_abs = 0.f;   // max |coordinate| over the uploaded scene
   float rt_normal_abs = 1.f;  // max(1, max |normal component|): scales the 1e-5 * normal shadow-ray offset (:394)
-  int pending = 0;            // 1 = RT, 2 = RAST render, 3 = RT ray query whose counters are not read back yet
+  int pending = 0;            // 1 = RT frame or direct-light query, 2 = RAST render, 3 = RT ray query whose counters are
+                              // not read back yet
 
   // RAST scene (device)
   DevBuf rast_src;    // rast_triangle[n] clipped list
@@ -271,6 +276,9 @@ int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int
 // rt_rays.cu: one ray query on the uploaded scene, n > 0 rays; d_hits (closest hits) or d_occ + d_max (occlusion)
 int rt_launch_rays(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max, int n, rt_intersection *d_hits,
                    uint8_t *d_occ);
+// rt_rays.cu: DirectLight for n > 0 hits and 1..8 lights on the uploaded scene, d_power[(i * n_lights + l) * 3 + c]
+int rt_launch_direct_light(b200_ctx *ctx, const rt_intersection *d_hits, int n, const light_t *lights, int n_lights,
+                           float *d_power);
 // whole frames of n_views cameras of one size, frame k of each output at k * W * H (rgb: times 3)
 int rt_launch_views(b200_ctx *ctx, const RtFrame *fs, int n_views, float *d_rgb, float *d_depth, int32_t *d_index,
                     uint32_t *d_argb);
@@ -292,6 +300,11 @@ int multi_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphe
                bool occlusion);
 int check_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
                const rt_ray *rays, const float *max_distance, int n_rays, const void *out, bool occlusion);   // api.cu
+int multi_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                       const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights, float *power_out);
+int check_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                       const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights,
+                       const float *power_out);   // api.cu
 int multi_raster(b200_ctx *ctx, const rast_triangle *room, int n_room, const rast_triangle *boxes, int n_boxes,
                  const camera_t *cam, const rast_light_t *light, int row_begin, int row_end, float *rgb_out,
                  float *depth_out, int32_t *index_out, uint32_t *argb_out);

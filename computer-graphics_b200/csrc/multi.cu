@@ -360,6 +360,27 @@ int multi_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphe
   return B200_OK;
 }
 
+// DirectLight for caller-supplied hits: device i shades the contiguous run [k_i, k_i+1) of the hits, every light.
+int multi_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                       const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights, float *power_out) {
+  b200_multi *mc = ctx->multi;
+  if (int rc = check_direct_light(ctx, tris, n_tris, spheres, n_spheres, hits, n_hits, lights, n_lights, power_out))
+    return rc;
+  if (n_hits == 0 || n_lights == 0) return B200_OK;
+  const int n = mc->n;
+  const int rc = multi_run(ctx, [&](int i) -> int {
+    const int a = (int)((long long)n_hits * i / n), b = (int)((long long)n_hits * (i + 1) / n);
+    b200_ctx *c = mc->child[i];
+    c->stats = b200_stats{};
+    if (b <= a) return B200_OK;
+    return rt_direct_light(c, tris, n_tris, spheres, n_spheres, hits + a, b - a, lights, n_lights,
+                           power_out + (size_t)a * n_lights * 3);
+  });
+  if (rc != B200_OK) return rc;
+  multi_sum_stats(ctx);
+  return B200_OK;
+}
+
 // ---- rasteriser -------------------------------------------------------------------------
 // Every device keeps its own copy of the images (each over its own PCIe link).
 int multi_rast_set_textures(b200_ctx *ctx, const rast_textures_t *tex) {

@@ -188,8 +188,8 @@ __device__ __forceinline__ void geom_preclip(const GeomXform &p, const rast_tria
 // (0 * inf, inf - inf, 0 / 0) yields the indefinite NaN 0xffc00000 and later operations pass it on unchanged; here
 // it yields 0x7fffffff.  With finite scene inputs every NaN the stage computes begins as such an operation (a
 // caller's NaN or inf vertex is dropped by the clip before it can reach the list), so the list writers store every
-// computed NaN -- vertices and shadow-volume normals, not attributes copied from the caller -- as 0xffc00000.
-__device__ __forceinline__ float x86_nan(float v) { return v != v ? __int_as_float(0xffc00000) : v; }
+// computed NaN -- vertices and shadow-volume normals, not attributes copied from the caller -- as 0xffc00000
+// (x86_nan, common.cuh).
 
 // A triangle inside all six planes comes out of the clip unchanged (one descendant).
 __device__ __forceinline__ bool geom_all_in(const GeomXform &p, const GTri &t) {

@@ -57,6 +57,24 @@ __device__ __forceinline__ void rt_surface(const RtKParams &p, int idx, float px
   }
 }
 
+// Colour and shading normal of a hit (skeleton.cpp:148-149, 377-387;
+// Sphere::getNormal TestModelH.h:68-75).
+__device__ __forceinline__ void rt_surface2(const rt_triangle *__restrict__ src, const rt_sphere *__restrict__ sph,
+                                            int idx, float px, float py, float pz, float *col, float &nx,
+                                            float &ny, float &nz) {
+  if (idx >= 0) {
+    const rt_triangle *t = src + idx;
+    col[0] = __ldg(&t->color[0]); col[1] = __ldg(&t->color[1]); col[2] = __ldg(&t->color[2]);
+    nx = __ldg(&t->normal[0]); ny = __ldg(&t->normal[1]); nz = __ldg(&t->normal[2]);
+  } else {
+    const rt_sphere *s = sph + (-1 - idx);
+    col[0] = s->color[0]; col[1] = s->color[1]; col[2] = s->color[2];
+    const float ax = xsub(px, s->centre[0]), ay = xsub(py, s->centre[1]), az = xsub(pz, s->centre[2]);
+    const float inv = xdiv(1.0f, xsqrt(xdot3(ax, ay, az, ax, ay, az)));
+    nx = xmul(ax, inv); ny = xmul(ay, inv); nz = xmul(az, inv);
+  }
+}
+
 // averageLight = pixelColour / 9 or black (skeleton.cpp:160-166), then the
 // optional PutPixelSDL quantisation.
 __device__ __forceinline__ void rt_store_pixel(const RtKParams &p, size_t pid, bool valid, const float *pix) {

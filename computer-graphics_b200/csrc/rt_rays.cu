@@ -1,5 +1,6 @@
 // Raytracer ray queries on sm_100a: ClosestIntersection (raytracer/Source/skeleton.cpp:263-363) for rays the
-// caller supplies, and the shadow test of DirectLight, `ClosestIntersection(...) && distance < r_mag` (:394-397).
+// caller supplies, the shadow test of DirectLight, `ClosestIntersection(...) && distance < r_mag` (:394-397), and
+// DirectLight itself for hits the caller supplies.
 //
 //   rt_rays_kernel<ANY>        one thread per ray, rays in the caller's order.  Every warp streams the scene's
 //                              48-byte RtGeom records through its own double-buffered shared-memory ring (1-D TMA
@@ -9,6 +10,9 @@
 //                              reference accepts below its limit, a warp leaves when its 32 rays are decided.
 //   rt_rays_bruteforce_kernel  B200_OPT_RT_BRUTEFORCE = 1: the per-ray exact loop over every pair
 //                              (rt_closest_bruteforce), no cull and no early exit (the on-device cross-check).
+//   rt_direct_light_kernel     DirectLight (:366-415) for caller-supplied hits, one thread per (hit, light) pair: the
+//                              shadow ray walks the scene like rt_rays_kernel<true> (rt_rays_walk), then the Lambert
+//                              term.  rt_direct_light_bruteforce_kernel is its B200_OPT_RT_BRUTEFORCE = 1 twin.
 //
 // There is no spatial index: a call costs rays x triangles, minus what the cull removes.  Large scenes stream every
 // record like small ones.  DESIGN.md section 3.4 has the exactness argument of the early exit and the soundness
@@ -140,30 +144,33 @@ __device__ __forceinline__ bool rt_rays_cull(const RtBundle &B, float4 g0, float
   return false;
 }
 
-template <bool ANY>
-__global__ void __launch_bounds__(RT_RAYS_THREADS) rt_rays_kernel(const __grid_constant__ RtRaysParams p) {
-  __shared__ __align__(128) float4 s_tiles[RT_RAYS_WARPS][2][RT_RAYS_TILE * 3];
-  __shared__ __align__(8) uint64_t s_bars[RT_RAYS_WARPS][2];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+// Each warp's double-buffered ring of triangle records.  Set up once per block by rt_rays_ring_init, whose barrier is
+// the only block barrier of the kernels that walk the scene: from there on every warp runs on its own.
+struct RtRing {
+  float4 tiles[RT_RAYS_WARPS][2][RT_RAYS_TILE * 3];
+  uint64_t bars[RT_RAYS_WARPS][2];
+};
+
+__device__ __forceinline__ void rt_rays_ring_init(RtRing &s) {
   if (threadIdx.x == 0) {
-    for (int w = 0; w < RT_RAYS_WARPS; ++w) { mbar_init(&s_bars[w][0], 1); mbar_init(&s_bars[w][1], 1); }
+    for (int w = 0; w < RT_RAYS_WARPS; ++w) { mbar_init(&s.bars[w][0], 1); mbar_init(&s.bars[w][1], 1); }
     mbar_fence_init();
   }
-  __syncthreads();   // the only block barrier: from here on every warp runs on its own
+  __syncthreads();
+}
 
-  const int i = blockIdx.x * RT_RAYS_THREADS + threadIdx.x;
-  const bool live = i < p.n;
-  float sx = 0.f, sy = 0.f, sz = 0.f, sw = 0.f, dx = 0.f, dy = 0.f, dz = 0.f, maxd = 0.f;
-  if (live) {
-    const rt_ray *r = p.rays + i;   // (4-byte alignment is all a caller's device pointer promises)
-    sx = __ldg(&r->start[0]); sy = __ldg(&r->start[1]); sz = __ldg(&r->start[2]); sw = __ldg(&r->start[3]);
-    dx = __ldg(&r->dir[0]); dy = __ldg(&r->dir[1]); dz = __ldg(&r->dir[2]);
-    if (ANY) maxd = p.max_distance[i];
-  }
-  RtHit best;
+// ClosestIntersection(start s, dir d) for one ray per thread, every thread of the block taking part, over the scene
+// of p (the kernel parameters' geom, n_tris, sph, n_sph and counters): the triangle records streamed through the
+// warp's ring, culled against the box of the warp's active rays, the survivors run in ascending index order, then the
+// spheres.  `active` = false: the thread traces nothing.  ANY: returns DirectLight's shadow test
+// `ClosestIntersection(...) && distance < maxd`, and stops at the first pair accepted below maxd when the ray and the
+// scene are tame (counters[2] == 0, rt_rays_scene_kernel).  Otherwise fills `best` and returns false.  Adds the exact
+// evaluations to counters[1].
+template <bool ANY, class Params>
+__device__ __forceinline__ bool rt_rays_walk(RtRing &S, const Params &p, float sx, float sy, float sz, float dx, float dy,
+                                             float dz, float maxd, bool active, RtHit &best) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   best.t = 0.f; best.dist = FLT_MAX; best.idx = 0;
-  // ANY: a NaN or non-positive limit answers 0 without a test
-  bool active = live && (!ANY || maxd > 0.0f);
   bool occ = false;
   const float len = xsqrt(xdot3(dx, dy, dz, dx, dy, dz));   // glm::length(dir3), :307
   const float dinf = fmaxf(fabsf(dx), fmaxf(fabsf(dy), fabsf(dz)));
@@ -189,8 +196,8 @@ __global__ void __launch_bounds__(RT_RAYS_THREADS) rt_rays_kernel(const __grid_c
 
   bool warp_busy = __any_sync(0xffffffffu, active);
   const int n_tiles = (p.n_tris + RT_RAYS_TILE - 1) / RT_RAYS_TILE;
-  float4 *ring = &s_tiles[warp][0][0];
-  uint64_t *bars = s_bars[warp];
+  float4 *ring = &S.tiles[warp][0][0];
+  uint64_t *bars = S.bars[warp];
   auto issue = [&](int k) {   // lane 0: tile k into buffer k & 1
     const int cnt = min(RT_RAYS_TILE, p.n_tris - k * RT_RAYS_TILE);
     uint64_t *bar = &bars[k & 1];
@@ -238,14 +245,32 @@ __global__ void __launch_bounds__(RT_RAYS_THREADS) rt_rays_kernel(const __grid_c
   }
   if (active) rt_exact_spheres(p.sph, p.n_sph, sx, sy, sz, dx, dy, dz, best);   // :341-355
   rt_count(p.counters + 1, n_exact);
+  return ANY && (occ || (active && best.dist < FLT_MAX && best.dist < maxd));   // :395-397
+}
+
+template <bool ANY>
+__global__ void __launch_bounds__(RT_RAYS_THREADS) rt_rays_kernel(const __grid_constant__ RtRaysParams p) {
+  __shared__ __align__(128) RtRing S;
+  rt_rays_ring_init(S);
+  const int i = blockIdx.x * RT_RAYS_THREADS + threadIdx.x;
+  const bool live = i < p.n;
+  float sx = 0.f, sy = 0.f, sz = 0.f, sw = 0.f, dx = 0.f, dy = 0.f, dz = 0.f, maxd = 0.f;
+  if (live) {
+    const rt_ray *r = p.rays + i;   // (4-byte alignment is all a caller's device pointer promises)
+    sx = __ldg(&r->start[0]); sy = __ldg(&r->start[1]); sz = __ldg(&r->start[2]); sw = __ldg(&r->start[3]);
+    dx = __ldg(&r->dir[0]); dy = __ldg(&r->dir[1]); dz = __ldg(&r->dir[2]);
+    if (ANY) maxd = p.max_distance[i];
+  }
+  RtHit best;
+  // ANY: a NaN or non-positive limit answers 0 without a test
+  const bool occ = rt_rays_walk<ANY>(S, p, sx, sy, sz, dx, dy, dz, maxd, live && (!ANY || maxd > 0.0f), best);
   if (!live) return;
-  const bool hit = best.dist < FLT_MAX;
   if (ANY) {
-    p.occluded[i] = (occ || (active && hit && best.dist < maxd)) ? 1 : 0;   // :395-397
+    p.occluded[i] = occ ? 1 : 0;
   } else {
     rt_intersection o;
     o.distance = best.dist;
-    if (hit) {
+    if (best.dist < FLT_MAX) {
       // position = start + vec4(t * dir3, 0)   (:326 / :345)
       o.position[0] = xadd(sx, xmul(best.t, dx)); o.position[1] = xadd(sy, xmul(best.t, dy));
       o.position[2] = xadd(sz, xmul(best.t, dz)); o.position[3] = rt_pos_w(sw);
@@ -287,6 +312,104 @@ __global__ void __launch_bounds__(128) rt_rays_bruteforce_kernel(const __grid_co
   rt_count(p.counters + 1, i < p.n ? (unsigned long long)p.n_tris : 0ull);
 }
 
+// ---- DirectLight (skeleton.cpp:366-415) for caller-supplied hits: one thread per (hit, light) pair ---------------
+struct RtDirectParams {
+  const float4 *geom;            // ctx->rt_geom: v0, e1, e2 per triangle
+  const rt_triangle *src;        // colour and normal
+  const rt_sphere *sph;
+  int n_tris, n_sph;
+  const rt_intersection *hits;
+  int n, n_lights;
+  float lights[B200_MAX_LIGHTS][7];   // pos[4], colour[3]
+  float *power;                  // [(i * n_lights + l) * 3 + c]
+  unsigned long long *counters;  // [0] shadow rays, [1] exact evaluations, [2] nonzero: some record is not tame
+};
+
+// What DirectLight forms before its shadow test (:370-394) for entry i and light L.  `named` = false: the entry
+// names no primitive (a miss record, an index out of range) and the pair is not traced.
+struct RtShadowRay {
+  bool named;
+  float cr, cg, cb, nx, ny, nz;   // colour and normal (rt_surface2)
+  float rx, ry, rz, r_mag;    // r = light - p (:370), r_mag (:371)
+  float ox, oy, oz;           // the start p + 1e-5 n (:394)
+};
+
+__device__ __forceinline__ RtShadowRay rt_shadow_ray(const RtDirectParams &p, int i, const float *L) {
+  RtShadowRay s;
+  s.named = false;
+  float col[3] = {0.f, 0.f, 0.f};
+  s.nx = s.ny = s.nz = 0.f;
+  float px = 0.f, py = 0.f, pz = 0.f;
+  int idx = 0;
+  if (i < p.n) {
+    const rt_intersection *h = p.hits + i;   // (4-byte alignment is all a caller's device pointer promises)
+    const int ti = __ldg(&h->triangle_index), si = __ldg(&h->sphere_index);
+    // `if (triangleIndex != -1)` (:377): that triangle, otherwise that sphere
+    s.named = ti != -1 ? (ti >= 0 && ti < p.n_tris) : (si >= 0 && si < p.n_sph);
+    idx = ti != -1 ? ti : -1 - si;
+    px = __ldg(&h->position[0]); py = __ldg(&h->position[1]); pz = __ldg(&h->position[2]);
+  }
+  if (s.named) rt_surface2(p.src, p.sph, idx, px, py, pz, col, s.nx, s.ny, s.nz);
+  s.cr = col[0]; s.cg = col[1]; s.cb = col[2];
+  s.rx = xsub(L[0], px); s.ry = xsub(L[1], py); s.rz = xsub(L[2], pz);
+  s.r_mag = rt_exact_rmag(s.rx, s.ry, s.rz);
+  s.ox = xadd(px, xmul(s.nx, 0.00001f)); s.oy = xadd(py, xmul(s.ny, 0.00001f)); s.oz = xadd(pz, xmul(s.nz, 0.00001f));
+  return s;
+}
+
+// The Lambert term of a clear shadow ray (:400-412), 0 for an occluded or unnamed pair.  Every NaN is stored as the
+// x86 indefinite NaN (x86_nan): from NaN-free inputs each one begins as an invalid operation (DESIGN.md 3.4).  Not
+// inlined, and it forms the pair's inputs again: nothing of them stays live through the walk.
+__device__ __noinline__ void rt_store_power(const RtDirectParams &p, int i, int l, bool occ) {
+  const float *L = p.lights[l];
+  const RtShadowRay s = rt_shadow_ray(p, i, L);
+  float pw[3] = {0.f, 0.f, 0.f};
+  const float col[3] = {s.cr, s.cg, s.cb};
+  if (s.named && !occ) rt_exact_lambert(s.rx, s.ry, s.rz, s.r_mag, s.nx, s.ny, s.nz, col, L + 4, pw);
+  float *o = p.power + ((size_t)i * p.n_lights + l) * 3;
+  o[0] = x86_nan(pw[0]); o[1] = x86_nan(pw[1]); o[2] = x86_nan(pw[2]);
+}
+
+// blockIdx.y = the light: the 32 shadow rays of a warp share their end point and start on neighbouring hits, which
+// is what the cull of rt_rays_walk needs.
+__global__ void __launch_bounds__(RT_RAYS_THREADS) rt_direct_light_kernel(const __grid_constant__ RtDirectParams p) {
+  __shared__ __align__(128) RtRing S;
+  rt_rays_ring_init(S);
+  const int i = blockIdx.x * RT_RAYS_THREADS + threadIdx.x, l = blockIdx.y;
+  const float *L = p.lights[l];
+  const RtShadowRay s = rt_shadow_ray(p, i, L);
+  RtHit best;
+  // a NaN or zero r_mag: no distance lies below it (:395), nothing to test
+  const bool occ = rt_rays_walk<true>(S, p, s.ox, s.oy, s.oz, s.rx, s.ry, s.rz, s.r_mag, s.named && s.r_mag > 0.0f, best);
+  rt_count(p.counters + 0, s.named ? 1ull : 0ull);
+  if (i < p.n) rt_store_power(p, i, l, occ);
+}
+
+__global__ void __launch_bounds__(128) rt_direct_light_bruteforce_kernel(const __grid_constant__ RtDirectParams p,
+                                                                         const __grid_constant__ RtKParams k) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x, l = blockIdx.y;
+  const float *L = p.lights[l];
+  const RtShadowRay s = rt_shadow_ray(p, i, L);
+  bool occ = false;
+  if (s.named) {
+    const RtHit best = rt_closest_bruteforce(k, s.ox, s.oy, s.oz, s.rx, s.ry, s.rz);
+    occ = best.dist < FLT_MAX && best.dist < s.r_mag;   // :394-397
+  }
+  rt_count(p.counters + 0, s.named ? 1ull : 0ull);
+  rt_count(p.counters + 1, s.named ? (unsigned long long)p.n_tris : 0ull);
+  if (i < p.n) rt_store_power(p, i, l, occ);
+}
+
+// The scene flag the occlusion walk's early exit reads (counters[2]).
+static int rt_launch_scene_flag(b200_ctx *ctx, const float4 *geom, int n_tris, unsigned long long *counters) {
+  if (n_tris == 0) return B200_OK;
+  rt_rays_scene_kernel<<<(n_tris + 255) / 256, 256, 0, ctx->stream>>>(geom, n_tris, counters);
+  tl_mark(ctx, "rt_rays_scene_kernel");
+  ctx->stats.kernel_launches++;
+  CU_CHECK(ctx, cudaGetLastError());
+  return B200_OK;
+}
+
 // Enqueues one query on ctx->stream: d_hits (closest) or d_occ with d_max (occlusion); n > 0.
 int rt_launch_rays(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max, int n, rt_intersection *d_hits, uint8_t *d_occ) {
   RtRaysParams p;
@@ -310,16 +433,45 @@ int rt_launch_rays(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max, int 
     CU_CHECK(ctx, cudaGetLastError());
     return B200_OK;
   }
-  if (any && p.n_tris > 0) {
-    rt_rays_scene_kernel<<<(p.n_tris + 255) / 256, 256, 0, ctx->stream>>>(p.geom, p.n_tris, p.counters);
-    tl_mark(ctx, "rt_rays_scene_kernel");
-    ctx->stats.kernel_launches++;
-    CU_CHECK(ctx, cudaGetLastError());
-  }
+  if (any) if (int rc = rt_launch_scene_flag(ctx, p.geom, p.n_tris, p.counters)) return rc;
   const unsigned blocks = (unsigned)((n + RT_RAYS_THREADS - 1) / RT_RAYS_THREADS);
   if (any) rt_rays_kernel<true><<<blocks, RT_RAYS_THREADS, 0, ctx->stream>>>(p);
   else rt_rays_kernel<false><<<blocks, RT_RAYS_THREADS, 0, ctx->stream>>>(p);
   tl_mark(ctx, "rt_rays_kernel");
+  ctx->stats.kernel_launches++;
+  CU_CHECK(ctx, cudaGetLastError());
+  return B200_OK;
+}
+
+int rt_launch_direct_light(b200_ctx *ctx, const rt_intersection *d_hits, int n, const light_t *lights, int n_lights,
+                           float *d_power) {
+  RtDirectParams p;
+  memset(&p, 0, sizeof p);
+  p.geom = (const float4 *)ctx->rt_geom.p;
+  p.src = (const rt_triangle *)ctx->rt_src.p;
+  p.sph = (const rt_sphere *)ctx->rt_spheres.p;
+  p.n_tris = ctx->rt_n_tris; p.n_sph = ctx->rt_n_spheres;
+  p.hits = d_hits; p.n = n; p.n_lights = n_lights;
+  for (int l = 0; l < n_lights; ++l) {
+    memcpy(&p.lights[l][0], lights[l].pos, 4 * sizeof(float));
+    memcpy(&p.lights[l][4], lights[l].colour, 3 * sizeof(float));
+  }
+  p.power = d_power;
+  p.counters = (unsigned long long *)ctx->counters.p;
+  const dim3 grid((unsigned)((n + RT_RAYS_THREADS - 1) / RT_RAYS_THREADS), (unsigned)n_lights);
+  if (ctx->opt_rt_bruteforce) {
+    RtKParams k;   // the scene fields rt_closest_bruteforce reads
+    memset(&k, 0, sizeof k);
+    k.geom = p.geom; k.sph = p.sph; k.n_tris = p.n_tris; k.n_sph = p.n_sph;
+    rt_direct_light_bruteforce_kernel<<<grid, RT_RAYS_THREADS, 0, ctx->stream>>>(p, k);
+    tl_mark(ctx, "rt_direct_light_bruteforce_kernel");
+    ctx->stats.kernel_launches++;
+    CU_CHECK(ctx, cudaGetLastError());
+    return B200_OK;
+  }
+  if (int rc = rt_launch_scene_flag(ctx, p.geom, p.n_tris, p.counters)) return rc;
+  rt_direct_light_kernel<<<grid, RT_RAYS_THREADS, 0, ctx->stream>>>(p);
+  tl_mark(ctx, "rt_direct_light_kernel");
   ctx->stats.kernel_launches++;
   CU_CHECK(ctx, cudaGetLastError());
   return B200_OK;

@@ -329,6 +329,39 @@ int rt_closest_hits_device(b200_ctx *ctx, const rt_ray *d_rays, int n_rays, rt_i
 int rt_occluded_device(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max_distance, int n_rays,
                        uint8_t *d_out);
 
+/* ---- RT, DirectLight for hits the caller supplies --------------------------------
+ * skeleton.cpp:366-415 for every (hit, light) pair, bit for bit, so that Draw composes from library calls for any
+ * set of sample rays: rt_closest_hits -> rt_direct_light -> the caller's own accumulation.
+ *   - Per light, not summed: Draw adds each light's DirectLight into its running pixel sum one at a time
+ *     (:151-153), and a sum over the lights would round differently.
+ *   - The entry rule of the reference's `if (triangleIndex != -1)`: triangle_index != -1 names that triangle,
+ *     which must lie in [0, n_tris); otherwise sphere_index names a sphere in [0, n_spheres).  Any other entry
+ *     (the miss records of rt_closest_hits, indices out of range) gives 0 and traces nothing.
+ *   - position is read; position.w reaches only the shadow ray's start.w, so no output.  distance is not read.
+ *   - A NaN output component that the arithmetic creates from NaN-free inputs (a light exactly at the hit point, a
+ *     hit at a sphere's centre, inf - inf) is stored as 0xffc00000, the NaN the reference makes on x86.  Where an
+ *     input carries a NaN the NaN's payload is not specified.
+ *   - n_hits < 0, n_lights < 0 or > B200_MAX_LIGHTS (8), a null hits / power_out when n_hits > 0 and n_lights > 0,
+ *     a null lights when n_lights > 0, or bad scene arguments: B200_EINVAL.  n_hits == 0 or n_lights == 0:
+ *     B200_OK, nothing written.
+ *   - One thread per (hit, light) pair; the shadow ray walks the scene like rt_occluded (per-warp cull, exact early
+ *     exit).  B200_OPT_RT_BRUTEFORCE = 1: the per-ray exact loop over every pair, without cull or early exit.
+ *   - b200_get_stats afterwards: primary_rays = 0, shadow_rays = pairs that traced a shadow ray (entries naming a
+ *     primitive x n_lights, counted on the device), prim_tests = shadow_rays * (n_tris + n_spheres), exact_evals,
+ *     kernel_launches and gpu_ms as for the ray queries.
+ *   - The context is left as the ray queries leave it; a pipelined raster frame in flight is finished first.
+ *   - On a b200_init_multi context rt_direct_light gives each device a contiguous run of the hits;
+ *     rt_direct_light_device returns B200_EINVAL there. */
+
+/* power_out[(i * n_lights + l) * 3 + c] = DirectLight(hits[i]) for lights[l] (skeleton.cpp:366-415), bit for bit.
+ * Host pointers; uploads the scene like render_raytrace. */
+int rt_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                    const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights, float *power_out);
+/* Device-resident: the scene of rt_upload_scene, DEVICE hits / power, HOST lights (as rt_render_device),
+ * asynchronous on b200_stream(ctx). */
+int rt_direct_light_device(b200_ctx *ctx, const rt_intersection *d_hits, int n_hits, const light_t *lights,
+                           int n_lights, float *d_power);
+
 /* ---- RAST: replaces rasteriser Draw(screen*) (skeleton.cpp:203-308) --------*/
 
 /* Tier 1: the triangle loop + post pass (skeleton.cpp:243-307) on an
