@@ -270,7 +270,9 @@ static int rt_set_smem_limits(b200_ctx *ctx) {
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_views_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_views_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
-  CU_CHECK(ctx, cudaFuncSetAttribute(rt_lattice_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_LAT_SMEM));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_lattice_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_LAT_LAUNCH_SMEM));
+  // four blocks per SM need 220 KB of it: all that the SM can give to shared memory
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_lattice_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
   ctx->rt_grid_smem_set = 1;
   return B200_OK;
 }
@@ -411,7 +413,7 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
       rt_filtered_kernel<false, true><<<lgrid, RT_THREADS, gsmem, ctx->stream>>>(p);
     tl_mark(ctx, "rt_filtered_kernel<grid>");
   } else if (f.n_lights <= 1 && rt_lattice_exact(f)) {
-    rt_lattice_kernel<<<grid, RT_THREADS, RT_LAT_SMEM, ctx->stream>>>(p);
+    rt_lattice_kernel<<<grid, RT_THREADS, RT_LAT_LAUNCH_SMEM, ctx->stream>>>(p);
     tl_mark(ctx, "rt_lattice_kernel");
   } else {
     if (f.n_lights > 1)
@@ -506,6 +508,14 @@ int rt_launch_views(b200_ctx *ctx, const RtFrame *fs, int n_views, float *d_rgb,
     ctx->stats.kernel_launches++;
     CU_CHECK(ctx, cudaGetLastError());
   }
+  return B200_OK;
+}
+
+// Profiling: resident blocks per SM of rt_lattice_kernel at the shared memory and attributes of its launches.
+extern "C" int b200_debug_rt_lattice_blocks_per_sm(b200_ctx *ctx, int *blocks) {
+  if (!ctx || ctx->multi || !blocks) return B200_EINVAL;
+  if (int rc = rt_set_smem_limits(ctx)) return rc;
+  CU_CHECK(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, rt_lattice_kernel, RT_THREADS, RT_LAT_LAUNCH_SMEM));
   return B200_OK;
 }
 

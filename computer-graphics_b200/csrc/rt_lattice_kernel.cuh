@@ -19,10 +19,22 @@
 constexpr int RT_LAT_N = 33;                        // lattice points per block edge
 constexpr int RT_LAT_PTS = RT_LAT_N * RT_LAT_N;
 constexpr int RT_LAT_SLOTS = 5;
-// ring, then t / distance / index / ray length per (slot, thread), then pw[3] / col[3] per lattice point, then hit flags
-constexpr size_t RT_LAT_SMEM = 2 * (size_t)RT_TILE * RT_REC_F4 * sizeof(float4) +
+// Records per tile of the ring.  Smaller than RT_TILE so that four blocks fit on an SM (4 x (53 852 B + 1 KB the
+// system keeps per block) of 228 KB); the plane records keep their layout, origins RT_TILE-record units apart.
+constexpr int RT_LAT_TILE = 64;
+// ring, then t / distance / index / ray length per (slot, thread) (after the primary phase: hit point x / y / index / z),
+// then pw[3] / col[3] per lattice point, then hit flags
+constexpr size_t RT_LAT_SMEM = 2 * (size_t)RT_LAT_TILE * RT_REC_F4 * sizeof(float4) +
                                4 * (size_t)RT_LAT_SLOTS * RT_THREADS * sizeof(float) +
                                6 * (size_t)RT_LAT_PTS * sizeof(float) + ((RT_LAT_PTS + 3) & ~3);
+static_assert(RT_LAT_SMEM == 53852, "four blocks per SM");
+// Dynamic shared memory of a launch.  RT_LAT_FORCE_BLOCKS (profiling only): padded so that no more than that many
+// blocks fit on an SM (228 KB), to tell what the fourth block gives from what the code gives.
+#ifdef RT_LAT_FORCE_BLOCKS
+constexpr size_t RT_LAT_LAUNCH_SMEM = 228 * 1024 / (RT_LAT_FORCE_BLOCKS + 1) > RT_LAT_SMEM ? 228 * 1024 / (RT_LAT_FORCE_BLOCKS + 1) : RT_LAT_SMEM;
+#else
+constexpr size_t RT_LAT_LAUNCH_SMEM = RT_LAT_SMEM;
+#endif
 
 // The point of column 32 or row 32 that (warp, lane) traces in slot 4: i | j << 8, or -1.  Row 32 goes to the two
 // bottom pixel rows of the bottom warps, column 32 to the two right pixel columns of the right warps; the five
@@ -47,7 +59,7 @@ __device__ __forceinline__ float rt_lat_off(int i) {
   return xmul(0.5f, (float)(kx - 1));
 }
 
-__global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(const __grid_constant__ RtKParams p) {
+__global__ void __launch_bounds__(RT_THREADS, 4) rt_lattice_kernel(const __grid_constant__ RtKParams p) {
   extern __shared__ __align__(128) float4 tile_smem[];
   __shared__ __align__(8) uint64_t bars[2];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -60,6 +72,13 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
   const float *R = p.R;
   const float focal = p.focal, dz = focal;
   const float cx = p.cam[0], cy = p.cam[1], cz = p.cam[2];
+#ifdef RT_PROFILE_PHASES   // diagnostic build: clock64 of every warp at the phase boundaries (profiles/rt_lattice_phases.py)
+  __shared__ long long s_phase[RT_THREADS / 32][8];
+#define RT_PHASE(k) do { __syncwarp(); if (lane == 0) s_phase[warp][k] = clock64(); } while (0)
+#else
+#define RT_PHASE(k) do { } while (0)
+#endif
+  RT_PHASE(0);
 
   if (threadIdx.x == 0) {
     mbar_init(&bars[0], 1); mbar_init(&bars[1], 1);
@@ -68,7 +87,7 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
   __syncthreads();
   RtRing ring;
   ring.smem = tile_smem; ring.bars = bars; ring.phase_bits = 0; ring.issued = 0; ring.smem_idx = nullptr;
-  float *s_ht = reinterpret_cast<float *>(tile_smem + 2 * RT_TILE * RT_REC_F4);
+  float *s_ht = reinterpret_cast<float *>(tile_smem + 2 * RT_LAT_TILE * RT_REC_F4);
   float *s_hd = s_ht + RT_LAT_SLOTS * RT_THREADS;
   int *s_hi = reinterpret_cast<int *>(s_hd + RT_LAT_SLOTS * RT_THREADS);
   float *s_len = s_hd + 2 * RT_LAT_SLOTS * RT_THREADS;
@@ -114,7 +133,7 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
     }
   }
   unsigned n_exact = 0;
-  const float4 *T0 = ring.smem, *T1 = ring.smem + RT_TILE * RT_REC_F4;
+  const float4 *T0 = ring.smem, *T1 = ring.smem + RT_LAT_TILE * RT_REC_F4;
 
   // ============================ primary rays ============================
   {
@@ -127,15 +146,15 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
 
     RtCursor cursor = rt_cursor_scene(p.planes, p.n_tris);
     RtItem item;
-    bool have = rt_cursor_next<false, RT_TILE>(p, cursor, item);
-    if (threadIdx.x == 0 && have) rt_ring_issue<RT_TILE>(ring, item);
+    bool have = rt_cursor_next<false, RT_LAT_TILE>(p, cursor, item);
+    if (threadIdx.x == 0 && have) rt_ring_issue<RT_LAT_TILE>(ring, item);
     while (have) {
       const int buf = ring.issued & 1;
       ++ring.issued;
       __syncthreads();   // everyone is done with the other buffer: refill it
       RtItem next_item;
-      const bool have_next = rt_cursor_next<false, RT_TILE>(p, cursor, next_item);
-      if (threadIdx.x == 0 && have_next) rt_ring_issue<RT_TILE>(ring, next_item);
+      const bool have_next = rt_cursor_next<false, RT_LAT_TILE>(p, cursor, next_item);
+      if (threadIdx.x == 0 && have_next) rt_ring_issue<RT_LAT_TILE>(ring, next_item);
       mbar_wait(&bars[buf], (ring.phase_bits >> buf) & 1u);
       ring.phase_bits ^= 1u << buf;
       const float4 *T = buf ? T1 : T0;
@@ -162,13 +181,16 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
           const float4 q0 = T[(r0 + j) * 3], q1 = T[(r0 + j) * 3 + 1], q2 = T[(r0 + j) * 3 + 2];
           if (valid && rt_box_may_hit_cam<false>(q0, q1, q2, lc0, lc1, lh0, lh1)) mine |= 1u << j;
         }
-        // ---- L2 / EX: each lane walks its own candidates, per lattice point ----
+        // ---- L2 / EX: each lane walks its own candidates, per lattice point.  The filter marks the points the
+        //      reference arithmetic must decide (and those inside all three edges), then one call site serves them:
+        //      each point's state is its own, so the order of the calls does not matter ----
         while (mine) {
           const int j = __ffs(mine) - 1;
           mine &= mine - 1;
           const int tri = base + r0 + j;
           const float4 q0 = T[(r0 + j) * 3], q1 = T[(r0 + j) * 3 + 1], q2 = T[(r0 + j) * 3 + 2];
           const float E = q2.y, dt_lo = q2.z;
+          unsigned ex = 0, inside = 0;
 #pragma unroll
           for (int s = 0; s < RT_LAT_SLOTS; ++s) {
             if (!((valid >> s) & 1u)) continue;
@@ -179,21 +201,25 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
             const float m3 = fminf(fminf(mU, mV), mW);
             if (m3 >= -E) {
               const float mN = mU + mV + mW;
-              RtHit hb;
-              hb.dist = LD(s);
-              const bool farther = (mN > E) && (dt_lo * LLEN(s) > hb.dist * (mN + E));
-              if (!farther) {
-                ++n_exact;
-                hb.t = LT(s); hb.idx = LI(s);
-                const RtHit nb = rt_ex_primary(p.geom, p.dt_cam, cx, cy, cz, tri, m3 >= E ? 1 : 0, dx, dy, dz, LLEN(s), hb);
-                if (nb.idx != hb.idx || nb.dist != hb.dist) { LT(s) = nb.t; LD(s) = nb.dist; LI(s) = nb.idx; }
-              }
+              const bool farther = (mN > E) && (dt_lo * LLEN(s) > LD(s) * (mN + E));
+              if (!farther) ex |= 1u << s;
+              if (m3 >= E) inside |= 1u << s;
             }
+          }
+          while (ex) {
+            const int s = __ffs(ex) - 1;
+            ex &= ex - 1;
+            ++n_exact;
+            RtHit hb;
+            hb.t = LT(s); hb.dist = LD(s); hb.idx = LI(s);
+            const RtHit nb = rt_ex_primary(p.geom, p.dt_cam, cx, cy, cz, tri, (inside >> s) & 1u, SDX(s), SDY(s), dz, LLEN(s), hb);
+            if (nb.idx != hb.idx || nb.dist != hb.dist) { LT(s) = nb.t; LD(s) = nb.dist; LI(s) = nb.idx; }
           }
         }
       }
     }
   }
+  RT_PHASE(1);
 
   // spheres (skeleton.cpp:341-355), per lattice point in ascending sphere order
   for (int sp = 0; sp < p.n_sph && valid; ++sp) {
@@ -226,6 +252,7 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
       if (h.hit && h.t < LD(s)) { LT(s) = h.t; LD(s) = h.t; LI(s) = -1 - sp; }
     }
   }
+  RT_PHASE(2);
   unsigned active = 0;
 #pragma unroll
   for (int s = 0; s < RT_LAT_SLOTS; ++s)
@@ -234,6 +261,17 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
     const bool hit3 = (active >> 3) & 1u;
     if (p.depth) p.depth[pid] = hit3 ? LD(3) : INFINITY;
     if (p.index) p.index[pid] = hit3 ? LI(3) : INT32_MIN;
+  }
+  // Hit point p = cam + t d of each point (:326 / :345), formed once: it takes the place of t, distance and ray length,
+  // which nothing reads from here on.
+#define PX(s) s_ht[(s) * RT_THREADS + threadIdx.x]
+#define PY(s) s_hd[(s) * RT_THREADS + threadIdx.x]
+#define PZ(s) s_len[(s) * RT_THREADS + threadIdx.x]
+#pragma unroll
+  for (int s = 0; s < RT_LAT_SLOTS; ++s) {
+    if (!((active >> s) & 1u)) continue;
+    const float t = LT(s);
+    PX(s) = xadd(cx, xmul(t, SDX(s))); PY(s) = xadd(cy, xmul(t, SDY(s))); PZ(s) = xadd(cz, xmul(t, dz));
   }
 
   // ============================ shadow rays (at most one light) ============================
@@ -245,9 +283,7 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
 #pragma unroll
     for (int s = 0; s < RT_LAT_SLOTS; ++s) {
       if ((active >> s) & 1u) {
-        const float gx = -xsub(Lx, xadd(cx, xmul(LT(s), SDX(s))));
-        const float gy = -xsub(Ly, xadd(cy, xmul(LT(s), SDY(s))));
-        const float gz = -xsub(Lz, xadd(cz, xmul(LT(s), dz)));
+        const float gx = -xsub(Lx, PX(s)), gy = -xsub(Ly, PY(s)), gz = -xsub(Lz, PZ(s));
         glo[0] = fminf(glo[0], gx); ghi[0] = fmaxf(ghi[0], gx);
         glo[1] = fminf(glo[1], gy); ghi[1] = fmaxf(ghi[1], gy);
         glo[2] = fminf(glo[2], gz); ghi[2] = fmaxf(ghi[2], gz);
@@ -274,15 +310,15 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
     __syncthreads();
     RtCursor cursor = rt_cursor_scene(p.planes + (size_t)((p.n_tris + RT_TILE - 1) / RT_TILE) * RT_TILE * RT_REC_F4, p.n_tris);
     RtItem item;
-    bool have = rt_cursor_next<false, RT_TILE>(p, cursor, item);
-    if (threadIdx.x == 0 && have) rt_ring_issue<RT_TILE>(ring, item);
+    bool have = rt_cursor_next<false, RT_LAT_TILE>(p, cursor, item);
+    if (threadIdx.x == 0 && have) rt_ring_issue<RT_LAT_TILE>(ring, item);
     while (have) {
       const int buf = ring.issued & 1;
       ++ring.issued;
       __syncthreads();
       RtItem next_item;
-      const bool have_next = rt_cursor_next<false, RT_TILE>(p, cursor, next_item);
-      if (threadIdx.x == 0 && have_next) rt_ring_issue<RT_TILE>(ring, next_item);
+      const bool have_next = rt_cursor_next<false, RT_LAT_TILE>(p, cursor, next_item);
+      if (threadIdx.x == 0 && have_next) rt_ring_issue<RT_LAT_TILE>(ring, next_item);
       mbar_wait(&bars[buf], (ring.phase_bits >> buf) & 1u);
       ring.phase_bits ^= 1u << buf;
       const float4 *T = buf ? T1 : T0;
@@ -336,9 +372,7 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
 #pragma unroll
           for (int s = 0; s < RT_LAT_SLOTS; ++s) {
             if (!((todo >> s) & 1u)) continue;
-            const float px = xadd(cx, xmul(LT(s), SDX(s))), py = xadd(cy, xmul(LT(s), SDY(s))),
-                        pz = xadd(cz, xmul(LT(s), dz));
-            const float gx = -xsub(Lx, px), gy = -xsub(Ly, py), gz = -xsub(Lz, pz);
+            const float gx = -xsub(Lx, PX(s)), gy = -xsub(Ly, PY(s)), gz = -xsub(Lz, PZ(s));
             const float mU = fmaf(q0.x, gx, fmaf(q0.y, gy, q0.z * gz));
             const float mV = fmaf(q0.w, gx, fmaf(q1.x, gy, q1.y * gz));
             const float mW = fmaf(q1.z, gx, fmaf(q1.w, gy, q2.x * gz));
@@ -361,10 +395,8 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
             for (unsigned m = amb; m; m &= m - 1) {
               const int s = __ffs(m) - 1;
               if (sD == 0.0f || LI(s) != tri) continue;
-              const float px = xadd(cx, xmul(LT(s), SDX(s))), py = xadd(cy, xmul(LT(s), SDY(s))),
-                          pz = xadd(cz, xmul(LT(s), dz));
-              const float ox = xadd(px, xmul(n0, 0.00001f)), oy = xadd(py, xmul(n1, 0.00001f)),
-                          oz = xadd(pz, xmul(n2, 0.00001f));                                    // :394
+              const float ox = xadd(PX(s), xmul(n0, 0.00001f)), oy = xadd(PY(s), xmul(n1, 0.00001f)),
+                          oz = xadd(PZ(s), xmul(n2, 0.00001f));                                    // :394
               const float Dt = xdet3(xsub(ox, g0.x), xsub(oy, g0.y), xsub(oz, g0.z), g0.w, g1.x, g1.y, g1.z, g1.w, e2z);
               if (((Dt < 0.0f) != (sD < 0.0f)) && fabsf(Dt) > 1e-20f * fabsf(sD)) amb &= ~(1u << s);
             }
@@ -373,15 +405,14 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
           while (amb) {
             const int s = __ffs(amb) - 1;
             amb &= amb - 1;
-            const float px = xadd(cx, xmul(LT(s), SDX(s))), py = xadd(cy, xmul(LT(s), SDY(s))),
-                        pz = xadd(cz, xmul(LT(s), dz));
             ++n_exact;
-            if (rt_ex_shadow(p.geom, p.src, p.sph, tri, LI(s), px, py, pz, Lx, Ly, Lz)) occluded |= 1u << s;
+            if (rt_ex_shadow(p.geom, p.src, p.sph, tri, LI(s), PX(s), PY(s), PZ(s), Lx, Ly, Lz)) occluded |= 1u << s;
           }
         }
       }
     }
   }
+  RT_PHASE(3);
 
   // ---- sphere occluders + the lighting tail of DirectLight, and the surface colour, per hit point ----
 #pragma unroll
@@ -389,8 +420,7 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
     if ((valid >> s) & 1u) s_hit[SPT(s)] = (active >> s) & 1u;
   for (unsigned m = active; m; m &= m - 1) {
     const int s = __ffs(m) - 1;
-    const float px = xadd(cx, xmul(LT(s), SDX(s))), py = xadd(cy, xmul(LT(s), SDY(s))), pz = xadd(cz, xmul(LT(s), dz));
-    const RtShade o = rt_ex_shade(p.src, p.sph, p.n_sph, LI(s), px, py, pz, Lx, Ly, Lz, p.lights[0][4], p.lights[0][5],
+    const RtShade o = rt_ex_shade(p.src, p.sph, p.n_sph, LI(s), PX(s), PY(s), PZ(s), Lx, Ly, Lz, p.lights[0][4], p.lights[0][5],
                                   p.lights[0][6], (occluded >> s) & 1u, p.n_lights > 0);
     const int pt = SPT(s);
 #pragma unroll
@@ -399,7 +429,12 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
       s_shade[(3 + c) * RT_LAT_PTS + pt] = o.col[c];
     }
   }
+#ifdef RT_PROFILE_PHASES
+  if (lane == 0) s_phase[warp][4] = clock64();   // lane 0's own shade loop; [5] once the whole warp is through
+#endif
+  RT_PHASE(5);
   __syncthreads();
+  RT_PHASE(6);
 
   // ---- each pixel sums its nine samples in the reference's order (:151-156) ----
   unsigned n_hit = 0;
@@ -421,10 +456,24 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_lattice_kernel(c
   // the reference's counts: one shadow ray per hit sample of every pixel, shared points counted once per pixel
   rt_count(p.counters + 0, (unsigned long long)n_hit * p.n_lights);
   rt_count(p.counters + 1, (unsigned long long)n_exact);
+  RT_PHASE(7);
+#ifdef RT_PROFILE_PHASES
+  // index plane, top pixel row of every warp's 8 x 4 patch: lane k < 8 holds stamp k minus stamp 0 (lane 0: the SM)
+  __syncwarp();
+  if (live && p.index && lane < 8) {
+    unsigned smid;
+    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
+    p.index[pid] = lane == 0 ? (int)smid : (int)(s_phase[warp][lane] - s_phase[warp][0]);
+  }
+#endif
+#undef RT_PHASE
 #undef LT
 #undef LD
 #undef LI
 #undef LLEN
+#undef PX
+#undef PY
+#undef PZ
 #undef SDX
 #undef SDY
 #undef SPT
