@@ -104,6 +104,7 @@ ABI_SYMBOLS = [
     "render_raytrace", "render_raytrace_band", "draw_raytrace", "draw_raytrace_band",
     "b200_measure_fp32_peak", "rt_upload_scene", "rt_render_device",
     "render_raytrace_views", "draw_raytrace_views", "rt_render_views_device",
+    "render_raytrace_samples", "draw_raytrace_samples", "rt_render_samples_device",
     "rt_closest_hits", "rt_occluded", "rt_closest_hits_device", "rt_occluded_device",
     "rt_direct_light", "rt_direct_light_device",
     "render_raster_clipped", "render_raster", "render_raster_band", "draw_raster", "raster_read_buffers",
@@ -133,6 +134,9 @@ def load_library():
         _lib.rt_occluded_device.argtypes = [vp, vp, vp, i32, vp]
         _lib.rt_direct_light.argtypes = [vp, vp, i32, vp, i32, vp, i32, vp, i32, vp]
         _lib.rt_direct_light_device.argtypes = [vp, vp, i32, vp, i32, vp]
+        _lib.render_raytrace_samples.argtypes = [vp, vp, i32, vp, i32, vp, vp, i32, vp, i32, i32, vp, vp, vp]
+        _lib.draw_raytrace_samples.argtypes = [vp, vp, i32, vp, i32, vp, vp, i32, vp, i32, i32, vp]
+        _lib.rt_render_samples_device.argtypes = [vp, vp, vp, i32, vp, i32, i32, i32, i32, vp, vp, vp, vp]
     return _lib
 
 
@@ -329,6 +333,53 @@ class Renderer:
         rc = self.lib.rt_render_views_device(self.ctx, ca, int(k), la, len(lights), _ptr(d_rgb), _ptr(d_depth),
                                              _ptr(d_index), _ptr(d_argb))
         self._check(rc, "rt_render_views_device")
+
+    # ---- RT, the caller's sample pattern ------------------------------------------
+    @staticmethod
+    def _offsets(offsets):
+        """offsets: (S, 2) float32 -- sample k of a pixel is the ray along (dir.x + offsets[k, 0], dir.y + offsets[k, 1], f)."""
+        o = np.ascontiguousarray(offsets, np.float32)
+        if o.ndim != 2 or o.shape[1] != 2:
+            raise ValueError("offsets must be an (S, 2) array")
+        return o
+
+    def render_raytrace_samples(self, tris, spheres, cam, lights, offsets, depth_sample, want=("rgb", "depth", "index")):
+        """Draw with the caller's per-pixel sample offsets (render_raytrace_samples): rgb (H, W, 3), depth and index
+        (H, W) of sample depth_sample.  The reference's pattern, 0.5 * (i, j) for i, j in -1..1 with i outer, and
+        depth_sample = 4 give render_raytrace's frame."""
+        o = self._offsets(offsets)
+        W, H = cam.width, cam.height
+        rgb = np.zeros((H, W, 3), np.float32) if "rgb" in want else None
+        depth = np.zeros((H, W), np.float32) if "depth" in want else None
+        index = np.zeros((H, W), np.int32) if "index" in want else None
+        la = make_lights(lights)
+        rc = self.lib.render_raytrace_samples(
+            self.ctx, _ptr(tris), len(tris), _ptr(spheres), 0 if spheres is None else len(spheres),
+            ctypes.byref(cam), la, len(lights), _ptr(o), len(o), int(depth_sample), _ptr(rgb), _ptr(depth), _ptr(index))
+        self._check(rc, "render_raytrace_samples")
+        return dict(rgb=rgb, depth=depth, index=index)
+
+    def draw_raytrace_samples(self, tris, spheres, cam, lights, offsets, depth_sample=0, out=None):
+        """Packed frame (H, W) uint32 of render_raytrace_samples."""
+        o = self._offsets(offsets)
+        argb = np.zeros((cam.height, cam.width), np.uint32) if out is None else out
+        la = make_lights(lights)
+        rc = self.lib.draw_raytrace_samples(self.ctx, _ptr(tris), len(tris), _ptr(spheres),
+                                            0 if spheres is None else len(spheres), ctypes.byref(cam), la,
+                                            len(lights), _ptr(o), len(o), int(depth_sample), _ptr(argb))
+        self._check(rc, "draw_raytrace_samples")
+        return argb
+
+    def rt_render_samples_device(self, cam, lights, offsets, depth_sample, row_begin, row_end, d_rgb=None,
+                                 d_depth=None, d_index=None, d_argb=None):
+        """The uploaded scene with the caller's sample offsets into device pointers (ints) addressed as full
+        frames; asynchronous."""
+        o = self._offsets(offsets)
+        la = make_lights(lights)
+        rc = self.lib.rt_render_samples_device(self.ctx, ctypes.byref(cam), la, len(lights), _ptr(o), len(o),
+                                               int(depth_sample), int(row_begin), int(row_end), _ptr(d_rgb),
+                                               _ptr(d_depth), _ptr(d_index), _ptr(d_argb))
+        self._check(rc, "rt_render_samples_device")
 
     # ---- RT, ray queries --------------------------------------------------------
     @staticmethod

@@ -269,10 +269,11 @@ static int fill_frame(b200_ctx *ctx, const camera_t *cam, const light_t *lights,
   return B200_OK;
 }
 
-// One RT frame on device buffers; il_n / il_r: the 16-row block interleave (1, 0 = every row).
+// One RT frame on device buffers; il_n / il_r: the 16-row block interleave (1, 0 = every row); sp: the caller's
+// sample pattern (render_raytrace_samples), null for Draw's nine samples.
 static int rt_frame_device(b200_ctx *ctx, const camera_t *cam, const light_t *lights, int n_lights,
                            int row_begin, int row_end, float *d_rgb, float *d_depth, int32_t *d_index,
-                           uint32_t *d_argb, int il_n, int il_r) {
+                           uint32_t *d_argb, int il_n, int il_r, const RtSamplesParams *sp = nullptr) {
   RtFrame f;
   if (int rc = fill_frame(ctx, cam, lights, n_lights, row_begin, row_end, f)) return rc;
   cudaSetDevice(ctx->device);
@@ -283,12 +284,12 @@ static int rt_frame_device(b200_ctx *ctx, const camera_t *cam, const light_t *li
   CU_CHECK(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
   ctx->tl_n = 0;
   tl_mark(ctx, "frame start");
-  if (int rc = rt_launch(ctx, f, d_rgb, d_depth, d_index, d_argb)) return rc;
+  if (int rc = rt_launch(ctx, f, d_rgb, d_depth, d_index, d_argb, sp)) return rc;
   CU_CHECK(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
   uint64_t my_rows = 0;   // rows of this context's 16-row blocks
   for (int b = f.il_r; b * 16 < row_end - row_begin; b += f.il_n)
     my_rows += (uint64_t)((row_end - row_begin - b * 16) < 16 ? (row_end - row_begin - b * 16) : 16);
-  ctx->stats.primary_rays = (uint64_t)f.W * my_rows * 9u;
+  ctx->stats.primary_rays = (uint64_t)f.W * my_rows * (sp ? (uint64_t)sp->n : 9u);
   if (int rc = enqueue_counter_readback(ctx)) return rc;
   ctx->pending = 1;
   return B200_OK;
@@ -303,6 +304,104 @@ int rt_render_device(b200_ctx *ctx, const camera_t *cam, const light_t *lights, 
   SINGLE_ONLY(ctx);
   return rt_frame_device(ctx, cam, lights, n_lights, row_begin, row_end, d_rgb, d_depth, d_index, d_argb,
                          ctx->opt_rt_il_n, ctx->opt_rt_il_r);
+}
+
+}  // extern "C"
+
+// ---- RT, the caller's sample pattern per pixel (render_raytrace_samples) ----------------
+// (also the multi-GPU context's check, before the rows are shared out)
+int check_samples(b200_ctx *ctx, const camera_t *cam, const light_t *lights, int n_lights, const float *offsets,
+                  int n_samples, int depth_sample) {
+  if (int rc = check_camera(ctx, cam)) return rc;
+  if (n_lights < 0 || n_lights > B200_MAX_LIGHTS || (n_lights > 0 && !lights))
+    return ctx_fail(ctx, B200_EINVAL, "bad lights (at most 8)");
+  if (n_samples < 1 || n_samples > B200_RT_MAX_SAMPLES) return ctx_fail(ctx, B200_EINVAL, "n_samples must be 1..64");
+  if (!offsets) return ctx_fail(ctx, B200_EINVAL, "null offsets");
+  // every bound of the primary-ray filters is built for offsets within +-0.5 (DESIGN §3.5); !(<=) also catches NaN
+  for (int k = 0; k < 2 * n_samples; ++k)
+    if (!(fabsf(offsets[k]) <= 0.5f)) return ctx_fail(ctx, B200_EINVAL, "every offset must be finite and within +-0.5");
+  if (depth_sample < 0 || depth_sample >= n_samples) return ctx_fail(ctx, B200_EINVAL, "depth_sample must be below n_samples");
+  return B200_OK;
+}
+
+static void samples_params(const float *offsets, int n_samples, int depth_sample, RtSamplesParams &sp) {
+  memset(&sp, 0, sizeof sp);
+  sp.n = n_samples;
+  sp.depth_sample = depth_sample;
+  memcpy(sp.off, offsets, 2 * (size_t)n_samples * sizeof(float));
+}
+
+extern "C" {
+static int copy_out(b200_ctx *ctx, void *host, const void *dev, size_t bytes);
+}
+
+// The host-pointer samples entries on one device: rows [row0, row1) into the staging buffers, then one copy per
+// output into the band-sized host buffers.
+int rt_samples_band(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                    const camera_t *cam, const light_t *lights, int n_lights, const float *offsets, int n_samples,
+                    int depth_sample, int row0, int row1, float *rgb_out, float *depth_out, int32_t *index_out,
+                    uint32_t *argb_out) {
+  if (int rc = check_samples(ctx, cam, lights, n_lights, offsets, n_samples, depth_sample)) return rc;
+  RtSamplesParams sp;
+  samples_params(offsets, n_samples, depth_sample, sp);
+  if (int rc = rt_upload_scene(ctx, tris, n_tris, spheres, n_spheres)) return rc;
+  const size_t npix = (size_t)cam->width * cam->height;
+  if (rgb_out) if (int rc = ensure(ctx, ctx->out_rgb, npix * 3 * sizeof(float))) return rc;
+  if (depth_out) if (int rc = ensure(ctx, ctx->out_depth, npix * sizeof(float))) return rc;
+  if (index_out) if (int rc = ensure(ctx, ctx->out_index, npix * sizeof(int32_t))) return rc;
+  if (argb_out) if (int rc = ensure(ctx, ctx->out_argb, npix * sizeof(uint32_t))) return rc;
+  if (int rc = rt_frame_device(ctx, cam, lights, n_lights, row0, row1, rgb_out ? (float *)ctx->out_rgb.p : nullptr,
+                               depth_out ? (float *)ctx->out_depth.p : nullptr,
+                               index_out ? (int32_t *)ctx->out_index.p : nullptr,
+                               argb_out ? (uint32_t *)ctx->out_argb.p : nullptr, 1, 0, &sp))
+    return rc;
+  const size_t off = (size_t)row0 * cam->width, cnt = (size_t)(row1 - row0) * cam->width;
+  if (int rc = copy_out(ctx, rgb_out, (float *)ctx->out_rgb.p + 3 * off, cnt * 3 * sizeof(float))) return rc;
+  if (int rc = copy_out(ctx, depth_out, (float *)ctx->out_depth.p + off, cnt * sizeof(float))) return rc;
+  if (int rc = copy_out(ctx, index_out, (int32_t *)ctx->out_index.p + off, cnt * sizeof(int32_t))) return rc;
+  if (int rc = copy_out(ctx, argb_out, (uint32_t *)ctx->out_argb.p + off, cnt * sizeof(uint32_t))) return rc;
+  return finish_stats(ctx);
+}
+
+extern "C" {
+
+int render_raytrace_samples(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres,
+                            int n_spheres, const camera_t *cam, const light_t *lights, int n_lights,
+                            const float *offsets, int n_samples, int depth_sample, float *rgb_out, float *depth_out,
+                            int32_t *index_out) {
+  if (!ctx) return B200_EINVAL;
+  if (ctx->multi)
+    return multi_raytrace_samples(ctx, tris, n_tris, spheres, n_spheres, cam, lights, n_lights, offsets, n_samples,
+                                  depth_sample, rgb_out, depth_out, index_out, nullptr);
+  if (int rc = check_camera(ctx, cam)) return rc;
+  return rt_samples_band(ctx, tris, n_tris, spheres, n_spheres, cam, lights, n_lights, offsets, n_samples,
+                         depth_sample, 0, cam->height, rgb_out, depth_out, index_out, nullptr);
+}
+
+int draw_raytrace_samples(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres,
+                          int n_spheres, const camera_t *cam, const light_t *lights, int n_lights,
+                          const float *offsets, int n_samples, int depth_sample, uint32_t *argb_out) {
+  if (!ctx) return B200_EINVAL;
+  if (!argb_out) return ctx_fail(ctx, B200_EINVAL, "null framebuffer");
+  if (ctx->multi)
+    return multi_raytrace_samples(ctx, tris, n_tris, spheres, n_spheres, cam, lights, n_lights, offsets, n_samples,
+                                  depth_sample, nullptr, nullptr, nullptr, argb_out);
+  if (int rc = check_camera(ctx, cam)) return rc;
+  return rt_samples_band(ctx, tris, n_tris, spheres, n_spheres, cam, lights, n_lights, offsets, n_samples,
+                         depth_sample, 0, cam->height, nullptr, nullptr, nullptr, argb_out);
+}
+
+// The interleave options apply here as they do to rt_render_device.
+int rt_render_samples_device(b200_ctx *ctx, const camera_t *cam, const light_t *lights, int n_lights,
+                             const float *offsets, int n_samples, int depth_sample, int row_begin, int row_end,
+                             float *d_rgb, float *d_depth, int32_t *d_index, uint32_t *d_argb) {
+  if (!ctx) return B200_EINVAL;
+  SINGLE_ONLY(ctx);
+  if (int rc = check_samples(ctx, cam, lights, n_lights, offsets, n_samples, depth_sample)) return rc;
+  RtSamplesParams sp;
+  samples_params(offsets, n_samples, depth_sample, sp);
+  return rt_frame_device(ctx, cam, lights, n_lights, row_begin, row_end, d_rgb, d_depth, d_index, d_argb,
+                         ctx->opt_rt_il_n, ctx->opt_rt_il_r, &sp);
 }
 
 }  // extern "C"

@@ -232,6 +232,14 @@ struct RtFrame {
   float lights[8][7];  // pos[4], colour[3]
 };
 #define B200_MAX_LIGHTS 8
+// The caller's per-pixel sample pattern (render_raytrace_samples): sample k of a pixel is the ray along
+// (dir.x + off[2k], dir.y + off[2k+1], f), k < n; depth / index are those of sample depth_sample.  A kernel
+// parameter of its own (__grid_constant__), so that RtKParams -- and every other kernel -- stays as it is.
+struct RtSamplesParams {
+  int n;
+  int depth_sample;
+  float off[2 * B200_RT_MAX_SAMPLES];
+};
 constexpr int RT_GRID_AUTO_TRIS = 1024;   // B200_OPT_RT_GRID = 0: scenes this large get direction grids
 
 // spec = true: pipelined (no host synchronisation; see b200_ctx::rast_spec)
@@ -271,8 +279,9 @@ static inline int band_slice_edge(int row0, int rows, int i, int k, int align) {
   const int e = (int)((long long)rows * (all - rem) / all) / align * align;
   return row0 + e;
 }
+// sp: the caller's sample pattern (render_raytrace_samples), or null for Draw's nine samples
 int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int32_t *d_index,
-              uint32_t *d_argb);
+              uint32_t *d_argb, const RtSamplesParams *sp = nullptr);
 // rt_rays.cu: one ray query on the uploaded scene, n > 0 rays; d_hits (closest hits) or d_occ + d_max (occlusion)
 int rt_launch_rays(b200_ctx *ctx, const rt_ray *d_rays, const float *d_max, int n, rt_intersection *d_hits,
                    uint8_t *d_occ);
@@ -305,6 +314,17 @@ int multi_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const
 int check_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
                        const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights,
                        const float *power_out);   // api.cu
+int multi_raytrace_samples(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                           const camera_t *cam, const light_t *lights, int n_lights, const float *offsets,
+                           int n_samples, int depth_sample, float *rgb_out, float *depth_out, int32_t *index_out,
+                           uint32_t *argb_out);
+int check_samples(b200_ctx *ctx, const camera_t *cam, const light_t *lights, int n_lights, const float *offsets,
+                  int n_samples, int depth_sample);   // api.cu
+// The host-pointer samples entry on one device: rows [row0, row1) into band-sized outputs (api.cu)
+int rt_samples_band(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                    const camera_t *cam, const light_t *lights, int n_lights, const float *offsets, int n_samples,
+                    int depth_sample, int row0, int row1, float *rgb_out, float *depth_out, int32_t *index_out,
+                    uint32_t *argb_out);
 int multi_raster(b200_ctx *ctx, const rast_triangle *room, int n_room, const rast_triangle *boxes, int n_boxes,
                  const camera_t *cam, const rast_light_t *light, int row_begin, int row_end, float *rgb_out,
                  float *depth_out, int32_t *index_out, uint32_t *argb_out);

@@ -310,6 +310,32 @@ int multi_raytrace(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_
   return B200_OK;
 }
 
+// The caller's sample pattern: device i renders an even share of the 16-row blocks, [a_i, a_i+1) rows, with the
+// single-device entry and returns it straight into its slice of the caller's buffers.  The balanced bands of
+// ordinary frames are neither read nor moved: their costs are for Draw's nine samples.
+int multi_raytrace_samples(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
+                           const camera_t *cam, const light_t *lights, int n_lights, const float *offsets,
+                           int n_samples, int depth_sample, float *rgb_out, float *depth_out, int32_t *index_out,
+                           uint32_t *argb_out) {
+  b200_multi *mc = ctx->multi;
+  if (int rc = check_samples(ctx, cam, lights, n_lights, offsets, n_samples, depth_sample)) return rc;
+  const int H = cam->height, blocks = (H + 15) / 16, n = mc->n;
+  const size_t W = (size_t)cam->width;
+  const int rc = multi_run(ctx, [&](int i) -> int {
+    const int a = std::min(H, (int)((long long)blocks * i / n) * 16), b = std::min(H, (int)((long long)blocks * (i + 1) / n) * 16);
+    b200_ctx *c = mc->child[i];
+    c->stats = b200_stats{};
+    if (b <= a) return B200_OK;
+    const size_t off = (size_t)a * W;
+    return rt_samples_band(c, tris, n_tris, spheres, n_spheres, cam, lights, n_lights, offsets, n_samples, depth_sample,
+                           a, b, rgb_out ? rgb_out + 3 * off : nullptr, depth_out ? depth_out + off : nullptr,
+                           index_out ? index_out + off : nullptr, argb_out ? argb_out + off : nullptr);
+  });
+  if (rc != B200_OK) return rc;
+  multi_sum_stats(ctx);
+  return B200_OK;
+}
+
 // Batched views: whole views go to whole devices -- device i renders the contiguous run [k_i, k_i+1) of the views
 // with the single-device views path and returns it straight into its slice of the caller's buffers.  No bands.
 int multi_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,

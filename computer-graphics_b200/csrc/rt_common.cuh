@@ -84,6 +84,16 @@ __device__ __forceinline__ void rt_store_pixel(const RtKParams &p, size_t pid, b
   if (p.argb) p.argb[pid] = put_pixel_argb(o[0], o[1], o[2]);
 }
 
+// The same for n samples per pixel (render_raytrace_samples): pixelColour / (float)n.  A NaN sum is passed on as it
+// is, as x86 and xdiv_const do (__fdiv_rn would give its own NaN), so n = 9 stores what rt_store_pixel stores.
+__device__ __forceinline__ void rt_store_pixel_n(const RtKParams &p, size_t pid, bool valid, const float *pix, int n) {
+  float o[3] = {0.f, 0.f, 0.f};
+  if (valid)
+    for (int c = 0; c < 3; ++c) o[c] = pix[c] != pix[c] ? pix[c] : xdiv(pix[c], (float)n);
+  if (p.rgb) { p.rgb[3 * pid] = o[0]; p.rgb[3 * pid + 1] = o[1]; p.rgb[3 * pid + 2] = o[2]; }
+  if (p.argb) p.argb[pid] = put_pixel_argb(o[0], o[1], o[2]);
+}
+
 __device__ __forceinline__ void rt_count(unsigned long long *counter, unsigned long long n) {
   // warp-level sum, then one atomic per warp
 #pragma unroll

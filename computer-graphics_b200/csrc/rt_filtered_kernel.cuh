@@ -249,13 +249,20 @@ __device__ __forceinline__ size_t rt_views_pid(const RtKParams &p) {
 
 // VIEWS (scene streaming only): blockIdx.z is the view of a batched launch; its camera comes from vp, its camera
 // records and dt_cam from its own slices, its pixels go to frame blockIdx.z of the outputs.
-template <bool MULTI, bool GRID, bool VIEWS>
-__device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtViewsParams *vp) {
+// SAMPLES: the pixel's samples are the caller's table sp (render_raytrace_samples) instead of the 3x3 grid.  They
+// run in groups of up to nine in the nine slots of the hit state -- a primary walk and the shadow phase per group --
+// and the pixel's running sum carries over from group to group in sample order.  Every bound of the primary-ray
+// filters is built for a bundle of +-0.5 around the pixel's direction; rounding is monotone, so RN(dir + o) for
+// |o| <= 0.5 lies between RN(dir - 0.5) and RN(dir + 0.5) and those bounds hold unchanged (DESIGN §3.5).
+template <bool MULTI, bool GRID, bool VIEWS, bool SAMPLES = false>
+__device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtViewsParams *vp,
+                                                 const RtSamplesParams *sp = nullptr) {
   // Scene streaming (GRID = false): the block shares one double-buffered ring of RT_TILE-record
   // tiles, refilled under __syncthreads.  Cell lists (GRID = true): every WARP has its own ring of
   // RT_WTILE-record tiles, its own cell set and no block barrier at all -- the lists are short,
   // and a warp on a dense or silhouette patch no longer holds the other seven back.
   static_assert(!(GRID && VIEWS), "batched views run the scene-streaming kernel");
+  static_assert(!(SAMPLES && VIEWS), "batched views take Draw's nine samples");
   constexpr int TILE = GRID ? RT_WTILE : RT_TILE;
   constexpr int NRING = GRID ? RT_THREADS / 32 : 1;
   extern __shared__ __align__(128) float4 tile_smem[];  // NRING x 2 x TILE x 3 float4 (+ GRID: NRING x 2 x TILE int)
@@ -328,6 +335,21 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
   // the nine sample directions (:134-137): three x offsets, three y offsets
   const float dxs[3] = {xadd(dir0, xmul(0.5f, -1.0f)), xadd(dir0, xmul(0.5f, 0.0f)), xadd(dir0, xmul(0.5f, 1.0f))};
   const float dys[3] = {xadd(dir1, xmul(0.5f, -1.0f)), xadd(dir1, xmul(0.5f, 0.0f)), xadd(dir1, xmul(0.5f, 1.0f))};
+  // SAMPLES: slot k of the current group is sample smp0 + k of the caller's table, for k < ng
+  int smp0 = 0, ng = 9;
+#define RT_SDX(k) (SAMPLES ? xadd(dir0, sp->off[2 * (smp0 + (k))]) : dxs[(k) / 3])
+#define RT_SDY(k) (SAMPLES ? xadd(dir1, sp->off[2 * (smp0 + (k)) + 1]) : dys[(k) % 3])
+  unsigned n_exact = 0;
+#ifdef RT_PROFILE_COUNTERS
+  unsigned prof_cnt[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+#define RT_PC(i) (++prof_cnt[i])
+#else
+#define RT_PC(i)
+#endif
+#ifdef RT_PROFILE_CLOCK   // diagnostic build: where the long-running warps are and why (profiles/rt_block_cycles.py)
+  const long long prof_t0 = clock64();
+  unsigned prof_recs = 0, prof_cells = 0, prof_l1 = 0, prof_l2 = 0, prof_ex0 = 0;
+#endif
 
   // The closest hit of each of the nine samples lives in shared memory (thread-private slices,
   // conflict-free: word k of thread t at [k][t]) instead of 27 registers.
@@ -345,22 +367,22 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
   float len_r[GRID ? 9 : 1], pix_r[GRID ? 3 : 1];
 #define LEN(k) (GRID ? len_r[GRID ? (k) : 0] : s_len[(k) * RT_THREADS + threadIdx.x])
 #define PIX(c) (GRID ? pix_r[GRID ? (c) : 0] : s_len[(9 + (c)) * RT_THREADS + threadIdx.x])
+  // SAMPLES: hit samples of the earlier groups (shadow-ray count), and whether any sample of the pixel hit
+  unsigned n_hit = 0;
+  bool any_hit = false;
+  const int n_groups = SAMPLES ? (sp->n + 8) / 9 : 1;
+  for (int grp = 0; grp < n_groups; ++grp) {   // (one pass without SAMPLES; the body keeps its indentation)
+  if (SAMPLES) {
+    smp0 = 9 * grp;
+    ng = min(9, sp->n - smp0);
+    if (grp > 0) ring_sync();   // the last light phase of the previous group is done with the ring and the cell set
+  }
 #pragma unroll
   for (int k = 0; k < 9; ++k) {
     HT(k) = 0.f; HD(k) = FLT_MAX; HI(k) = 0;
-    LEN(k) = xsqrt(xdot3(dxs[k / 3], dys[k % 3], dz, dxs[k / 3], dys[k % 3], dz));
+    if (SAMPLES && k >= ng) continue;
+    LEN(k) = xsqrt(xdot3(RT_SDX(k), RT_SDY(k), dz, RT_SDX(k), RT_SDY(k), dz));
   }
-  unsigned n_exact = 0;
-#ifdef RT_PROFILE_COUNTERS
-  unsigned prof_cnt[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-#define RT_PC(i) (++prof_cnt[i])
-#else
-#define RT_PC(i)
-#endif
-#ifdef RT_PROFILE_CLOCK   // diagnostic build: where the long-running warps are and why (profiles/rt_block_cycles.py)
-  const long long prof_t0 = clock64();
-  unsigned prof_recs = 0, prof_cells = 0, prof_l1 = 0, prof_l2 = 0, prof_ex0 = 0;
-#endif
 
   // ============================ primary rays ============================
   {
@@ -435,7 +457,8 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
           // ---- L2 / EX: per ray ----
 #pragma unroll
           for (int k = 0; k < 9; ++k) {
-            const float dx = dxs[k / 3], dy = dys[k % 3];
+            if (SAMPLES && k >= ng) continue;
+            const float dx = RT_SDX(k), dy = RT_SDY(k);
             const float mU = fmaf(q0.x, dx, fmaf(q0.y, dy, q0.z));
             const float mV = fmaf(q0.w, dx, fmaf(q1.x, dy, q1.y));
             const float mW = fmaf(q1.z, dx, fmaf(q1.w, dy, q2.x));
@@ -483,7 +506,8 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
       }
 #pragma unroll
       for (int k = 0; k < 9; ++k) {
-        const float dx = dxs[k / 3], dy = dys[k % 3];
+        if (SAMPLES && k >= ng) continue;
+        const float dx = RT_SDX(k), dy = RT_SDY(k);
         if (!rt_sphere_may_hit(p.sph[s], cx, cy, cz, dx, dy, dz)) continue;
         const RtSphT h = rt_ex_sphere(p.sph + s, cx, cy, cz, dx, dy, dz);
         if (h.hit && h.t < HD(k)) { HT(k) = h.t; HD(k) = h.t; HI(k) = -1 - s; }
@@ -495,7 +519,16 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
 #pragma unroll
   for (int k = 0; k < 9; ++k)
     if (live && HD(k) < FLT_MAX) active |= 1u << k;
-  if (live) {
+  if (SAMPLES) {
+    const int kd = sp->depth_sample - smp0;   // the depth sample's slot, if it is in this group
+    if (live && kd >= 0 && kd < ng) {
+      const bool hit = (active >> kd) & 1u;
+      if (p.depth) p.depth[PID] = hit ? HD(kd) : INFINITY;
+      if (p.index) p.index[PID] = hit ? HI(kd) : INT32_MIN;
+    }
+    n_hit += __popc(active);
+    any_hit = any_hit || active != 0;
+  } else if (live) {
     const bool hit4 = (active >> 4) & 1u;
     if (p.depth) p.depth[PID] = hit4 ? HD(4) : INFINITY;
     if (p.index) p.index[PID] = hit4 ? HI(4) : INT32_MIN;
@@ -507,8 +540,10 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
   // ============================ shadow rays ============================
   constexpr int NL = MULTI ? B200_MAX_LIGHTS : 1;
   float dl[MULTI ? NL * 27 : 1];
+  if (!SAMPLES || grp == 0) {
 #pragma unroll
-  for (int c = 0; c < 3; ++c) PIX(c) = 0.f;
+    for (int c = 0; c < 3; ++c) PIX(c) = 0.f;
+  }
   const unsigned warp_active = __ballot_sync(0xffffffffu, active != 0);
   for (int l = 0; l < p.n_lights; ++l) {
     const float Lx = p.lights[l][0], Ly = p.lights[l][1], Lz = p.lights[l][2];
@@ -518,8 +553,8 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
 #pragma unroll(GRID ? 1 : 9)   // grid kernels: smaller code (their warps run out of step and miss in the instruction cache)
     for (int k = 0; k < 9; ++k) {
       if ((active >> k) & 1u) {
-        const float gx = -xsub(Lx, xadd(cx, xmul(HT(k), dxs[k / 3])));
-        const float gy = -xsub(Ly, xadd(cy, xmul(HT(k), dys[k % 3])));
+        const float gx = -xsub(Lx, xadd(cx, xmul(HT(k), RT_SDX(k))));
+        const float gy = -xsub(Ly, xadd(cy, xmul(HT(k), RT_SDY(k))));
         const float gz = -xsub(Lz, xadd(cz, xmul(HT(k), dz)));
         glo[0] = fminf(glo[0], gx); ghi[0] = fmaxf(ghi[0], gx);
         glo[1] = fminf(glo[1], gy); ghi[1] = fmaxf(ghi[1], gy);
@@ -554,7 +589,7 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
 #pragma unroll(GRID ? 1 : 9)   // grid kernels: smaller code (their warps run out of step and miss in the instruction cache)
       for (int k = 0; k < 9; ++k) {
         if ((active >> k) & 1u) {
-          const float g[3] = {-xsub(Lx, xadd(cx, xmul(HT(k), dxs[k / 3]))), -xsub(Ly, xadd(cy, xmul(HT(k), dys[k % 3]))),
+          const float g[3] = {-xsub(Lx, xadd(cx, xmul(HT(k), RT_SDX(k)))), -xsub(Ly, xadd(cy, xmul(HT(k), RT_SDY(k)))),
                               -xsub(Lz, xadd(cz, xmul(HT(k), dz)))};
           const bool in_a = (ax == 0 ? g[0] : (ax == 1 ? g[1] : g[2])) < mid;
 #pragma unroll
@@ -606,8 +641,8 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
 #pragma unroll(GRID ? 1 : 9)   // grid kernels: smaller code (their warps run out of step and miss in the instruction cache)
       for (int k = 0; k < 9; ++k) {
         if (!((active >> k) & 1u)) continue;
-        const float gx = -xsub(Lx, xadd(cx, xmul(HT(k), dxs[k / 3])));
-        const float gy = -xsub(Ly, xadd(cy, xmul(HT(k), dys[k % 3])));
+        const float gx = -xsub(Lx, xadd(cx, xmul(HT(k), RT_SDX(k))));
+        const float gy = -xsub(Ly, xadd(cy, xmul(HT(k), RT_SDY(k))));
         const float gz = -xsub(Lz, xadd(cz, xmul(HT(k), dz)));
         if (last >= 0) {
           // Usually the same cell as the previous sample: four products instead of two divisions.
@@ -743,7 +778,7 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
 #pragma unroll
             for (int k = 0; k < 9; ++k) {
               if (!((todo >> k) & 1u) || ((occluded >> k) & 1u)) continue;
-              const float px = xadd(cx, xmul(HT(k), dxs[k / 3])), py = xadd(cy, xmul(HT(k), dys[k % 3])),
+              const float px = xadd(cx, xmul(HT(k), RT_SDX(k))), py = xadd(cy, xmul(HT(k), RT_SDY(k))),
                           pz = xadd(cz, xmul(HT(k), dz));
               const float gx = -xsub(Lx, px), gy = -xsub(Ly, py), gz = -xsub(Lz, pz);
               const float mU = fmaf(q0.x, gx, fmaf(q0.y, gy, q0.z * gz));
@@ -772,7 +807,7 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
 #pragma unroll
           for (int k = 0; k < 9; ++k) {
             if (!((todo >> k) & 1u) || ((occluded >> k) & 1u)) continue;
-            const float px = xadd(cx, xmul(HT(k), dxs[k / 3])), py = xadd(cy, xmul(HT(k), dys[k % 3])),
+            const float px = xadd(cx, xmul(HT(k), RT_SDX(k))), py = xadd(cy, xmul(HT(k), RT_SDY(k))),
                         pz = xadd(cz, xmul(HT(k), dz));
             const float gx = -xsub(Lx, px), gy = -xsub(Ly, py), gz = -xsub(Lz, pz);
             const float mU = fmaf(q0.x, gx, fmaf(q0.y, gy, q0.z * gz));
@@ -802,7 +837,8 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
               const int k = __ffs(m) - 1;
               if (sD == 0.0f || HI(k) != tri) continue;
               float px, py, pz;
-              rt_hit_point(cx, cy, cz, dxs[1], dys[1], dz, HT(k), k, px, py, pz);
+              if (SAMPLES) { px = xadd(cx, xmul(HT(k), RT_SDX(k))); py = xadd(cy, xmul(HT(k), RT_SDY(k))); pz = xadd(cz, xmul(HT(k), dz)); }
+              else rt_hit_point(cx, cy, cz, dxs[1], dys[1], dz, HT(k), k, px, py, pz);
               const float ox = xadd(px, xmul(n0, 0.00001f)), oy = xadd(py, xmul(n1, 0.00001f)),
                           oz = xadd(pz, xmul(n2, 0.00001f));                                    // :394
               const float Dt = xdet3(xsub(ox, g0.x), xsub(oy, g0.y), xsub(oz, g0.z), g0.w, g1.x, g1.y, g1.z, g1.w, e2z);
@@ -814,7 +850,8 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
             const int k = __ffs(amb) - 1;
             amb &= amb - 1;
             float px, py, pz;
-            rt_hit_point(cx, cy, cz, dxs[1], dys[1], dz, HT(k), k, px, py, pz);
+            if (SAMPLES) { px = xadd(cx, xmul(HT(k), RT_SDX(k))); py = xadd(cy, xmul(HT(k), RT_SDY(k))); pz = xadd(cz, xmul(HT(k), dz)); }
+            else rt_hit_point(cx, cy, cz, dxs[1], dys[1], dz, HT(k), k, px, py, pz);
             ++n_exact;
 #ifdef RT_PROFILE_COUNTERS
             RT_PC(7);
@@ -831,7 +868,7 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
 #pragma unroll(GRID ? 1 : 9)   // grid kernels: smaller code (their warps run out of step and miss in the instruction cache)
     for (int k = 0; k < 9; ++k) {
       if (!((active >> k) & 1u)) continue;
-      const float px = xadd(cx, xmul(HT(k), dxs[k / 3])), py = xadd(cy, xmul(HT(k), dys[k % 3])),
+      const float px = xadd(cx, xmul(HT(k), RT_SDX(k))), py = xadd(cy, xmul(HT(k), RT_SDY(k))),
                   pz = xadd(cz, xmul(HT(k), dz));
       const RtShade s = rt_ex_shade(p.src, p.sph, p.n_sph, HI(k), px, py, pz, Lx, Ly, Lz, p.lights[l][4],
                                     p.lights[l][5], p.lights[l][6], (occluded >> k) & 1u, 1);
@@ -857,7 +894,7 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
             PIX(1) = xadd(PIX(1), dl[(l * 9 + k) * 3 + 1]);
             PIX(2) = xadd(PIX(2), dl[(l * 9 + k) * 3 + 2]);
           }
-        const float px = xadd(cx, xmul(HT(k), dxs[k / 3])), py = xadd(cy, xmul(HT(k), dys[k % 3])),
+        const float px = xadd(cx, xmul(HT(k), RT_SDX(k))), py = xadd(cy, xmul(HT(k), RT_SDY(k))),
                     pz = xadd(cz, xmul(HT(k), dz));
         const RtShade s = rt_ex_shade(p.src, p.sph, 0, HI(k), px, py, pz, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0, 0);
         PIX(0) = xadd(PIX(0), xmul(s.col[0], 0.5f));
@@ -865,10 +902,20 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
         PIX(2) = xadd(PIX(2), xmul(s.col[2], 0.5f));
       }
     }
-    const float pix[3] = {PIX(0), PIX(1), PIX(2)};
-    rt_store_pixel(p, PID, active != 0, pix);
+    if (!SAMPLES) {
+      const float pix[3] = {PIX(0), PIX(1), PIX(2)};
+      rt_store_pixel(p, PID, active != 0, pix);
+    }
   }
-  rt_count(p.counters + 0, (unsigned long long)__popc(active) * p.n_lights);
+  if (!SAMPLES) rt_count(p.counters + 0, (unsigned long long)__popc(active) * p.n_lights);
+  }   // groups of samples
+  if (SAMPLES) {
+    if (live) {
+      const float pix[3] = {PIX(0), PIX(1), PIX(2)};
+      rt_store_pixel_n(p, PID, any_hit, pix, sp->n);
+    }
+    rt_count(p.counters + 0, (unsigned long long)n_hit * p.n_lights);
+  }
   rt_count(p.counters + 1, (unsigned long long)n_exact);
   if (GRID && p.block_cost && lane == 0)   // what the next frame's plan is made from
     atomicMax(p.block_cost + s_cost_at[warp], (((unsigned)clock() - s_cost_t0[warp]) >> 8) * (s_split ? 8u : 1u));
@@ -898,5 +945,11 @@ __global__ void __launch_bounds__(RT_THREADS, RT_MIN_BLOCKS) rt_filtered_views_k
                                                                                       const __grid_constant__ RtViewsParams v) {
   rt_filtered_body<MULTI, false, true>(p, &v);
 }
+// The caller's sample pattern (render_raytrace_samples): launched as rt_filtered_kernel, with the table in s.
+template <bool MULTI, bool GRID>
+__global__ void __launch_bounds__(RT_THREADS, GRID ? 2 : RT_MIN_BLOCKS)
+    rt_filtered_samples_kernel(const __grid_constant__ RtKParams p, const __grid_constant__ RtSamplesParams s) {
+  rt_filtered_body<MULTI, GRID, false, true>(p, nullptr, &s);
+}
 
-int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p);
+int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p, const RtSamplesParams *sp = nullptr);

@@ -10,6 +10,8 @@
 //   rt_lattice_kernel     (rt_lattice_kernel.cuh) the same filters for frames whose
 //                         sample rays form a half-pixel lattice: each shared sample
 //                         ray is traced once per 16x16 pixel block.
+// Frames with the caller's own sample offsets (render_raytrace_samples) run the *_samples_kernel instantiations
+// of the filtered and brute-force bodies, never the lattice kernel.
 #include "rt_exact.cuh"
 #include "rt_filtered.cuh"
 #include "rt_lattice_kernel.cuh"
@@ -64,7 +66,9 @@ __global__ void rt_prep_geom_kernel(const rt_triangle *__restrict__ src, int n, 
 // ------------------------------------------------------------------------------
 // brute force, reference arithmetic everywhere
 // ------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) rt_bruteforce_kernel(const __grid_constant__ RtKParams p) {
+// SAMPLES: the caller's sample table sp (render_raytrace_samples) instead of the 3x3 grid.
+template <bool SAMPLES>
+__device__ __forceinline__ void rt_bruteforce_body(const RtKParams &p, const RtSamplesParams *sp) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   // each warp owns an 8x4 pixel patch; a 128-thread block covers 16x8 pixels
   const int u = blockIdx.x * 16 + (warp & 1) * 8 + (lane & 7);
@@ -78,14 +82,15 @@ __global__ void __launch_bounds__(128) rt_bruteforce_kernel(const __grid_constan
     float pix[3] = {0.f, 0.f, 0.f};
     bool valid = false;
     const size_t pid = (size_t)v * p.W + u;
-    for (int i = -1; i <= 1; ++i) {
-      for (int j = -1; j <= 1; ++j) {
-        const float dx = xadd(dir0, xmul(0.5f, (float)i));   // :137
-        const float dy = xadd(dir1, xmul(0.5f, (float)j));
+    // (SAMPLES: one loop over the table, i = 0 and j = k)
+    for (int i = SAMPLES ? 0 : -1; i <= (SAMPLES ? 0 : 1); ++i) {
+      for (int j = SAMPLES ? 0 : -1; j <= (SAMPLES ? sp->n - 1 : 1); ++j) {
+        const float dx = SAMPLES ? xadd(dir0, sp->off[2 * j]) : xadd(dir0, xmul(0.5f, (float)i));   // :137
+        const float dy = SAMPLES ? xadd(dir1, sp->off[2 * j + 1]) : xadd(dir1, xmul(0.5f, (float)j));
         const float dz = p.focal;
         const RtHit h = rt_closest_bruteforce(p, p.cam[0], p.cam[1], p.cam[2], dx, dy, dz);
         const bool hit = h.dist < FLT_MAX;
-        if (i == 0 && j == 0) {
+        if (SAMPLES ? j == sp->depth_sample : (i == 0 && j == 0)) {
           if (p.depth) p.depth[pid] = hit ? h.dist : INFINITY;
           if (p.index) p.index[pid] = hit ? h.idx : INT32_MIN;
         }
@@ -116,9 +121,18 @@ __global__ void __launch_bounds__(128) rt_bruteforce_kernel(const __grid_constan
         pix[2] = xadd(pix[2], xmul(col[2], 0.5f));
       }
     }
-    rt_store_pixel(p, pid, valid, pix);
+    if (SAMPLES) rt_store_pixel_n(p, pid, valid, pix, sp->n);
+    else rt_store_pixel(p, pid, valid, pix);
   }
   rt_count_shadow(p, n_shadow);
+}
+
+__global__ void __launch_bounds__(128) rt_bruteforce_kernel(const __grid_constant__ RtKParams p) {
+  rt_bruteforce_body<false>(p, nullptr);
+}
+__global__ void __launch_bounds__(128) rt_bruteforce_samples_kernel(const __grid_constant__ RtKParams p,
+                                                                    const __grid_constant__ RtSamplesParams s) {
+  rt_bruteforce_body<true>(p, &s);
 }
 
 // ------------------------------------------------------------------------------
@@ -168,7 +182,7 @@ static void rt_kparams(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_d
 }
 
 int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int32_t *d_index,
-              uint32_t *d_argb) {
+              uint32_t *d_argb, const RtSamplesParams *sp) {
   RtKParams p;
   rt_kparams(ctx, f, d_rgb, d_depth, d_index, d_argb, p);
   const int rows = f.row1 - f.row0;
@@ -178,13 +192,18 @@ int rt_launch(b200_ctx *ctx, const RtFrame &f, float *d_rgb, float *d_depth, int
   if (my_blocks == 0) return B200_OK;
   if (ctx->opt_rt_bruteforce) {
     dim3 grid((f.W + 15) / 16, 2 * my_blocks);
-    rt_bruteforce_kernel<<<grid, 128, 0, ctx->stream>>>(p);
-    tl_mark(ctx, "rt_bruteforce_kernel");
+    if (sp) {
+      rt_bruteforce_samples_kernel<<<grid, 128, 0, ctx->stream>>>(p, *sp);
+      tl_mark(ctx, "rt_bruteforce_samples_kernel");
+    } else {
+      rt_bruteforce_kernel<<<grid, 128, 0, ctx->stream>>>(p);
+      tl_mark(ctx, "rt_bruteforce_kernel");
+    }
     ctx->stats.kernel_launches++;
     CU_CHECK(ctx, cudaGetLastError());
     return B200_OK;
   }
-  return rt_launch_filtered(ctx, f, p);
+  return rt_launch_filtered(ctx, f, p, sp);
 }
 
 // scenes this large get direction grids (declared in common.cuh; measured crossover at 4K: ~800 triangles)
@@ -270,6 +289,10 @@ static int rt_set_smem_limits(b200_ctx *ctx) {
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_views_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_views_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_samples_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)most));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_samples_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)most));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_samples_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
+  CU_CHECK(ctx, cudaFuncSetAttribute(rt_filtered_samples_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_STREAM_SMEM));
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_lattice_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RT_LAT_LAUNCH_SMEM));
   // four blocks per SM need 220 KB of it: all that the SM can give to shared memory
   CU_CHECK(ctx, cudaFuncSetAttribute(rt_lattice_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared));
@@ -277,7 +300,9 @@ static int rt_set_smem_limits(b200_ctx *ctx) {
   return B200_OK;
 }
 
-int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
+// sp (the caller's sample pattern): the filtered kernels' samples instantiations, never the lattice kernel, and
+// the block plan of gridded frames is neither read nor written.
+int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p, const RtSamplesParams *sp) {
   const int n = ctx->rt_n_tris;
   const int n_tiles = (n + RT_TILE - 1) / RT_TILE;
   const size_t origin_stride = (size_t)n_tiles * RT_TILE * RT_REC_F4;
@@ -384,7 +409,7 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
     const unsigned nb = grid.x * grid.y;
     dim3 lgrid = grid;
     p.plan = nullptr; p.plan_n = nullptr; p.block_cost = nullptr; p.gx = (int)grid.x;
-    if (grid.x <= 4096 && grid.y <= 4096 && ctx->opt_rt_plan) {
+    if (grid.x <= 4096 && grid.y <= 4096 && ctx->opt_rt_plan && !sp) {
       const size_t frame_blocks = (size_t)grid.x * (size_t)((f.H + 15) / 16 + 1);
       const size_t plan_cap = (size_t)nb + 7 * (size_t)RT_PLAN_MAX_SPLIT;
       // (sized for the whole frame whatever this launch's share: a buffer that grew would lose the cost history)
@@ -407,11 +432,21 @@ int rt_launch_filtered(b200_ctx *ctx, const RtFrame &f, RtKParams &p) {
       p.block_cost = cost + (size_t)cur * frame_blocks;
       ctx->rt_plan_shape = shape; ctx->rt_plan_valid = 1; ctx->rt_plan_flip = cur;
     }
-    if (f.n_lights > 1)
+    if (sp && f.n_lights > 1)
+      rt_filtered_samples_kernel<true, true><<<lgrid, RT_THREADS, gsmem, ctx->stream>>>(p, *sp);
+    else if (sp)
+      rt_filtered_samples_kernel<false, true><<<lgrid, RT_THREADS, gsmem, ctx->stream>>>(p, *sp);
+    else if (f.n_lights > 1)
       rt_filtered_kernel<true, true><<<lgrid, RT_THREADS, gsmem, ctx->stream>>>(p);
     else
       rt_filtered_kernel<false, true><<<lgrid, RT_THREADS, gsmem, ctx->stream>>>(p);
-    tl_mark(ctx, "rt_filtered_kernel<grid>");
+    tl_mark(ctx, sp ? "rt_filtered_samples_kernel<grid>" : "rt_filtered_kernel<grid>");
+  } else if (sp) {
+    if (f.n_lights > 1)
+      rt_filtered_samples_kernel<true, false><<<grid, RT_THREADS, smem, ctx->stream>>>(p, *sp);
+    else
+      rt_filtered_samples_kernel<false, false><<<grid, RT_THREADS, smem, ctx->stream>>>(p, *sp);
+    tl_mark(ctx, "rt_filtered_samples_kernel");
   } else if (f.n_lights <= 1 && rt_lattice_exact(f)) {
     rt_lattice_kernel<<<grid, RT_THREADS, RT_LAT_LAUNCH_SMEM, ctx->stream>>>(p);
     tl_mark(ctx, "rt_lattice_kernel");

@@ -278,6 +278,44 @@ int rt_render_views_device(b200_ctx *ctx, const camera_t *cams, int n_views, con
                            int n_lights, float *d_rgb, float *d_depth, int32_t *d_index,
                            uint32_t *d_argb);
 
+/* ---- RT, the caller's own sample pattern per pixel -----------------------------
+ * Draw (skeleton.cpp:123-168) with the 3x3 sample grid replaced by the caller's n_samples offsets.
+ * Sample k of pixel (u, v) is the ray from cam->pos along (dir.x + offsets[2k], dir.y + offsets[2k+1], focal),
+ *   where dir = R * vec4(u - W/2, v - H/2, focal, 1) exactly as in Draw, and the offset is added to the rotated
+ *   direction in float32, one rounding.  The reference's pattern is offsets = 0.5*(i, j) with i = -1..1 outer
+ *   and j = -1..1 inner.
+ * Per pixel, samples are taken in the caller's order.  A sample that hits adds DirectLight for each light in order,
+ *   then colour * 0.5f.  The pixel is pix / (float)n_samples if any sample hit, else 0.
+ * depth / index are those of sample depth_sample.  The meaning is render_raytrace's (distance or +inf;
+ *   triangle, -1 - sphere, or B200_INDEX_MISS).  Passing the reference's pattern with depth_sample = 4 gives
+ *   render_raytrace's frame bit for bit.
+ *   - 1 <= n_samples <= 64; every offset finite with |offset| <= 0.5 (+-0.5 and -0.0 allowed);
+ *     0 <= depth_sample < n_samples; camera and lights as render_raytrace.  Otherwise B200_EINVAL.
+ *   - b200_get_stats: primary_rays = W * rows * n_samples, shadow_rays = hit samples * n_lights (device-counted),
+ *     prim_tests, exact_evals, kernel_launches, gpu_ms as for frames.
+ *   - Any output may be NULL, except that draw_raytrace_samples needs argb_out.  B200_OPT_RT_BRUTEFORCE = 1 runs
+ *     the per-pixel exact loop; B200_OPT_RT_GRID chooses streaming or gridded as for frames.  The samples run in
+ *     groups of up to nine per walk of the scene, so a frame costs about ceil(n_samples / 9) nine-sample frames of
+ *     the filtered kernel; the half-pixel lattice kernel of render_raytrace is never used, and the gridded-frame
+ *     block plan of B200_OPT_RT_PLAN is neither read nor written.
+ *   - On a b200_init_multi context the host entries give each device an even, 16-row-aligned band of rows,
+ *     returned straight into its slice of the caller's buffers; rt_render_samples_device returns B200_EINVAL
+ *     there.  A pipelined raster frame in flight is finished first. */
+#define B200_RT_MAX_SAMPLES 64
+int render_raytrace_samples(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres,
+                            int n_spheres, const camera_t *cam, const light_t *lights, int n_lights,
+                            const float *offsets, int n_samples, int depth_sample,
+                            float *rgb_out, float *depth_out, int32_t *index_out);
+int draw_raytrace_samples(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres,
+                          int n_spheres, const camera_t *cam, const light_t *lights, int n_lights,
+                          const float *offsets, int n_samples, int depth_sample, uint32_t *argb_out);
+/* The scene of rt_upload_scene, DEVICE outputs addressed as full frames, rows [row_begin, row_end),
+ * asynchronous on b200_stream(ctx).  Offsets are HOST memory, as lights are.  B200_OPT_RT_INTERLEAVE_N / _R
+ * apply as for rt_render_device. */
+int rt_render_samples_device(b200_ctx *ctx, const camera_t *cam, const light_t *lights, int n_lights,
+                             const float *offsets, int n_samples, int depth_sample, int row_begin, int row_end,
+                             float *d_rgb, float *d_depth, int32_t *d_index, uint32_t *d_argb);
+
 /* ---- RT, ray queries: ClosestIntersection for rays the caller supplies --------
  * raytracer/Source/skeleton.cpp:40-45 (struct Intersection), :263-363 (ClosestIntersection) and
  * :394-397 (DirectLight's shadow test `ClosestIntersection(...) && distance < r_mag`), for any rays:
