@@ -149,6 +149,18 @@ def _ptr(a):
     return a.ctypes.data_as(ctypes.c_void_p)
 
 
+def _len(a):
+    """Length of an optional array: 0 for None."""
+    return 0 if a is None else len(a)
+
+
+def _outputs(want, shape):
+    """(rgb, depth, index) arrays of `shape` pixels for the outputs named in `want`, None for the others."""
+    return (np.zeros(shape + (3,), np.float32) if "rgb" in want else None,
+            np.zeros(shape, np.float32) if "depth" in want else None,
+            np.zeros(shape, np.int32) if "index" in want else None)
+
+
 def make_camera(pos, focal, R, width, height):
     c = Camera()
     c.pos[:] = [float(x) for x in pos]
@@ -251,12 +263,10 @@ class Renderer:
         W, H = cam.width, cam.height
         row_end = H if row_end is None else row_end
         rows = row_end - row_begin
-        rgb = np.zeros((rows, W, 3), np.float32) if "rgb" in want else None
-        depth = np.zeros((rows, W), np.float32) if "depth" in want else None
-        index = np.zeros((rows, W), np.int32) if "index" in want else None
+        rgb, depth, index = _outputs(want, (rows, W))
         la = make_lights(lights)
         rc = self.lib.render_raytrace_band(
-            self.ctx, _ptr(tris), len(tris), _ptr(spheres), 0 if spheres is None else len(spheres),
+            self.ctx, _ptr(tris), len(tris), _ptr(spheres), _len(spheres),
             ctypes.byref(cam), la, len(lights), int(row_begin), int(row_end),
             _ptr(rgb), _ptr(depth), _ptr(index))
         self._check(rc, "render_raytrace_band")
@@ -266,7 +276,7 @@ class Renderer:
         argb = np.zeros((cam.height, cam.width), np.uint32) if out is None else out
         la = make_lights(lights)
         rc = self.lib.draw_raytrace(self.ctx, _ptr(tris), len(tris), _ptr(spheres),
-                                    0 if spheres is None else len(spheres), ctypes.byref(cam), la,
+                                    _len(spheres), ctypes.byref(cam), la,
                                     len(lights), _ptr(argb))
         self._check(rc, "draw_raytrace")
         return argb
@@ -275,7 +285,7 @@ class Renderer:
         """out_ptr: host address (e.g. pinned memory) of a band-sized uint32 buffer."""
         la = make_lights(lights)
         rc = self.lib.draw_raytrace_band(self.ctx, _ptr(tris), len(tris), _ptr(spheres),
-                                         0 if spheres is None else len(spheres), ctypes.byref(cam), la,
+                                         _len(spheres), ctypes.byref(cam), la,
                                          len(lights), int(row_begin), int(row_end), _ptr(out_ptr))
         self._check(rc, "draw_raytrace_band")
 
@@ -286,7 +296,7 @@ class Renderer:
 
     def rt_upload_scene(self, tris, spheres):
         rc = self.lib.rt_upload_scene(self.ctx, _ptr(tris), len(tris), _ptr(spheres),
-                                      0 if spheres is None else len(spheres))
+                                      _len(spheres))
         self._check(rc, "rt_upload_scene")
 
     def rt_render_device(self, cam, lights, row_begin, row_end, d_rgb=None, d_depth=None,
@@ -303,12 +313,10 @@ class Renderer:
         (K, H, W, 3) / (K, H, W), view k equal to render_raytrace with cams[k]."""
         ca, k = _cameras(cams)
         W, H = (ca[0].width, ca[0].height) if k else (0, 0)
-        rgb = np.zeros((k, H, W, 3), np.float32) if "rgb" in want else None
-        depth = np.zeros((k, H, W), np.float32) if "depth" in want else None
-        index = np.zeros((k, H, W), np.int32) if "index" in want else None
+        rgb, depth, index = _outputs(want, (k, H, W))
         la = make_lights(lights)
         rc = self.lib.render_raytrace_views(
-            self.ctx, _ptr(tris), len(tris), _ptr(spheres), 0 if spheres is None else len(spheres),
+            self.ctx, _ptr(tris), len(tris), _ptr(spheres), _len(spheres),
             ca, int(k), la, len(lights), _ptr(rgb), _ptr(depth), _ptr(index))
         self._check(rc, "render_raytrace_views")
         return dict(rgb=rgb, depth=depth, index=index)
@@ -320,7 +328,7 @@ class Renderer:
         argb = np.zeros((k, H, W), np.uint32) if out is None else out
         la = make_lights(lights)
         rc = self.lib.draw_raytrace_views(self.ctx, _ptr(tris), len(tris), _ptr(spheres),
-                                          0 if spheres is None else len(spheres), ca, int(k), la, len(lights),
+                                          _len(spheres), ca, int(k), la, len(lights),
                                           _ptr(argb))
         self._check(rc, "draw_raytrace_views")
         return argb
@@ -349,12 +357,10 @@ class Renderer:
         depth_sample = 4 give render_raytrace's frame."""
         o = self._offsets(offsets)
         W, H = cam.width, cam.height
-        rgb = np.zeros((H, W, 3), np.float32) if "rgb" in want else None
-        depth = np.zeros((H, W), np.float32) if "depth" in want else None
-        index = np.zeros((H, W), np.int32) if "index" in want else None
+        rgb, depth, index = _outputs(want, (H, W))
         la = make_lights(lights)
         rc = self.lib.render_raytrace_samples(
-            self.ctx, _ptr(tris), len(tris), _ptr(spheres), 0 if spheres is None else len(spheres),
+            self.ctx, _ptr(tris), len(tris), _ptr(spheres), _len(spheres),
             ctypes.byref(cam), la, len(lights), _ptr(o), len(o), int(depth_sample), _ptr(rgb), _ptr(depth), _ptr(index))
         self._check(rc, "render_raytrace_samples")
         return dict(rgb=rgb, depth=depth, index=index)
@@ -365,7 +371,7 @@ class Renderer:
         argb = np.zeros((cam.height, cam.width), np.uint32) if out is None else out
         la = make_lights(lights)
         rc = self.lib.draw_raytrace_samples(self.ctx, _ptr(tris), len(tris), _ptr(spheres),
-                                            0 if spheres is None else len(spheres), ctypes.byref(cam), la,
+                                            _len(spheres), ctypes.byref(cam), la,
                                             len(lights), _ptr(o), len(o), int(depth_sample), _ptr(argb))
         self._check(rc, "draw_raytrace_samples")
         return argb
@@ -395,8 +401,8 @@ class Renderer:
         sphere_index (distance < FLT_MAX iff the ray hit something)."""
         rays = self._rays(rays)
         out = np.zeros(len(rays), RT_INTERSECTION)
-        rc = self.lib.rt_closest_hits(self.ctx, _ptr(tris), 0 if tris is None else len(tris), _ptr(spheres),
-                                      0 if spheres is None else len(spheres), _ptr(rays), len(rays), _ptr(out))
+        rc = self.lib.rt_closest_hits(self.ctx, _ptr(tris), _len(tris), _ptr(spheres),
+                                      _len(spheres), _ptr(rays), len(rays), _ptr(out))
         self._check(rc, "rt_closest_hits")
         return dict(position=out["position"].copy(), distance=out["distance"].copy(),
                     triangle_index=out["triangle_index"].copy(), sphere_index=out["sphere_index"].copy())
@@ -408,8 +414,8 @@ class Renderer:
         if len(md) != len(rays):
             raise ValueError("one max_distance per ray")
         out = np.zeros(len(rays), np.uint8)
-        rc = self.lib.rt_occluded(self.ctx, _ptr(tris), 0 if tris is None else len(tris), _ptr(spheres),
-                                  0 if spheres is None else len(spheres), _ptr(rays), _ptr(md), len(rays), _ptr(out))
+        rc = self.lib.rt_occluded(self.ctx, _ptr(tris), _len(tris), _ptr(spheres),
+                                  _len(spheres), _ptr(rays), _ptr(md), len(rays), _ptr(out))
         self._check(rc, "rt_occluded")
         return out.astype(bool)
 
@@ -442,8 +448,8 @@ class Renderer:
         hits = self._hits(hits)
         out = np.zeros((len(hits), len(lights), 3), np.float32)
         la = make_lights(lights)
-        rc = self.lib.rt_direct_light(self.ctx, _ptr(tris), 0 if tris is None else len(tris), _ptr(spheres),
-                                      0 if spheres is None else len(spheres), _ptr(hits), len(hits), la, len(lights),
+        rc = self.lib.rt_direct_light(self.ctx, _ptr(tris), _len(tris), _ptr(spheres),
+                                      _len(spheres), _ptr(hits), len(hits), la, len(lights),
                                       _ptr(out))
         self._check(rc, "rt_direct_light")
         return out
@@ -458,9 +464,7 @@ class Renderer:
     # ---- RAST ----------------------------------------------------------------
     def render_raster_clipped(self, clipped, cam, light, want=("rgb", "depth", "index")):
         W, H = cam.width, cam.height
-        rgb = np.zeros((H, W, 3), np.float32) if "rgb" in want else None
-        depth = np.zeros((H, W), np.float32) if "depth" in want else None
-        index = np.zeros((H, W), np.int32) if "index" in want else None
+        rgb, depth, index = _outputs(want, (H, W))
         rc = self.lib.render_raster_clipped(self.ctx, _ptr(clipped), len(clipped), ctypes.byref(cam),
                                             ctypes.byref(light), _ptr(rgb), _ptr(depth), _ptr(index))
         self._check(rc, "render_raster_clipped")
@@ -470,9 +474,7 @@ class Renderer:
         W, H = cam.width, cam.height
         row_end = H if row_end is None else row_end
         rows = row_end - row_begin
-        rgb = np.zeros((rows, W, 3), np.float32) if "rgb" in want else None
-        depth = np.zeros((rows, W), np.float32) if "depth" in want else None
-        index = np.zeros((rows, W), np.int32) if "index" in want else None
+        rgb, depth, index = _outputs(want, (rows, W))
         rc = self.lib.render_raster_band(self.ctx, _ptr(room), len(room), _ptr(boxes), len(boxes),
                                          ctypes.byref(cam), ctypes.byref(light), int(row_begin), int(row_end),
                                          _ptr(rgb), _ptr(depth), _ptr(index))

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <string.h>
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -291,40 +292,31 @@ int rt_launch_direct_light(b200_ctx *ctx, const rt_intersection *d_hits, int n, 
 // whole frames of n_views cameras of one size, frame k of each output at k * W * H (rgb: times 3)
 int rt_launch_views(b200_ctx *ctx, const RtFrame *fs, int n_views, float *d_rgb, float *d_depth, int32_t *d_index,
                     uint32_t *d_argb);
+// The four outputs of a frame, host or device pointers; a null pointer is an output nobody asked for.
+struct Outputs {
+  float *rgb = nullptr, *depth = nullptr;
+  int32_t *index = nullptr;
+  uint32_t *argb = nullptr;
+  // the same outputs from pixel `px` on
+  Outputs at(size_t px) const {
+    return {rgb ? rgb + 3 * px : nullptr, depth ? depth + px : nullptr, index ? index + px : nullptr,
+            argb ? argb + px : nullptr};
+  }
+};
+// api.cu: rows [row_begin, row_end) of the whole Draw on the scene already uploaded, into band-sized host outputs
+int rast_band_resident(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, int row_begin, int row_end,
+                       const Outputs &host);
 // multi.cu: entry points of a multi-GPU context (api.cu forwards to these)
 void multi_destroy(b200_ctx *ctx);
 int multi_synchronize(b200_ctx *ctx);
 int multi_set_option(b200_ctx *ctx, int option, int value);
 int multi_rast_set_textures(b200_ctx *ctx, const rast_textures_t *tex);
-int multi_raytrace(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-                   const camera_t *cam, const light_t *lights, int n_lights, int row_begin, int row_end,
-                   float *rgb_out, float *depth_out, int32_t *index_out, uint32_t *argb_out);
-int multi_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-                         const camera_t *cams, int n_views, const light_t *lights, int n_lights, float *rgb_out,
-                         float *depth_out, int32_t *index_out, uint32_t *argb_out);
-int check_views(b200_ctx *ctx, const camera_t *cams, int n_views, const light_t *lights, int n_lights);   // api.cu
-// ray queries: max_distance / occ_out for an occlusion query, out for a closest-hit query
-int multi_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-               const rt_ray *rays, const float *max_distance, int n_rays, rt_intersection *out, uint8_t *occ_out,
-               bool occlusion);
-int check_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-               const rt_ray *rays, const float *max_distance, int n_rays, const void *out, bool occlusion);   // api.cu
-int multi_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-                       const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights, float *power_out);
-int check_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-                       const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights,
-                       const float *power_out);   // api.cu
-int multi_raytrace_samples(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-                           const camera_t *cam, const light_t *lights, int n_lights, const float *offsets,
-                           int n_samples, int depth_sample, float *rgb_out, float *depth_out, int32_t *index_out,
-                           uint32_t *argb_out);
-int check_samples(b200_ctx *ctx, const camera_t *cam, const light_t *lights, int n_lights, const float *offsets,
-                  int n_samples, int depth_sample);   // api.cu
-// The host-pointer samples entry on one device: rows [row0, row1) into band-sized outputs (api.cu)
-int rt_samples_band(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-                    const camera_t *cam, const light_t *lights, int n_lights, const float *offsets, int n_samples,
-                    int depth_sample, int row0, int row1, float *rgb_out, float *depth_out, int32_t *index_out,
-                    uint32_t *argb_out);
+// job(child, a, b): the single-device work of items [a, b) on one device of a multi-GPU context
+using MultiJob = std::function<int(b200_ctx *, int, int)>;
+// Items [0, count) in even shares of whole `align`-item units, one share per device; sums the devices' stats.
+int multi_split(b200_ctx *ctx, int count, int align, const MultiJob &job);
+// Rows [0, rows) of a raytraced frame in bands balanced on the measured cost of earlier frames.
+int multi_raytrace(b200_ctx *ctx, int rows, const MultiJob &job);
+// The whole Draw of rows [row_begin, row_end) in balanced bands; the arguments have been checked (api.cu).
 int multi_raster(b200_ctx *ctx, const rast_triangle *room, int n_room, const rast_triangle *boxes, int n_boxes,
-                 const camera_t *cam, const rast_light_t *light, int row_begin, int row_end, float *rgb_out,
-                 float *depth_out, int32_t *index_out, uint32_t *argb_out);
+                 const camera_t *cam, const rast_light_t *light, int row_begin, int row_end, const Outputs &host);

@@ -273,137 +273,50 @@ int multi_set_option(b200_ctx *ctx, int option, int value) {
   return rc;
 }
 
-// ---- raytracer ------------------------------------------------------------------------
-int multi_raytrace(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-                   const camera_t *cam, const light_t *lights, int n_lights, int row_begin, int row_end,
-                   float *rgb_out, float *depth_out, int32_t *index_out, uint32_t *argb_out) {
+// Runs job(child i, edges[i], edges[i + 1]) on every device whose share is not empty and sums the devices' stats.
+static int multi_run_edges(b200_ctx *ctx, const std::vector<int> &edges, const MultiJob &job) {
   b200_multi *mc = ctx->multi;
-  if (!cam || cam->width <= 0 || cam->height <= 0) return ctx_fail(ctx, B200_EINVAL, "bad camera");
-  if (row_begin < 0 || row_end > cam->height || row_begin > row_end) return ctx_fail(ctx, B200_EINVAL, "bad row band");
-  const int rows = row_end - row_begin, n = mc->n;
+  const int rc = multi_run(ctx, [&](int i) -> int {
+    b200_ctx *c = mc->child[i];
+    c->stats = b200_stats{};
+    return edges[i + 1] > edges[i] ? job(c, edges[i], edges[i + 1]) : B200_OK;
+  });
+  if (rc == B200_OK) multi_sum_stats(ctx);
+  return rc;
+}
+
+// Views, rays, hits and the rows of sample-pattern frames (whose cost says nothing about Draw's nine samples, so the
+// balanced bands are neither read nor moved): device i takes the contiguous run of units [u_i, u_i+1) and returns
+// it straight into its slice of the caller's buffers.
+int multi_split(b200_ctx *ctx, int count, int align, const MultiJob &job) {
+  const int n = ctx->multi->n;
+  const long long units = ((long long)count + align - 1) / align;
+  std::vector<int> edges(n + 1);
+  for (int i = 0; i <= n; ++i) edges[i] = (int)std::min<long long>(count, units * i / n * align);
+  return multi_run_edges(ctx, edges, job);
+}
+
+// Edges of the next frame of `kind` on bands of `rows` rows: the bands move only on the evidence of a frame that ran
+// on the same bands as its predecessor -- every other frame while they are still converging.
+static void multi_settled_edges(b200_multi *mc, int kind, int rows, int align, double tolerance,
+                                std::vector<int> &edges) {
+  const bool have = mc->edges_h[kind] == rows && (int)mc->edges[kind].size() == mc->n + 1;
+  if (have && !mc->settled[kind]) edges = mc->edges[kind];
+  else multi_band_edges(have ? mc->edges[kind] : std::vector<int>(), mc->cost[kind], rows, mc->n, align, edges, tolerance);
+  mc->settled[kind] = have && edges == mc->edges[kind];
+}
+
+// ---- raytracer ------------------------------------------------------------------------
+int multi_raytrace(b200_ctx *ctx, int rows, const MultiJob &job) {
+  b200_multi *mc = ctx->multi;
   std::vector<int> edges;
   // Large scenes run their blocks from a plan made of the previous frame's block costs, which every device keeps
   // for the rows IT rendered (rt_plan_kernel): the frame after a band moved is dearer on the rows it gained, and
   // balancing on that cost sent the edges back and forth (8 GPUs, 100 800 triangles: costs +-50 % from frame to
-  // frame, never settled).  So the bands move only on the evidence of a frame that ran on the same bands as its
-  // predecessor -- every other frame while they are still converging.
-  const bool have = mc->edges_h[0] == rows && (int)mc->edges[0].size() == n + 1;
-  if (have && !mc->settled[0]) edges = mc->edges[0];
-  else multi_band_edges(have ? mc->edges[0] : std::vector<int>(), mc->cost[0], rows, n, 16, edges);
-  mc->settled[0] = have && edges == mc->edges[0];
-  const size_t W = (size_t)cam->width;
-  const int rc = multi_run(ctx, [&](int i) -> int {
-    const int a = row_begin + edges[i], b = row_begin + edges[i + 1];
-    b200_ctx *c = mc->child[i];
-    c->stats = b200_stats{};
-    if (b <= a) return B200_OK;
-    const size_t off = (size_t)(a - row_begin) * W;
-    if (argb_out)
-      return draw_raytrace_band(c, tris, n_tris, spheres, n_spheres, cam, lights, n_lights, a, b, argb_out + off);
-    return render_raytrace_band(c, tris, n_tris, spheres, n_spheres, cam, lights, n_lights, a, b,
-                                rgb_out ? rgb_out + 3 * off : nullptr, depth_out ? depth_out + off : nullptr,
-                                index_out ? index_out + off : nullptr);
-  });
-  if (rc != B200_OK) return rc;
+  // frame, never settled).  Hence settled edges only.
+  multi_settled_edges(mc, 0, rows, 16, 1.06, edges);
+  if (int rc = multi_run_edges(ctx, edges, job)) return rc;
   multi_note_cost(mc, 0, edges, rows);
-  multi_sum_stats(ctx);
-  return B200_OK;
-}
-
-// The caller's sample pattern: device i renders an even share of the 16-row blocks, [a_i, a_i+1) rows, with the
-// single-device entry and returns it straight into its slice of the caller's buffers.  The balanced bands of
-// ordinary frames are neither read nor moved: their costs are for Draw's nine samples.
-int multi_raytrace_samples(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-                           const camera_t *cam, const light_t *lights, int n_lights, const float *offsets,
-                           int n_samples, int depth_sample, float *rgb_out, float *depth_out, int32_t *index_out,
-                           uint32_t *argb_out) {
-  b200_multi *mc = ctx->multi;
-  if (int rc = check_samples(ctx, cam, lights, n_lights, offsets, n_samples, depth_sample)) return rc;
-  const int H = cam->height, blocks = (H + 15) / 16, n = mc->n;
-  const size_t W = (size_t)cam->width;
-  const int rc = multi_run(ctx, [&](int i) -> int {
-    const int a = std::min(H, (int)((long long)blocks * i / n) * 16), b = std::min(H, (int)((long long)blocks * (i + 1) / n) * 16);
-    b200_ctx *c = mc->child[i];
-    c->stats = b200_stats{};
-    if (b <= a) return B200_OK;
-    const size_t off = (size_t)a * W;
-    return rt_samples_band(c, tris, n_tris, spheres, n_spheres, cam, lights, n_lights, offsets, n_samples, depth_sample,
-                           a, b, rgb_out ? rgb_out + 3 * off : nullptr, depth_out ? depth_out + off : nullptr,
-                           index_out ? index_out + off : nullptr, argb_out ? argb_out + off : nullptr);
-  });
-  if (rc != B200_OK) return rc;
-  multi_sum_stats(ctx);
-  return B200_OK;
-}
-
-// Batched views: whole views go to whole devices -- device i renders the contiguous run [k_i, k_i+1) of the views
-// with the single-device views path and returns it straight into its slice of the caller's buffers.  No bands.
-int multi_raytrace_views(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-                         const camera_t *cams, int n_views, const light_t *lights, int n_lights, float *rgb_out,
-                         float *depth_out, int32_t *index_out, uint32_t *argb_out) {
-  b200_multi *mc = ctx->multi;
-  if (int rc = check_views(ctx, cams, n_views, lights, n_lights)) return rc;
-  const size_t npix = (size_t)cams[0].width * cams[0].height;
-  const int n = mc->n;
-  const int rc = multi_run(ctx, [&](int i) -> int {
-    const int a = (int)((long long)n_views * i / n), b = (int)((long long)n_views * (i + 1) / n);
-    b200_ctx *c = mc->child[i];
-    c->stats = b200_stats{};
-    if (b <= a) return B200_OK;
-    const size_t off = (size_t)a * npix;
-    if (argb_out)
-      return draw_raytrace_views(c, tris, n_tris, spheres, n_spheres, cams + a, b - a, lights, n_lights, argb_out + off);
-    return render_raytrace_views(c, tris, n_tris, spheres, n_spheres, cams + a, b - a, lights, n_lights,
-                                 rgb_out ? rgb_out + 3 * off : nullptr, depth_out ? depth_out + off : nullptr,
-                                 index_out ? index_out + off : nullptr);
-  });
-  if (rc != B200_OK) return rc;
-  multi_sum_stats(ctx);
-  return B200_OK;
-}
-
-// Ray queries: device i answers the contiguous run [k_i, k_i+1) of the rays with the single-device entry and returns
-// it straight into its slice of the caller's output, as multi_raytrace_views does with views.
-int multi_rays(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-               const rt_ray *rays, const float *max_distance, int n_rays, rt_intersection *out, uint8_t *occ_out,
-               bool occlusion) {
-  b200_multi *mc = ctx->multi;
-  if (int rc = check_rays(ctx, tris, n_tris, spheres, n_spheres, rays, max_distance, n_rays,
-                          occlusion ? (const void *)occ_out : (const void *)out, occlusion))
-    return rc;
-  if (n_rays == 0) return B200_OK;
-  const int n = mc->n;
-  const int rc = multi_run(ctx, [&](int i) -> int {
-    const int a = (int)((long long)n_rays * i / n), b = (int)((long long)n_rays * (i + 1) / n);
-    b200_ctx *c = mc->child[i];
-    c->stats = b200_stats{};
-    if (b <= a) return B200_OK;
-    if (occlusion) return rt_occluded(c, tris, n_tris, spheres, n_spheres, rays + a, max_distance + a, b - a, occ_out + a);
-    return rt_closest_hits(c, tris, n_tris, spheres, n_spheres, rays + a, b - a, out + a);
-  });
-  if (rc != B200_OK) return rc;
-  multi_sum_stats(ctx);
-  return B200_OK;
-}
-
-// DirectLight for caller-supplied hits: device i shades the contiguous run [k_i, k_i+1) of the hits, every light.
-int multi_direct_light(b200_ctx *ctx, const rt_triangle *tris, int n_tris, const rt_sphere *spheres, int n_spheres,
-                       const rt_intersection *hits, int n_hits, const light_t *lights, int n_lights, float *power_out) {
-  b200_multi *mc = ctx->multi;
-  if (int rc = check_direct_light(ctx, tris, n_tris, spheres, n_spheres, hits, n_hits, lights, n_lights, power_out))
-    return rc;
-  if (n_hits == 0 || n_lights == 0) return B200_OK;
-  const int n = mc->n;
-  const int rc = multi_run(ctx, [&](int i) -> int {
-    const int a = (int)((long long)n_hits * i / n), b = (int)((long long)n_hits * (i + 1) / n);
-    b200_ctx *c = mc->child[i];
-    c->stats = b200_stats{};
-    if (b <= a) return B200_OK;
-    return rt_direct_light(c, tris, n_tris, spheres, n_spheres, hits + a, b - a, lights, n_lights,
-                           power_out + (size_t)a * n_lights * 3);
-  });
-  if (rc != B200_OK) return rc;
-  multi_sum_stats(ctx);
   return B200_OK;
 }
 
@@ -413,27 +326,16 @@ int multi_rast_set_textures(b200_ctx *ctx, const rast_textures_t *tex) {
   return multi_run(ctx, [&](int i) -> int { return rast_set_textures(ctx->multi->child[i], tex); });
 }
 
-int rast_band_resident(b200_ctx *ctx, const camera_t *cam, const rast_light_t *light, int row_begin, int row_end,
-                       float *rgb_out, float *depth_out, int32_t *index_out, uint32_t *argb_out);   // api.cu
-
 int multi_raster(b200_ctx *ctx, const rast_triangle *room, int n_room, const rast_triangle *boxes, int n_boxes,
-                 const camera_t *cam, const rast_light_t *light, int row_begin, int row_end, float *rgb_out,
-                 float *depth_out, int32_t *index_out, uint32_t *argb_out) {
+                 const camera_t *cam, const rast_light_t *light, int row_begin, int row_end, const Outputs &host) {
   b200_multi *mc = ctx->multi;
-  if (!cam || cam->width <= 0 || cam->height <= 0) return ctx_fail(ctx, B200_EINVAL, "bad camera");
-  if (!light) return ctx_fail(ctx, B200_EINVAL, "null light");
-  if (n_room < 0 || n_boxes < 0 || (n_room > 0 && !room) || (n_boxes > 0 && !boxes)) return ctx_fail(ctx, B200_EINVAL, "bad scene arguments");
-  if (row_begin < 0 || row_end > cam->height || row_begin > row_end) return ctx_fail(ctx, B200_EINVAL, "bad row band");
   const int rows = row_end - row_begin, n = mc->n;
   std::vector<int> edges;
-  // As for the raytracer, the bands move only on the evidence of a frame that ran on the bands of its predecessor:
-  // the frame after a move cannot be pipelined (two host waits, sometimes reallocations -- a 75 ms frame was seen
-  // on 8 GPUs when all devices grew their buffers at once), and balancing on its cost kept the edges moving.  The
-  // tolerance is wider than the raytracer's: a band costs 0.10 - 0.12 ms, of which timing noise is a tenth.
-  const bool have = mc->edges_h[1] == rows && (int)mc->edges[1].size() == n + 1;
-  if (have && !mc->settled[1]) edges = mc->edges[1];
-  else multi_band_edges(have ? mc->edges[1] : std::vector<int>(), mc->cost[1], rows, n, 8, edges, 1.12);
-  mc->settled[1] = have && edges == mc->edges[1];
+  // As for the raytracer, settled edges only: the frame after a move cannot be pipelined (two host waits, sometimes
+  // reallocations -- a 75 ms frame was seen on 8 GPUs when all devices grew their buffers at once), and balancing on
+  // its cost kept the edges moving.  The tolerance is wider than the raytracer's: a band costs 0.10 - 0.12 ms, of
+  // which timing noise is a tenth.
+  multi_settled_edges(mc, 1, rows, 8, 1.12, edges);
   const bool colour = mc->child[0]->opt_rast_colour != 0;
   if (colour) edges.assign(n + 1, rows), edges[0] = 0;   // colour modes number the fragments of the whole frame: one device draws it
   const size_t W = (size_t)cam->width;
@@ -483,9 +385,7 @@ int multi_raster(b200_ctx *ctx, const rast_triangle *room, int n_room, const ras
     if (rc_i != B200_OK) return rc_i;
     const int a = row_begin + edges[i], b = row_begin + edges[i + 1];
     if (b <= a) return b200_synchronize(c);
-    const size_t off = (size_t)(a - row_begin) * W;
-    return rast_band_resident(c, cam, light, a, b, rgb_out ? rgb_out + 3 * off : nullptr, depth_out ? depth_out + off : nullptr,
-                              index_out ? index_out + off : nullptr, argb_out ? argb_out + off : nullptr);
+    return rast_band_resident(c, cam, light, a, b, host.at((size_t)(a - row_begin) * W));
   });
   if (rc != B200_OK) return rc;
   if (!colour) multi_note_cost(mc, 1, edges, rows);

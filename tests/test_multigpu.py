@@ -54,6 +54,11 @@ def test_library_multi_context_raytracer(b200, renderer):
         b = m.render_raytrace(big, sph, cam, h.DEFAULT_RT_LIGHTS, row_begin=40, row_end=171)
         for k in ("rgb", "depth", "index"):
             assert np.array_equal(a[k].view(np.uint32), b[k].view(np.uint32)), k
+        # the camera and row checks of a single context
+        wide = b200.make_camera((0, 0, -3, 1), 200.0, h.identity_R(), 40000, 200)
+        for c, r0, r1 in ((cam, 10, 5), (cam, 0, 201), (wide, 0, 200)):
+            with pytest.raises(b200.B200Error):
+                m.render_raytrace(tris, sph, c, h.DEFAULT_RT_LIGHTS, row_begin=r0, row_end=r1, want=())
         with pytest.raises(b200.B200Error):
             m.rt_upload_scene(tris, sph)          # device-pointer entries exist per device only
     finally:
@@ -83,6 +88,8 @@ def test_library_multi_context_rasteriser(b200, renderer):
                     assert np.array_equal(got[k].view(np.uint32), want[k].view(np.uint32)), (len(rm), frame, k)
                 assert np.array_equal(m.draw_raster(rm, bx, cam, light), want_argb), (len(rm), frame)
         assert m.stats()["fragments"] >= renderer.stats()["fragments"]      # bands overlap by their 2-row halos
+        with pytest.raises(b200.B200Error):
+            m.render_raster(room, boxes, cam, L, want=(), row_begin=10, row_end=5)
     finally:
         m.close()
 

@@ -397,6 +397,60 @@ def test_pipelined_class_changes(b200, tl_renderer, capfd):
 
 
 @pytest.mark.gpu
+def test_pipelined_frame_settled_before_host_draw(b200):
+    """A pipelined whole-Draw frame that outgrew its guess and is still in flight when a host-pointer Draw (raytraced
+    or rasterised) starts on the same context is rendered again before that Draw's rows begin to leave for the
+    caller's buffer: nothing is written around the band, the band equals the same Draw on a fresh context, and the
+    frame in flight equals its own fresh render."""
+    import torch
+    W, H, f = 200, 160, 110.0
+    soup = h.scene_soup_rast(3000, edge=0.03)
+    none = np.zeros(0, h.RAST_TRI)
+    light = h.DEFAULT_RAST_LIGHT
+    L = b200.make_rast_light(light["pos"], light["power"], light["indirect"])
+    far, near = -3.001, 0.2      # far -> near outgrows the guess (test_pipelined_whole_draw_short_and_long)
+    cam_at = lambda z: b200.make_camera(h.f32(0.0, 0.0, z, 1.0), f, h.identity_R(), W, H)
+    tris, sph = h.golden_cornell_rt()
+    rt_cam = b200.make_camera(h.f32(0, 0, -3, 1), 100.0, h.identity_R(), W, H)
+    r0, r1, guard, sentinel = 40, 60, H, 0x5A5A5A5A
+    argb = torch.zeros(H, W, dtype=torch.int32, device="cuda")
+    r, fresh = b200.Renderer(0), b200.Renderer(0)
+
+    def guarded(draw):
+        buf = np.full((guard + r1 - r0 + guard, W), sentinel, np.uint32)
+        draw(buf.ctypes.data + guard * W * 4)
+        assert (buf[:guard] == sentinel).all() and (buf[guard + r1 - r0:] == sentinel).all(), "written outside the band"
+        return buf[guard:guard + r1 - r0]
+
+    try:
+        fresh.rast_upload_scene(soup, none)
+        fresh.rast_draw_device(cam_at(near), L, 0, H, None, None, None, argb.data_ptr())
+        fresh.synchronize()
+        want_frame = argb.cpu().numpy().copy()
+        r.set_option(b200.OPT_RAST_PIPELINED, 1)
+        r.rast_upload_scene(soup, none)
+        host_draws = (
+            (lambda p: r.draw_raytrace_band(tris, sph, rt_cam, h.DEFAULT_RT_LIGHTS, r0, r1, p),
+             fresh.draw_raytrace(tris, sph, rt_cam, h.DEFAULT_RT_LIGHTS)[r0:r1]),
+            (lambda p: r.draw_raster_band(soup, none, cam_at(far), L, r0, r1, p),
+             fresh.draw_raster(soup, none, cam_at(far), L)[r0:r1]))
+        for k, (draw, want_band) in enumerate(host_draws):
+            for z in (far, far):
+                r.rast_draw_device(cam_at(z), L, 0, H, None, None, None, argb.data_ptr())
+                r.synchronize()
+            before = r.stats()["respeculated"]
+            argb.zero_()
+            r.rast_draw_device(cam_at(near), L, 0, H, None, None, None, argb.data_ptr())   # in flight, outgrown
+            band = guarded(draw)
+            assert r.stats()["respeculated"] == before + 1, k
+            assert np.array_equal(band, want_band), k
+            assert np.array_equal(argb.cpu().numpy(), want_frame), k
+    finally:
+        r.close()
+        fresh.close()
+
+
+@pytest.mark.gpu
 def test_pipelined_whole_draw_short_and_long(b200, tl_renderer, capfd):
     """Whole-Draw frames of one scene whose clipped list crosses 2048 triangles with the camera: the guessed
     list length of a short frame cannot hold the long one (rendered again), the long frame's guess holds a

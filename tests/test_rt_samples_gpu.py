@@ -266,6 +266,7 @@ def test_multi_context_equals_one_device(b200, renderer, cornell_rt):
         assert m.stats()["primary_rays"] == 150 * 117 * 10
         assert np.array_equal(m.draw_raytrace_samples(tris, sph, c, LIGHTS8[:2], off, 2),
                               renderer.draw_raytrace_samples(tris, sph, c, LIGHTS8[:2], off, 2))
+        assert m.stats()["primary_rays"] == 150 * 117 * 10
         la = b200.make_lights(LIGHTS8[:2])
         o = np.ascontiguousarray(off)
         assert m.lib.rt_render_samples_device(m.ctx, ctypes.byref(c), la, 2, h.ptr(o), len(o), 0, 0, 117, None, None,
