@@ -25,8 +25,8 @@
 //   L1  for each survivor, each lane tests its pixel's 9-ray bundle box;
 //   L2  per ray: the three plane values decide miss / inside / ambiguous;
 //   EX  reference arithmetic for what is left (about two per ray).
-// Plane records are streamed through shared memory in tiles by 1-D TMA bulk
-// copies (cp.async.bulk + mbarrier), double buffered.
+// Plane records (RT_REC_F4 float4s each) are streamed through shared memory in
+// tiles by 1-D TMA bulk copies (the tile ring of rt_tma.cuh), double buffered.
 #pragma once
 #include "rt_common.cuh"
 #include "rt_exact.cuh"
@@ -34,7 +34,6 @@
 
 constexpr int RT_TILE = 256;      // triangles per shared-memory tile
 constexpr int RT_THREADS = 256;   // 8 warps: a 16x16 pixel block
-constexpr int RT_REC_F4 = 3;      // float4s per plane record (48 bytes)
 // direction grids (rt_grid.cuh)
 constexpr int RT_GRID_G = 64;              // light cube map: cells per face edge
 constexpr int RT_GRID_FACE = RT_GRID_G * RT_GRID_G;

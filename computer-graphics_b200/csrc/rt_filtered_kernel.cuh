@@ -127,31 +127,6 @@ __device__ __forceinline__ void rt_hit_point(float cx, float cy, float cz, float
   px = xadd(cx, xmul(t, dx)); py = xadd(cy, xmul(t, dy)); pz = xadd(cz, xmul(t, dz));
 }
 
-// The TMA tile ring shared by the primary and the shadow passes.
-struct RtRing {
-  float4 *smem;
-  int *smem_idx;     // GRID: triangle index of each record of the tile
-  uint64_t *bars;
-  uint32_t phase_bits;
-  int issued;
-};
-
-// One tile of work: up to TILE consecutive records of a list.
-struct RtItem {
-  const float4 *rec;
-  const int *idx;    // null: the list is the scene itself, record i is triangle base + i
-  int base, cnt;
-};
-
-template <int TILE>
-__device__ __forceinline__ void rt_ring_issue(RtRing &ring, const RtItem &it) {
-  const int buf = ring.issued & 1;
-  const uint32_t rec_bytes = (uint32_t)it.cnt * 48u, idx_bytes = it.idx ? (((uint32_t)it.cnt + 3u) & ~3u) * 4u : 0u;
-  mbar_expect_tx(&ring.bars[buf], rec_bytes + idx_bytes);
-  tma_bulk_g2s(ring.smem + (size_t)buf * TILE * RT_REC_F4, it.rec, rec_bytes, &ring.bars[buf]);
-  if (it.idx) tma_bulk_g2s(ring.smem_idx + buf * TILE, it.idx, idx_bytes, &ring.bars[buf]);
-}
-
 // Walks the lists a pixel block has to stream, tile by tile: the whole scene, or
 // (GRID) the lists of the direction cells in cells[0 .. nc).  Uniform over the block.
 struct RtCursor {
@@ -322,9 +297,9 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
   int *s_seen = s_seen_all + (GRID ? ring_id * RT_SEEN : 0);
   const bool issuer = GRID ? lane == 0 : threadIdx.x == 0;     // who issues the ring's TMA copies
   auto ring_sync = [] { if (GRID) __syncwarp(); else __syncthreads(); };
-  RtRing ring;
-  ring.smem = tile_smem + (size_t)ring_id * 2 * TILE * RT_REC_F4; ring.bars = bars; ring.phase_bits = 0; ring.issued = 0;
-  ring.smem_idx = reinterpret_cast<int *>(tile_smem + (size_t)NRING * 2 * TILE * RT_REC_F4) + ring_id * 2 * TILE;
+  RtRing ring = rt_ring<TILE>(tile_smem + (size_t)ring_id * 2 * TILE * RT_REC_F4,
+                              reinterpret_cast<int *>(tile_smem + (size_t)NRING * 2 * TILE * RT_REC_F4) + ring_id * 2 * TILE,
+                              bars);
 
   // dir = R * vec4(u - W/2, v - H/2, f, 1)   (skeleton.cpp:126-128)
   const float x = (float)(u - p.W / 2), y = (float)(v - p.H / 2);
@@ -412,7 +387,7 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
       if (issuer && have_next) rt_ring_issue<TILE>(ring, next_item);
       mbar_wait(&bars[buf], (ring.phase_bits >> buf) & 1u);
       ring.phase_bits ^= 1u << buf;
-      const float4 *T = ring.smem + (size_t)buf * TILE * RT_REC_F4;
+      const float4 *T = ring.buf[0] + (size_t)buf * TILE * RT_REC_F4;
       const int *Tidx = ring.smem_idx + buf * TILE;
       const bool listed = GRID && item.idx != nullptr;
       const int base = item.base;
@@ -694,7 +669,7 @@ __device__ __forceinline__ void rt_filtered_body(const RtKParams &p, const RtVie
       if (issuer && have_next) rt_ring_issue<TILE>(ring, next_item);
       mbar_wait(&bars[buf], (ring.phase_bits >> buf) & 1u);
       ring.phase_bits ^= 1u << buf;
-      const float4 *T = ring.smem + (size_t)buf * TILE * RT_REC_F4;
+      const float4 *T = ring.buf[0] + (size_t)buf * TILE * RT_REC_F4;
       const int *Tidx = ring.smem_idx + buf * TILE;
       const bool listed = GRID && item.idx != nullptr;
       const int base = item.base;

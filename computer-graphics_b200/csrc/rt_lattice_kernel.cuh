@@ -85,8 +85,7 @@ __global__ void __launch_bounds__(RT_THREADS, 4) rt_lattice_kernel(const __grid_
     mbar_fence_init();
   }
   __syncthreads();
-  RtRing ring;
-  ring.smem = tile_smem; ring.bars = bars; ring.phase_bits = 0; ring.issued = 0; ring.smem_idx = nullptr;
+  RtRing ring = rt_ring<RT_LAT_TILE>(tile_smem, nullptr, bars);
   float *s_ht = reinterpret_cast<float *>(tile_smem + 2 * RT_LAT_TILE * RT_REC_F4);
   float *s_hd = s_ht + RT_LAT_SLOTS * RT_THREADS;
   int *s_hi = reinterpret_cast<int *>(s_hd + RT_LAT_SLOTS * RT_THREADS);
@@ -133,7 +132,7 @@ __global__ void __launch_bounds__(RT_THREADS, 4) rt_lattice_kernel(const __grid_
     }
   }
   unsigned n_exact = 0;
-  const float4 *T0 = ring.smem, *T1 = ring.smem + RT_LAT_TILE * RT_REC_F4;
+  const float4 *T0 = ring.buf[0], *T1 = ring.buf[1];
 
   // ============================ primary rays ============================
   {

@@ -3,8 +3,8 @@
 // DirectLight itself for hits the caller supplies.
 //
 //   rt_rays_kernel<ANY>        one thread per ray, rays in the caller's order.  Every warp streams the scene's
-//                              48-byte RtGeom records through its own double-buffered shared-memory ring (1-D TMA
-//                              bulk copies + mbarriers), culls each tile against the box of its 32 rays and runs the
+//                              48-byte RtGeom records through its own tile ring (rt_ring_stream in rt_tma.cuh, at
+//                              warp scope), culls each tile against the box of its 32 rays and runs the
 //                              reference arithmetic (rt_exact_triangle, ascending index) on the survivors, then the
 //                              spheres (rt_exact_spheres).  ANY = occlusion query: a ray stops at the first pair the
 //                              reference accepts below its limit, a warp leaves when its 32 rays are decided.
@@ -144,18 +144,15 @@ __device__ __forceinline__ bool rt_rays_cull(const RtBundle &B, float4 g0, float
   return false;
 }
 
-// Each warp's double-buffered ring of triangle records.  Set up once per block by rt_rays_ring_init, whose barrier is
-// the only block barrier of the kernels that walk the scene: from there on every warp runs on its own.
-struct RtRing {
-  float4 tiles[RT_RAYS_WARPS][2][RT_RAYS_TILE * 3];
+// The shared memory of the kernels that walk the scene: one ring of triangle records per warp.  Set up once per block by
+// rt_rays_smem_init, whose barrier is the only block barrier of those kernels: from there on every warp runs on its own.
+struct RtRaysSmem {
+  float4 tiles[RT_RAYS_WARPS][2][RT_RAYS_TILE * RT_REC_F4];
   uint64_t bars[RT_RAYS_WARPS][2];
 };
 
-__device__ __forceinline__ void rt_rays_ring_init(RtRing &s) {
-  if (threadIdx.x == 0) {
-    for (int w = 0; w < RT_RAYS_WARPS; ++w) { mbar_init(&s.bars[w][0], 1); mbar_init(&s.bars[w][1], 1); }
-    mbar_fence_init();
-  }
+__device__ __forceinline__ void rt_rays_smem_init(RtRaysSmem &s) {
+  if (threadIdx.x == 0) rt_ring_init(&s.bars[0][0], RT_RAYS_WARPS);
   __syncthreads();
 }
 
@@ -167,7 +164,7 @@ __device__ __forceinline__ void rt_rays_ring_init(RtRing &s) {
 // scene are tame (counters[2] == 0, rt_rays_scene_kernel).  Otherwise fills `best` and returns false.  Adds the exact
 // evaluations to counters[1].
 template <bool ANY, class Params>
-__device__ __forceinline__ bool rt_rays_walk(RtRing &S, const Params &p, float sx, float sy, float sz, float dx, float dy,
+__device__ __forceinline__ bool rt_rays_walk(RtRaysSmem &S, const Params &p, float sx, float sy, float sz, float dx, float dy,
                                              float dz, float maxd, bool active, RtHit &best) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   best.t = 0.f; best.dist = FLT_MAX; best.idx = 0;
@@ -195,28 +192,17 @@ __device__ __forceinline__ bool rt_rays_walk(RtRing &S, const Params &p, float s
   }
 
   bool warp_busy = __any_sync(0xffffffffu, active);
-  const int n_tiles = (p.n_tris + RT_RAYS_TILE - 1) / RT_RAYS_TILE;
-  float4 *ring = &S.tiles[warp][0][0];
-  uint64_t *bars = S.bars[warp];
-  auto issue = [&](int k) {   // lane 0: tile k into buffer k & 1
-    const int cnt = min(RT_RAYS_TILE, p.n_tris - k * RT_RAYS_TILE);
-    uint64_t *bar = &bars[k & 1];
-    mbar_expect_tx(bar, (uint32_t)cnt * 48u);
-    tma_bulk_g2s(ring + (size_t)(k & 1) * RT_RAYS_TILE * 3, p.geom + (size_t)k * RT_RAYS_TILE * 3, (uint32_t)cnt * 48u, bar);
+  RtRing ring = rt_ring<RT_RAYS_TILE>(&S.tiles[warp][0][0], nullptr, S.bars[warp]);
+  const int n_tiles = warp_busy ? (p.n_tris + RT_RAYS_TILE - 1) / RT_RAYS_TILE : 0;
+  int k = 0;
+  auto next = [&](RtItem &it) {   // the scene's records in order
+    if (k >= n_tiles) return false;
+    it.rec = p.geom + (size_t)k * RT_RAYS_TILE * RT_REC_F4; it.idx = nullptr;
+    it.base = k * RT_RAYS_TILE; it.cnt = min(RT_RAYS_TILE, p.n_tris - it.base);
+    ++k;
+    return true;
   };
-  uint32_t phase = 0;
-  if (warp_busy && n_tiles > 0 && lane == 0) issue(0);
-  for (int k = 0; k < n_tiles && warp_busy; ++k) {
-    const int buf = k & 1;
-    __syncwarp();   // every lane is done with the other buffer (tile k - 1): refill it
-    if (k + 1 < n_tiles && lane == 0) {
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // the generic-proxy reads before the async write
-      issue(k + 1);
-    }
-    mbar_wait(&bars[buf], (phase >> buf) & 1u);
-    phase ^= 1u << buf;
-    const float4 *T = ring + (size_t)buf * RT_RAYS_TILE * 3;
-    const int base = k * RT_RAYS_TILE, cnt = min(RT_RAYS_TILE, p.n_tris - base);
+  rt_ring_stream<true, RT_RAYS_TILE>(ring, lane == 0, next, [&](const float4 *T, const int *, int base, int cnt) {
     for (int r0 = 0; r0 < cnt && warp_busy; r0 += 32) {
       // cull: one record per lane against the whole bundle
       bool keep = false;
@@ -241,8 +227,8 @@ __device__ __forceinline__ bool rt_rays_walk(RtRing &S, const Params &p, float s
       }
       if (ANY) warp_busy = __any_sync(0xffffffffu, active);
     }
-    if (!warp_busy && k + 1 < n_tiles) mbar_wait(&bars[buf ^ 1], (phase >> (buf ^ 1)) & 1u);   // drain before leaving
-  }
+    return !ANY || warp_busy;   // only the occlusion query leaves early
+  });
   if (active) rt_exact_spheres(p.sph, p.n_sph, sx, sy, sz, dx, dy, dz, best);   // :341-355
   rt_count(p.counters + 1, n_exact);
   return ANY && (occ || (active && best.dist < FLT_MAX && best.dist < maxd));   // :395-397
@@ -250,8 +236,8 @@ __device__ __forceinline__ bool rt_rays_walk(RtRing &S, const Params &p, float s
 
 template <bool ANY>
 __global__ void __launch_bounds__(RT_RAYS_THREADS) rt_rays_kernel(const __grid_constant__ RtRaysParams p) {
-  __shared__ __align__(128) RtRing S;
-  rt_rays_ring_init(S);
+  __shared__ __align__(128) RtRaysSmem S;
+  rt_rays_smem_init(S);
   const int i = blockIdx.x * RT_RAYS_THREADS + threadIdx.x;
   const bool live = i < p.n;
   float sx = 0.f, sy = 0.f, sz = 0.f, sw = 0.f, dx = 0.f, dy = 0.f, dz = 0.f, maxd = 0.f;
@@ -373,8 +359,8 @@ __device__ __noinline__ void rt_store_power(const RtDirectParams &p, int i, int 
 // blockIdx.y = the light: the 32 shadow rays of a warp share their end point and start on neighbouring hits, which
 // is what the cull of rt_rays_walk needs.
 __global__ void __launch_bounds__(RT_RAYS_THREADS) rt_direct_light_kernel(const __grid_constant__ RtDirectParams p) {
-  __shared__ __align__(128) RtRing S;
-  rt_rays_ring_init(S);
+  __shared__ __align__(128) RtRaysSmem S;
+  rt_rays_smem_init(S);
   const int i = blockIdx.x * RT_RAYS_THREADS + threadIdx.x, l = blockIdx.y;
   const float *L = p.lights[l];
   const RtShadowRay s = rt_shadow_ray(p, i, L);
